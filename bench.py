@@ -41,6 +41,7 @@ if ROOT not in sys.path:
 METRIC = "aligned Gbases/s CallableLoci pileup"
 UNIT = "Gbases/s"
 WORKLOAD = "chr1-size synthetic 30x 2x150bp PE, pileup+classify+BED on one B200 per rank (BASELINE configs[1])"
+DUMP_INTERVAL_ROWS = 1 << 20       # 5 float64 columns of this many rows: 40 MiB, the rest of a dump is a few kB
 
 
 def parse_args():
@@ -60,7 +61,13 @@ def parse_args():
     ap.add_argument("--no-e2e-bam", action="store_true", help="skip the BAM -> BED leg through the C++ coverage command")
     ap.add_argument("--bam-mbp", type=float, default=50.818468, help="contig size of the e2e_bam leg (default: chr22)")
     ap.add_argument("--batch-reads", type=int, default=4_000_000, help="column-batch size of the e2e leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the result of the GPU path (--impl b200)")
+    return args
 
 
 def load_peak():
@@ -217,6 +224,22 @@ def oracle_run(c, reads, opt, length: int):
     oc = run.process_contig(c.name, 0, length, c.ref[:length], reads)
     dt = time.perf_counter() - t0
     return oc, run, dt, reads
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """What a caller of the resident step receives (a ContigDeviceResult) as out_dir/<name>.npy, float64: counters and bins
+    whole; of the interval list the rows interval_row, a seeded sample of DUMP_INTERVAL_ROWS rows (every row of a shorter
+    list), so that two builds computing the same intervals write the same files."""
+    iv = res.intervals
+    n = iv.shape[0]
+    rows = np.arange(n) if n <= DUMP_INTERVAL_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_INTERVAL_ROWS, replace=False))
+    arrays = {"state_counts": res.state_counts, "bins": res.bins, "stride": res.stride, "n_covered_bases": res.n_covered_bases,
+              "summed_coverage": res.summed_coverage, "summed_baseq": res.summed_baseq, "summed_mapq": res.summed_mapq,
+              "quality_bases": res.quality_bases, "n_intervals": n, "interval_row": rows, "interval_start": iv["start"][rows],
+              "interval_end": iv["end"][rows], "interval_state": iv["state"][rows], "interval_soft_start": iv["soft_start"][rows]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def run_reference(args, rank, world):
@@ -549,6 +572,8 @@ def main():
         dist.barrier()
     total_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.refresh_counters())     # the last timed step's result, before anything runs again
     step_ms = []                                         # per-step device times of three more steps, outside the timed region
     for _ in range(3):
         ms, _ = ctx.rerun_resident(fetch=False)
