@@ -12,6 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CLB_LIB") or os.path.join(_HERE, "libcallable_loci_b200.so")
 
 CLB_OK = 0
+CLB_E_IO = -5
 ERRORS = {-1: "CLB_E_INVALID", -2: "CLB_E_CUDA", -3: "CLB_E_INPUT", -4: "CLB_E_UNSUPPORTED", -5: "CLB_E_IO"}
 
 

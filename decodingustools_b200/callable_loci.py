@@ -281,10 +281,11 @@ class CallableProfiler:
 
     def __init__(self, bed_file: Optional[str], largest_contig_length: int):
         self._L = _lib.lib()
+        self.bed_file = bed_file
         self.largest_contig_length = int(largest_contig_length)
         self._w = self._L.clb_bed_writer_open(bed_file.encode() if bed_file else None, self.largest_contig_length)
         if not self._w:
-            raise ClbError(-5, f"cannot create {bed_file}")
+            raise ClbError(_lib.CLB_E_IO, f"cannot create {bed_file}")
         self.contig_counts: Dict[str, np.ndarray] = {}
         self._closed = False
 
@@ -295,7 +296,7 @@ class CallableProfiler:
         rc = self._L.clb_bed_writer_add_contig(self._w, name.encode(), int(length), _ptr(iv), iv.shape[0], _ptr(b),
                                                0 if b is None else b.shape[1], int(stride), C.byref(has))
         if rc != 0:
-            raise ClbError(rc, f"intervals of {name} do not tile [0,{length})")
+            raise ClbError(rc, f"cannot write {self.bed_file}" if rc == _lib.CLB_E_IO else f"intervals of {name} do not tile [0,{length})")
         self.contig_counts[name] = np.array(state_counts, dtype=np.uint64)
         return (b if has.value else None)
 
@@ -310,7 +311,9 @@ class CallableProfiler:
     def close(self):
         if not self._closed:
             self._closed = True
-            self._L.clb_bed_writer_close(self._w)
+            rc = self._L.clb_bed_writer_close(self._w)
+            if rc != 0:
+                raise ClbError(rc, f"cannot write {self.bed_file}")
 
     def __del__(self):
         try:

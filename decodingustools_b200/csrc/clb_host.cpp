@@ -299,13 +299,14 @@ struct clb_bed_writer {
     FILE *fp = nullptr;
     std::string mem;
     bool in_memory = false;
+    bool io_failed = false;        // the first failed stdio / pwrite call; add_contig and close report it as CLB_E_IO
     uint32_t largest = 0;
     bool have_pending = false;     // CallableProfiler::current_state survives finish_contig (quirk Q1)
     std::string pend_name;
     clb_interval pend{};
     std::vector<char> buf;
     struct Part { std::unique_ptr<char[]> p; size_t cap = 0; };
-    std::vector<Part> parts;                // per-thread formatting buffers of large contigs (reused, never zero-filled)
+    std::vector<Part> parts;                // per-thread formatting buffers (reused, never zero-filled)
     void put(const char *s, size_t n) {
         if (in_memory) mem.append(s, n);
         else {
@@ -313,15 +314,10 @@ struct clb_bed_writer {
             buf.insert(buf.end(), s, s + n);
         }
     }
-    void flush() { if (fp && !buf.empty()) { fwrite(buf.data(), 1, buf.size(), fp); buf.clear(); } }
+    void flush() {
+        if (fp && !buf.empty()) { if (fwrite(buf.data(), 1, buf.size(), fp) != buf.size()) io_failed = true; buf.clear(); }
+    }
 };
-
-static inline char *put_u32(char *p, uint32_t v) {
-    char tmp[10]; int n = 0;
-    do { tmp[n++] = (char)('0' + v % 10); v /= 10; } while (v);
-    while (n) *p++ = tmp[--n];
-    return p;
-}
 
 static const uint8_t kStateLen[6] = {5, 8, 11, 12, 18, 20};
 // decimal text of v, two digits per step
@@ -336,18 +332,25 @@ static inline char *put_u32_fast(char *p, uint32_t v) {
     return e;
 }
 
-static void write_line(clb_bed_writer *w, const std::string &name, const clb_interval &iv) {
-    char line[64];
-    char *p = line;
-    *p++ = '\t'; p = put_u32(p, iv.start); *p++ = '\t'; p = put_u32(p, iv.end); *p++ = '\t';
-    const char *sn = kStateName[iv.state < 6 ? iv.state : 0];
-    const size_t sl = strlen(sn);
-    memcpy(p, sn, sl); p += sl; *p++ = '\n';
-    w->put(name.data(), name.size());
-    w->put(line, (size_t)(p - line));
-}
-
 static inline bool binned_state(uint8_t s) { return s == CLB_CALLABLE || s == CLB_POOR_MAPPING_QUALITY || s == CLB_REF_N; }
+
+// The BED lines of iv[lo, hi) (states already validated) into out; returns their length.  *binned |= whether one of them
+// has a binned state.
+static size_t format_lines(clb_bed_writer::Part &out, const std::string &name, const clb_interval *iv, uint64_t lo, uint64_t hi, bool *binned) {
+    const size_t max_line = name.size() + 1 + 10 + 1 + 10 + 1 + 20 + 1;
+    if (out.cap < (size_t)(hi - lo) * max_line) { out.cap = (size_t)(hi - lo) * max_line; out.p.reset(new char[out.cap]); }
+    char *p = out.p.get();
+    bool any = false;
+    for (uint64_t i = lo; i < hi; i++) {
+        memcpy(p, name.data(), name.size()); p += name.size();
+        *p++ = '\t'; p = put_u32_fast(p, iv[i].start); *p++ = '\t'; p = put_u32_fast(p, iv[i].end); *p++ = '\t';
+        const uint8_t st = iv[i].state;
+        memcpy(p, kStateName[st], kStateLen[st]); p += kStateLen[st]; *p++ = '\n';
+        any |= binned_state(st);
+    }
+    *binned |= any;
+    return (size_t)(p - out.p.get());
+}
 
 extern "C" clb_bed_writer *clb_bed_writer_open(const char *path, uint32_t largest_contig_len) {
     clb_bed_writer *w = new clb_bed_writer();
@@ -370,12 +373,16 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
     }
     if (expect != contig_len) return CLB_E_INPUT;
     const std::string nm(name);
+    // large contigs are formatted on several threads (BED text of a 30x human chromosome is ~100 MB)
+    const uint32_t nt = n_iv < (1u << 16) ? 1 : clb_host_threads();
+    if (w->parts.size() < nt) w->parts.resize(nt);
     bool any_range = false;
     // Q1: the first position of a contig (or finish_contig of an empty one) flushes the previous contig's
     // last run once more; Q2: that flush also pushes it into THIS contig's coverage_ranges.
     if (w->have_pending) {
-        write_line(w, w->pend_name, w->pend);
-        if (binned_state(w->pend.state)) {
+        bool binned = false;
+        w->put(w->parts[0].p.get(), format_lines(w->parts[0], w->pend_name, &w->pend, 0, 1, &binned));
+        if (binned) {
             any_range = true;
             if (bins_inout && n_bins && stride) {
                 uint32_t *row = bins_inout + (size_t)(w->pend.state == CLB_CALLABLE ? 0 : w->pend.state == CLB_POOR_MAPPING_QUALITY ? 1 : 2) * n_bins;
@@ -390,23 +397,16 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
             }
         }
     }
-    if (n_iv < (1u << 16)) {
-        for (uint64_t i = 0; i < n_iv; i++) {
-            write_line(w, nm, iv[i]);
-            if (binned_state(iv[i].state)) any_range = true;
-        }
+    if (nt == 1) {
+        w->put(w->parts[0].p.get(), format_lines(w->parts[0], nm, iv, 0, n_iv, &any_range));
     } else {
-        // large contigs: format on several threads, each into its own reusable buffer, then copy / pwrite the parts to
-        // their final offsets in parallel (BED text of a 30x human chromosome is ~100 MB)
-        const uint32_t nt = clb_host_threads();
+        // each thread formats into its own reusable buffer, then the parts are copied / pwritten to their final offsets in parallel
         const bool dbg_t = getenv("CLB_ADMIT_DEBUG") != nullptr;
         auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
         const double t0 = now();
-        if (w->parts.size() < nt) w->parts.resize(nt);
         std::vector<size_t> sizes(nt, 0);
         std::vector<int> binned(nt, 0);
         const uint64_t per = (n_iv + nt - 1) / nt;
-        const size_t max_line = nm.size() + 1 + 10 + 1 + 10 + 1 + 20 + 1;
         auto run_threads = [&](auto &&fn) {
             std::vector<std::thread> th;
             for (uint32_t t = 1; t < nt; t++) th.emplace_back(fn, t);
@@ -415,18 +415,9 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
         };
         run_threads([&](uint32_t t) {
             const uint64_t lo = std::min(n_iv, t * per), hi = std::min(n_iv, lo + per);
-            clb_bed_writer::Part &out = w->parts[t];
-            if (out.cap < (size_t)(hi - lo) * max_line) { out.cap = (size_t)(hi - lo) * max_line; out.p.reset(new char[out.cap]); }
-            char *p = out.p.get();
-            int any = 0;
-            for (uint64_t i = lo; i < hi; i++) {
-                memcpy(p, nm.data(), nm.size()); p += nm.size();
-                *p++ = '\t'; p = put_u32_fast(p, iv[i].start); *p++ = '\t'; p = put_u32_fast(p, iv[i].end); *p++ = '\t';
-                const uint8_t st = iv[i].state;
-                memcpy(p, kStateName[st], kStateLen[st]); p += kStateLen[st]; *p++ = '\n';
-                any |= binned_state(st) ? 1 : 0;
-            }
-            sizes[t] = (size_t)(p - out.p.get()); binned[t] = any;
+            bool b = false;
+            sizes[t] = format_lines(w->parts[t], nm, iv, lo, hi, &b);
+            binned[t] = b;
         });
         const double t1 = now();
         std::vector<size_t> off(nt + 1, 0);
@@ -436,26 +427,31 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
             w->mem.resize(base + off[nt]);
             run_threads([&](uint32_t t) { memcpy(&w->mem[base + off[t]], w->parts[t].p.get(), sizes[t]); });
         } else {
-            w->flush(); fflush(w->fp);
+            w->flush();
+            if (fflush(w->fp) != 0) w->io_failed = true;
             const off_t base = ftello(w->fp);
-            const int fd = fileno(w->fp);
-            std::atomic<int> io_err{0};
-            run_threads([&](uint32_t t) {
-                size_t done = 0;
-                while (done < sizes[t]) {
-                    const ssize_t r = pwrite(fd, w->parts[t].p.get() + done, sizes[t] - done, base + (off_t)(off[t] + done));
-                    if (r <= 0) { io_err = 1; break; }
-                    done += (size_t)r;
-                }
-            });
-            if (io_err) return CLB_E_IO;
-            fseeko(w->fp, base + (off_t)off[nt], SEEK_SET);
+            if (base >= 0) {                                     // a seekable file: every part goes straight to its offset
+                const int fd = fileno(w->fp);
+                std::atomic<bool> io_err{false};
+                run_threads([&](uint32_t t) {
+                    size_t done = 0;
+                    while (done < sizes[t]) {
+                        const ssize_t r = pwrite(fd, w->parts[t].p.get() + done, sizes[t] - done, base + (off_t)(off[t] + done));
+                        if (r <= 0) { io_err = true; break; }
+                        done += (size_t)r;
+                    }
+                });
+                if (io_err || fseeko(w->fp, base + (off_t)off[nt], SEEK_SET) != 0) w->io_failed = true;
+            } else {                                             // a pipe or a terminal: in order
+                for (uint32_t t = 0; t < nt; t++)
+                    if (fwrite(w->parts[t].p.get(), 1, sizes[t], w->fp) != sizes[t]) w->io_failed = true;
+            }
         }
         if (dbg_t) fprintf(stderr, "clb_bed_writer_add_contig: %u threads, format %.3f s, output %.3f s (%zu bytes)\n", nt, t1 - t0, now() - t1, off[nt]);
     }
     if (n_iv) { w->have_pending = true; w->pend_name = nm; w->pend = iv[n_iv - 1]; }
     if (has_bins) *has_bins = any_range ? 1 : 0;
-    return CLB_OK;
+    return w->io_failed ? CLB_E_IO : CLB_OK;
 }
 
 extern "C" const char *clb_bed_writer_buffer(clb_bed_writer *w, uint64_t *len) {
@@ -466,8 +462,8 @@ extern "C" const char *clb_bed_writer_buffer(clb_bed_writer *w, uint64_t *len) {
 
 extern "C" int clb_bed_writer_close(clb_bed_writer *w) {
     if (!w) return CLB_E_INVALID;
-    int rc = CLB_OK;
-    if (w->fp) { w->flush(); if (fclose(w->fp) != 0) rc = CLB_E_IO; }
+    if (w->fp) { w->flush(); if (fclose(w->fp) != 0) w->io_failed = true; }
+    const int rc = w->io_failed ? CLB_E_IO : CLB_OK;
     delete w;
     return rc;
 }

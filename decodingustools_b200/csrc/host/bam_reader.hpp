@@ -95,14 +95,17 @@ class BgzfStream {
     }
     // Hands out the next batch of inflated bytes: buf[kHeadroom ..) is the data, the kHeadroom bytes in front of it are
     // free for the caller (the record scan copies the unfinished tail of the previous batch there instead of moving the
-    // batch).  Returns false at EOF.
+    // batch).  Returns false at EOF.  A read or inflate failure is thrown once the batches before it have been handed out,
+    // so it surfaces where the data ends, not whenever the read-ahead thread got there.
     static constexpr size_t kHeadroom = 4u << 20;
     bool next(std::vector<uint8_t> &buf) {
         if (!reader_.joinable() && !finished_) start_reader();
         std::unique_lock<std::mutex> g(m_);
         cv_.wait(g, [this] { return !q_.empty() || finished_; });
-        if (!error_.empty()) { const std::string e = error_; g.unlock(); die(e); }
-        if (q_.empty()) return false;
+        if (q_.empty()) {
+            if (!error_.empty()) { const std::string e = error_; g.unlock(); die(e); }
+            return false;
+        }
         buf = std::move(q_.front());
         q_.pop_front();
         g.unlock();

@@ -30,6 +30,7 @@
 #include <cstring>
 #include <fstream>
 #include <map>
+#include <memory>
 #include <set>
 #include <stdexcept>
 #include <string>
@@ -113,6 +114,12 @@ struct PinBatch {
     size_t n = 0, n_cigar = 0, n_qual = 0, cap_n = 0, cap_c = 0, cap_q = 0;
     int32_t *pos = nullptr; uint16_t *flag = nullptr; uint8_t *mapq = nullptr;
     uint32_t *cigar_off = nullptr, *cigar = nullptr; uint64_t *qual_off = nullptr; uint8_t *qual = nullptr;
+    PinBatch() = default;
+    PinBatch(const PinBatch &) = delete;
+    PinBatch &operator=(const PinBatch &) = delete;
+    ~PinBatch() {
+        for (void *p : {(void *)pos, (void *)flag, (void *)mapq, (void *)cigar_off, (void *)cigar, (void *)qual_off, (void *)qual}) clb_host_free(p);
+    }
     template <class T> static void grow(T *&p, size_t used, size_t ncap) {
         T *q = (T *)clb_host_alloc(ncap * sizeof(T));
         if (!q) die("cannot allocate page-locked host memory");
@@ -134,10 +141,6 @@ struct PinBatch {
         memcpy(qual + n_qual, r.qual, lq); n_qual += lq;
         n++;
         cigar_off[n] = (uint32_t)n_cigar; qual_off[n] = n_qual;
-    }
-    void release() {
-        for (void *p : {(void *)pos, (void *)flag, (void *)mapq, (void *)cigar_off, (void *)cigar, (void *)qual_off, (void *)qual}) clb_host_free(p);
-        *this = PinBatch();
     }
 };
 
@@ -183,21 +186,117 @@ struct NameStore {
     }
 };
 
-// decoder thread -> device thread
-struct Msg { PinBatch *batch = nullptr; bool end_of_contig = false; NameStore *names = nullptr; uint64_t admitted = 0; std::string error; };
+// A queue between the two threads.  close() wakes every waiter; from then on put() drops its value and returns false, and
+// take() returns false instead of blocking.
 template <class T> class Channel {
   public:
-    void put(T v) { { std::lock_guard<std::mutex> g(m_); q_.push_back(std::move(v)); } cv_.notify_one(); }
-    T take(double *waited_s = nullptr) {
+    bool put(T v) {
+        { std::lock_guard<std::mutex> g(m_); if (closed_) return false; q_.push_back(std::move(v)); }
+        cv_.notify_one();
+        return true;
+    }
+    bool take(T &v, double *waited_s = nullptr) {
         std::unique_lock<std::mutex> g(m_);
         const auto t0 = std::chrono::steady_clock::now();
-        cv_.wait(g, [this] { return !q_.empty(); });
+        cv_.wait(g, [this] { return !q_.empty() || closed_; });
         if (waited_s) *waited_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-        T v = std::move(q_.front()); q_.pop_front();
-        return v;
+        if (closed_) return false;
+        v = std::move(q_.front()); q_.pop_front();
+        return true;
     }
+    void close() { { std::lock_guard<std::mutex> g(m_); closed_ = true; } cv_.notify_all(); }
   private:
-    std::mutex m_; std::condition_variable cv_; std::deque<T> q_;
+    std::mutex m_; std::condition_variable cv_; std::deque<T> q_; bool closed_ = false;
+};
+
+double secs_since(std::chrono::steady_clock::time_point a) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - a).count(); }
+
+// decoder thread -> device thread: a full batch, or the end of a contig (its last batch, QNAMEs and admitted count), or an error
+struct Msg { PinBatch *batch = nullptr; bool end_of_contig = false; std::unique_ptr<NameStore> names; uint64_t admitted = 0; std::string error; };
+
+// The decoder thread: BGZF read-ahead + inflate pool (bam_reader.hpp) -> record scan -> htslib admission, one record at a time
+// (clb_admitter_*) -> admitted records packed into page-locked column batches + QNAME store, handed to the device thread.
+// It owns the thread, the three batches and both channels, and borrows the reader, the index (nullptr: scan the file from the
+// start) and the contig list (tid, length), which must outlive it.  Closing the channels is the stop request: a blocked take()
+// returns, the next hand-over fails and the thread returns.  The destructor closes them and joins, so a failure on the device
+// thread (an exception unwinding past this object) cannot leave the decoder running.
+class DecodeStage {
+  public:
+    DecodeStage(BamReader &bam, const BaiIndex *bai, const std::vector<std::pair<int32_t, uint32_t>> &contigs, uint32_t maxcnt, size_t batch_reads)
+        : bam_(bam), bai_(bai), contigs_(contigs), maxcnt_(maxcnt) {
+        for (auto &b : pool_) { b.reserve(batch_reads, 2 * batch_reads, 160 * batch_reads); free_.put(&b); }
+        thread_ = std::thread([this] { run(); });
+    }
+    ~DecodeStage() { free_.close(); ready_.close(); if (thread_.joinable()) thread_.join(); }
+    DecodeStage(const DecodeStage &) = delete;
+    DecodeStage &operator=(const DecodeStage &) = delete;
+
+    Msg take(double *waited_s) { Msg m; if (!ready_.take(m, waited_s)) m.error = "the decoder stopped"; return m; }
+    void give_back(PinBatch *b) { free_.put(b); }
+    void join() { thread_.join(); }   // after the last end-of-contig message; the timings below are final from then on
+    double total_s = 0, waited_for_batch_s = 0, admission_s = 0;
+
+  private:
+    void run() {
+        const auto t_start = std::chrono::steady_clock::now();
+        const uint64_t tick_start = ticks();
+        try {
+            scan();
+        } catch (const std::exception &e) {
+            Msg m; m.error = e.what(); m.end_of_contig = true; ready_.put(std::move(m));
+        }
+        total_s = secs_since(t_start);
+        admission_s = total_s > 0 ? (double)admit_ticks_ * total_s / (double)std::max<uint64_t>(1, ticks() - tick_start) : 0.0;
+    }
+    bool next_free(PinBatch *&b) {
+        if (!free_.take(b, &waited_for_batch_s)) return false;
+        b->clear();
+        return true;
+    }
+    void scan() {
+        BamRecordView rec; bool have = bai_ ? false : bam_.next(rec);
+        for (const auto &[tid, clen] : contigs_) {                        // ascending tid (api/coverage.rs:229-235)
+            if (bai_) {
+                have = bai_->first[(size_t)tid] != UINT64_MAX;
+                if (have) { bam_.seek(bai_->first[(size_t)tid]); have = bam_.next(rec); }
+            }
+            while (have && (rec.tid < tid && rec.tid >= 0)) have = bam_.next(rec);   // records of contigs that were not selected
+            const std::unique_ptr<clb_admitter, decltype(&clb_admitter_free)> adm(clb_admitter_new(tid, maxcnt_), clb_admitter_free);
+            auto names = std::make_unique<NameStore>();
+            PinBatch *cur = nullptr; uint64_t admitted = 0;
+            while (have && rec.tid == tid) {
+                const uint64_t ta = ticks();
+                const int k = clb_admitter_push(adm.get(), rec.pos, rec.flag, rec.cigar, rec.n_cigar);
+                admit_ticks_ += ticks() - ta;
+                if (k < 0) die("Error processing contig: records are not coordinate sorted");
+                if (k == 1) {
+                    if (!cur && !next_free(cur)) return;
+                    if (!cur->fits(rec)) {
+                        if (cur->n) { Msg m; m.batch = cur; if (!ready_.put(std::move(m)) || !next_free(cur)) return; }
+                        if (!cur->fits(rec)) cur->reserve(std::max<size_t>(cur->cap_n, 1), std::max<size_t>(cur->cap_c, 2 * (size_t)rec.n_cigar),
+                                                          std::max<size_t>(cur->cap_q, 2 * (size_t)std::max(0, rec.l_seq)));
+                    }
+                    cur->push(rec); admitted++;
+                    uint64_t span = 0;
+                    for (uint32_t c = 0; c < rec.n_cigar; c++) { const uint32_t op = rec.cigar[c] & 15; if ((0x18du >> op) & 1u) span += rec.cigar[c] >> 4; }
+                    if (span && (uint32_t)rec.pos < clen) names->add(rec.qname, rec.l_qname ? rec.l_qname - 1 : 0);
+                }
+                have = bam_.next(rec);
+            }
+            Msg m; m.batch = cur; m.end_of_contig = true; m.names = std::move(names); m.admitted = admitted;
+            if (!ready_.put(std::move(m))) return;
+        }
+    }
+
+    BamReader &bam_;
+    const BaiIndex *bai_;
+    const std::vector<std::pair<int32_t, uint32_t>> &contigs_;
+    const uint32_t maxcnt_;
+    uint64_t admit_ticks_ = 0;   // per-record timing with the cycle counter (a clock call per record would cost more than the admission)
+    PinBatch pool_[3];
+    Channel<PinBatch *> free_;
+    Channel<Msg> ready_;
+    std::thread thread_;
 };
 
 struct Options {
@@ -217,7 +316,7 @@ void usage() {
     exit(2);
 }
 
-int run(int argc, char **argv) {
+Options parse_options(int argc, char **argv) {
     if (argc < 3 || strcmp(argv[1], "coverage") != 0) usage();
     Options opt;
     for (int i = 2; i < argc; i++) {
@@ -244,218 +343,141 @@ int run(int argc, char **argv) {
         else usage();
     }
     if (opt.bam.empty() || opt.reference.empty()) usage();
+    return opt;
+}
 
-    BamReader bam(opt.bam, opt.threads);
-    const BamHeader &H = bam.header();
-    const auto fai = load_fai(opt.reference);
+// --progress: the reference API's ProgressEvent stream (api/mod.rs:12-18, emitted by CoverageAnalyzer::analyze at
+// api/coverage.rs:40-48), one serde-style JSON object per line on stderr; Progress counts finished contigs
+void progress(const Options &opt, const char *kind, const std::string &extra = "") {
+    if (opt.progress) fprintf(stderr, "{\"%s\":{\"task\":\"Coverage Analysis\"%s}}\n", kind, extra.c_str());
+}
 
-    // initialize_contig_stats + validate_contig_selection (api/coverage.rs:149-204)
-    std::set<std::string> selected(opt.contigs.begin(), opt.contigs.end());
-    std::map<int32_t, ContigStats> stats;
-    for (size_t tid = 0; tid < H.names.size(); tid++) {
-        if (opt.have_contigs && !selected.count(H.names[tid])) continue;
-        ContigStats s; s.name = H.names[tid]; s.length = H.lens[tid];
-        stats[(int32_t)tid] = s;
-    }
-    if (opt.have_contigs && stats.empty()) {
-        std::string l; for (size_t i = 0; i < opt.contigs.size(); i++) l += (i ? ", " : "") + opt.contigs[i];
-        die("None of the specified contigs (" + l + ") were found in the BAM file");
-    }
-    uint32_t largest = 0;                                               // initialize_counter (api/coverage.rs:206-219)
-    for (auto &kv : stats) if (kv.second.name != "chrM") largest = std::max<uint32_t>(largest, (uint32_t)kv.second.length);
+bool write_file(const std::string &path, const std::string &data) {
+    FILE *f = fopen(path.c_str(), "wb");
+    if (!f) return false;
+    const bool ok = fwrite(data.data(), 1, data.size(), f) == data.size();
+    return fclose(f) == 0 && ok;
+}
 
-    char err[512];
-    clb_ctx *ctx = clb_create(opt.device, &opt.o, err, sizeof err);
-    if (!ctx) die(std::string("GPU context: ") + err);
-    clb_bed_writer *bed = clb_bed_writer_open(opt.out_bed.c_str(), largest);
-    if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
+// What the contig loop measured, for the stderr summary line and --timing-json.
+struct Timing {
+    double wall_s = 0, decode_total_s = 0, decode_wait_s = 0, admit_s = 0;
+    double device_ms = 0, h2d_ms = 0, bed_s = 0, names_s = 0, ref_s = 0, device_wait_s = 0;
+    uint64_t total_admitted = 0, total_cells = 0;
+};
+
+// The pipeline over the selected contigs:
+// decoder thread: DecodeStage
+// this thread   : clb_begin_contig / clb_push_reads per batch (copies overlap the kernels of earlier windows and the
+//                 decoding of the next batch) / clb_finish_contig, BED text, plots
+Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, const std::map<std::string, FaiEntry> &fai,
+                       std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed) {
     auto check = [&](int rc, const char *what) { if (rc != 0) die(std::string("Error processing contig: ") + what + ": " + clb_last_error(ctx)); };
-
-    // BamStats: its own pass over the first 10 000 records of the file, primary alignments only (bam_stats.rs:44-76)
-    report::BamStats bs;
-    {
-        BamReader head(opt.bam, std::min(opt.threads, 4u));
-        BamRecordView r;
-        while (!bs.full() && head.next(r)) bs.add_record(std::string(r.qname, r.l_qname ? r.l_qname - 1 : 0), r.flag, (uint64_t)std::max(0, r.l_seq));
-    }
-    // With a contig selection and a .bai next to the BAM the reader jumps to each contig (what bam.fetch does, mod.rs:54);
-    // otherwise the coordinate-sorted file is scanned once from the start.
-    BaiIndex bai;
-    const bool indexed = opt.have_contigs && load_bai(opt.bam, bai) && bai.first.size() == H.names.size();
     // coverage plots land next to the BED file (callable_profiler.rs:24-27,80-83)
     const size_t slash = opt.out_bed.find_last_of('/');
     const std::string out_dir = slash == std::string::npos ? "" : opt.out_bed.substr(0, slash + 1);
-
-    // ------------------------------------------------------------------------------------------ the pipeline
-    // decoder thread: BGZF read-ahead + inflate pool (bam_reader.hpp) -> record scan -> htslib admission, one record at a
-    //                 time (clb_admitter_*) -> admitted records packed into page-locked column batches + QNAME store
-    // this thread   : clb_begin_contig / clb_push_reads per batch (copies overlap the kernels of earlier windows and the
-    //                 decoding of the next batch) / clb_finish_contig, BED text, plots
     const uint32_t maxcnt = opt.o.max_depth > 0 ? opt.o.max_depth : 500;
     const auto wall0 = std::chrono::steady_clock::now();
-    auto secs = [](std::chrono::steady_clock::time_point a) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - a).count(); };
     // batches of about a million reads for real inputs, small ones for small files (page-locking memory is not free)
     size_t kBatchReads = 1u << 20;
     {
         FILE *fsz = fopen(opt.bam.c_str(), "rb");
         if (fsz) { fseeko(fsz, 0, SEEK_END); const off_t sz = ftello(fsz); fclose(fsz); if (sz < (off_t)(256u << 20)) kBatchReads = std::max<size_t>(4096, (size_t)sz / 64); }
     }
-    constexpr int kBatches = 3;
-    PinBatch pool[kBatches];
-    Channel<PinBatch *> free_batches;
-    Channel<Msg> ready;
-    for (auto &b : pool) { b.reserve(kBatchReads, 2 * kBatchReads, 160 * kBatchReads); free_batches.put(&b); }
-    double decode_wait_s = 0, decode_total_s = 0, admit_s = 0;
-    uint64_t admit_ticks = 0;                      // per-record timing with the cycle counter (a clock call per record would cost more than the admission)
-    std::vector<int32_t> tids; std::map<int32_t, uint32_t> lens;
-    for (auto &kv : stats) { tids.push_back(kv.first); lens[kv.first] = (uint32_t)kv.second.length; }
-    std::thread decoder([&] {
-        const auto t_start = std::chrono::steady_clock::now();
-        const uint64_t tick_start = ticks();
-        try {
-            BamRecordView rec; bool have = indexed ? false : bam.next(rec);
-            for (const int32_t tid : tids) {                              // ascending tid (api/coverage.rs:229-235)
-                const uint32_t clen = lens.at(tid);
-                if (indexed) {
-                    have = bai.first[(size_t)tid] != UINT64_MAX;
-                    if (have) { bam.seek(bai.first[(size_t)tid]); have = bam.next(rec); }
-                }
-                while (have && (rec.tid < tid && rec.tid >= 0)) have = bam.next(rec);   // records of contigs that were not selected
-                clb_admitter *adm = clb_admitter_new(tid, maxcnt);
-                NameStore *names = new NameStore();
-                PinBatch *cur = nullptr; uint64_t admitted = 0;
-                while (have && rec.tid == tid) {
-                    const uint64_t ta = ticks();
-                    const int k = clb_admitter_push(adm, rec.pos, rec.flag, rec.cigar, rec.n_cigar);
-                    admit_ticks += ticks() - ta;
-                    if (k < 0) { clb_admitter_free(adm); die("Error processing contig: records are not coordinate sorted"); }
-                    if (k == 1) {
-                        if (!cur) { cur = free_batches.take(&decode_wait_s); cur->clear(); }
-                        if (!cur->fits(rec)) {
-                            if (cur->n) { Msg m; m.batch = cur; ready.put(std::move(m)); cur = free_batches.take(&decode_wait_s); cur->clear(); }
-                            if (!cur->fits(rec)) cur->reserve(std::max<size_t>(cur->cap_n, 1), std::max<size_t>(cur->cap_c, 2 * (size_t)rec.n_cigar),
-                                                              std::max<size_t>(cur->cap_q, 2 * (size_t)std::max(0, rec.l_seq)));
-                        }
-                        cur->push(rec); admitted++;
-                        uint64_t span = 0;
-                        for (uint32_t c = 0; c < rec.n_cigar; c++) { const uint32_t op = rec.cigar[c] & 15; if ((0x18du >> op) & 1u) span += rec.cigar[c] >> 4; }
-                        if (span && (uint32_t)rec.pos < clen) names->add(rec.qname, rec.l_qname ? rec.l_qname - 1 : 0);
+    std::vector<std::pair<int32_t, uint32_t>> contigs;
+    for (auto &kv : stats) contigs.emplace_back(kv.first, (uint32_t)kv.second.length);
+    Timing t;
+    {
+        DecodeStage decoder(bam, bai, contigs, maxcnt, kBatchReads);
+        size_t contigs_done = 0;
+        for (auto &kv : stats) {
+            ContigStats &st = kv.second;
+            const uint32_t clen = (uint32_t)st.length;
+            const auto tr = std::chrono::steady_clock::now();
+            std::vector<uint8_t> ref;
+            auto fe = fai.find(st.name);
+            if (fe != fai.end()) ref = load_contig(opt.reference, fe->second);   // missing contig / short sequence reads as 'N'
+            t.ref_s += secs_since(tr);
+            check(clb_begin_contig(ctx, kv.first, st.name.c_str(), clen, ref.data(), ref.size(), 0, largest, 0, clen, 0), "begin");
+            std::unique_ptr<NameStore> names; uint64_t admitted = 0;
+            for (;;) {
+                Msg m = decoder.take(&t.device_wait_s);
+                if (!m.error.empty()) die(m.error);
+                if (m.batch) {
+                    if (m.batch->n) {
+                        clb_read_batch rb{m.batch->n, m.batch->n_cigar, m.batch->n_qual, m.batch->pos, m.batch->flag, m.batch->mapq,
+                                          m.batch->cigar_off, m.batch->cigar, m.batch->qual_off, m.batch->qual};
+                        check(clb_push_reads(ctx, &rb), "push");
+                        check(clb_wait_uploads(ctx), "upload");                  // the batch's buffers go back to the decoder
                     }
-                    have = bam.next(rec);
+                    decoder.give_back(m.batch);
                 }
-                clb_admitter_free(adm);
-                Msg m; m.batch = cur; m.end_of_contig = true; m.names = names; m.admitted = admitted;
-                ready.put(std::move(m));
+                if (m.end_of_contig) { names = std::move(m.names); admitted = m.admitted; break; }
             }
-        } catch (const std::exception &e) {
-            Msg m; m.error = e.what(); m.end_of_contig = true; ready.put(std::move(m));
+            clb_contig_result res{};
+            check(clb_finish_contig(ctx, &res), "finish");
+            t.device_ms += res.kernel_ms; t.h2d_ms += res.h2d_ms;
+            const auto tn = std::chrono::steady_clock::now();
+            st.n_reads = names->count_unique(opt.threads);
+            names.reset();
+            t.names_s += secs_since(tn);
+            for (int s = 0; s < 6; s++) st.counts[s] = res.state_counts[s];
+            st.n_covered = res.n_covered_bases; st.sum_cov = res.summed_coverage; st.sum_bq = res.summed_baseq;
+            st.sum_mapq = res.summed_mapq; st.qbases = res.quality_bases;
+            t.total_admitted += admitted; t.total_cells += res.summed_coverage;
+            const auto tb = std::chrono::steady_clock::now();
+            std::vector<uint32_t> bins(res.bins, res.bins + 3 * (size_t)res.n_bins);
+            int has_bins = 0;
+            const int rc = clb_bed_writer_add_contig(bed, st.name.c_str(), clen, res.intervals, res.n_intervals, bins.data(), res.n_bins, res.stride, &has_bins);
+            if (rc == CLB_E_IO) die("Error processing contig: cannot write " + opt.out_bed);
+            if (rc != 0) die("Error processing contig: interval list does not tile the contig");
+            if (has_bins && res.stride) {                                        // finish_contig, callable_profiler.rs:64-86
+                const std::string path = out_dir + st.name + "_coverage.svg";
+                if (!write_file(path, report::render_coverage_svg(st.name, clen, res.stride, bins.data(), res.n_bins)))
+                    die("Error processing contig: cannot create " + path);
+            }
+            t.bed_s += secs_since(tb);
+            if (opt.verbose)
+                fprintf(stderr, "%s: %llu admitted reads, %llu cells, %.2f ms on device\n", st.name.c_str(), (unsigned long long)admitted,
+                        (unsigned long long)res.summed_coverage, res.kernel_ms);
+            progress(opt, "Progress", ",\"current\":" + std::to_string(++contigs_done) + ",\"total\":" + std::to_string(stats.size()));
         }
-        decode_total_s = secs(t_start);
-        admit_s = decode_total_s > 0 ? (double)admit_ticks * decode_total_s / (double)std::max<uint64_t>(1, ticks() - tick_start) : 0.0;
-    });
+        decoder.join();
+        t.decode_total_s = decoder.total_s; t.decode_wait_s = decoder.waited_for_batch_s; t.admit_s = decoder.admission_s;
+    }   // the batches are freed here, inside the wall time
+    t.wall_s = secs_since(wall0);
+    return t;
+}
 
-    double device_ms = 0, h2d_ms = 0, bed_s = 0, names_s = 0, ref_s = 0, device_wait_s = 0;
-    uint64_t total_admitted = 0, total_cells = 0;
-    std::string failure;
-    // --progress: the reference API's ProgressEvent stream (api/mod.rs:12-18, emitted by CoverageAnalyzer::analyze at
-    // api/coverage.rs:40-48), one serde-style JSON object per line on stderr; Progress counts finished contigs
-    auto progress = [&](const char *kind, const std::string &extra) {
-        if (opt.progress) fprintf(stderr, "{\"%s\":{\"task\":\"Coverage Analysis\"%s}}\n", kind, extra.c_str());
-    };
-    progress("Started", "");
-    size_t contigs_done = 0;
-    for (const int32_t tid : tids) {
-        ContigStats &st = stats[tid];
-        const uint32_t clen = (uint32_t)st.length;
-        const auto tr = std::chrono::steady_clock::now();
-        std::vector<uint8_t> ref;
-        auto fe = fai.find(st.name);
-        if (fe != fai.end()) ref = load_contig(opt.reference, fe->second);   // missing contig / short sequence reads as 'N'
-        ref_s += secs(tr);
-        check(clb_begin_contig(ctx, tid, st.name.c_str(), clen, ref.data(), ref.size(), 0, largest, 0, clen, 0), "begin");
-        NameStore *names = nullptr; uint64_t admitted = 0;
-        for (;;) {
-            Msg m = ready.take(&device_wait_s);
-            if (!m.error.empty()) { failure = m.error; break; }
-            if (m.batch) {
-                if (m.batch->n) {
-                    clb_read_batch rb{m.batch->n, m.batch->n_cigar, m.batch->n_qual, m.batch->pos, m.batch->flag, m.batch->mapq,
-                                      m.batch->cigar_off, m.batch->cigar, m.batch->qual_off, m.batch->qual};
-                    check(clb_push_reads(ctx, &rb), "push");
-                    check(clb_wait_uploads(ctx), "upload");                  // the batch's buffers go back to the decoder
-                }
-                free_batches.put(m.batch);
-            }
-            if (m.end_of_contig) { names = m.names; admitted = m.admitted; break; }
-        }
-        if (!failure.empty()) break;
-        clb_contig_result res{};
-        check(clb_finish_contig(ctx, &res), "finish");
-        device_ms += res.kernel_ms; h2d_ms += res.h2d_ms;
-        const auto tn = std::chrono::steady_clock::now();
-        st.n_reads = names ? names->count_unique(opt.threads) : 0;
-        delete names;
-        names_s += secs(tn);
-        for (int s = 0; s < 6; s++) st.counts[s] = res.state_counts[s];
-        st.n_covered = res.n_covered_bases; st.sum_cov = res.summed_coverage; st.sum_bq = res.summed_baseq;
-        st.sum_mapq = res.summed_mapq; st.qbases = res.quality_bases;
-        total_admitted += admitted; total_cells += res.summed_coverage;
-        const auto tb = std::chrono::steady_clock::now();
-        std::vector<uint32_t> bins(res.bins, res.bins + 3 * (size_t)res.n_bins);
-        int has_bins = 0;
-        if (clb_bed_writer_add_contig(bed, st.name.c_str(), clen, res.intervals, res.n_intervals, bins.data(), res.n_bins, res.stride, &has_bins) != 0)
-            die("Error processing contig: interval list does not tile the contig");
-        if (has_bins && res.stride) {                                        // finish_contig, callable_profiler.rs:64-86
-            const std::string svg = report::render_coverage_svg(st.name, clen, res.stride, bins.data(), res.n_bins);
-            const std::string path = out_dir + st.name + "_coverage.svg";
-            FILE *fs = fopen(path.c_str(), "wb");
-            if (!fs) die("Error processing contig: cannot create " + path);
-            fwrite(svg.data(), 1, svg.size(), fs); fclose(fs);
-        }
-        bed_s += secs(tb);
-        if (opt.verbose)
-            fprintf(stderr, "%s: %llu admitted reads, %llu cells, %.2f ms on device\n", st.name.c_str(), (unsigned long long)admitted,
-                    (unsigned long long)res.summed_coverage, res.kernel_ms);
-        progress("Progress", ",\"current\":" + std::to_string(++contigs_done) + ",\"total\":" + std::to_string(tids.size()));
-    }
-    if (!failure.empty()) {
-        // let the decoder run dry so that it can be joined
-        std::thread drain([&] { for (;;) { Msg m = ready.take(); if (m.batch) free_batches.put(m.batch); delete m.names; if (!m.error.empty()) break; } });
-        drain.detach();
-        decoder.detach();
-        progress("Error", ",\"error\":\"" + failure + "\"");
-        die(failure);
-    }
-    decoder.join();
-    for (auto &b : pool) b.release();
-    const double wall_s = secs(wall0);
+void report_timing(const Options &opt, const Timing &t, size_t n_contigs, double inflate_s) {
     fprintf(stderr, "coverage: %zu contigs, %llu admitted reads, %llu aligned bases | wall %.3f s | host decode %.3f s (BGZF inflate %.3f s on %u threads, "
                     "admission %.3f s inline, waiting for a free batch %.3f s) | device %.3f s kernels, %.3f s H2D | reference load %.3f s | "
                     "unique names %.3f s | BED + plots %.3f s | device thread waited %.3f s for the decoder\n",
-            tids.size(), (unsigned long long)total_admitted, (unsigned long long)total_cells, wall_s, decode_total_s - decode_wait_s,
-            bam.inflate_seconds(), opt.threads, admit_s, decode_wait_s, device_ms * 1e-3, h2d_ms * 1e-3, ref_s, names_s, bed_s, device_wait_s);
+            n_contigs, (unsigned long long)t.total_admitted, (unsigned long long)t.total_cells, t.wall_s, t.decode_total_s - t.decode_wait_s,
+            inflate_s, opt.threads, t.admit_s, t.decode_wait_s, t.device_ms * 1e-3, t.h2d_ms * 1e-3, t.ref_s, t.names_s, t.bed_s, t.device_wait_s);
     if (!opt.timing_json.empty()) {
         FILE *ft = fopen(opt.timing_json.c_str(), "wb");
         if (ft) {
             fprintf(ft, "{\"contigs\": %zu, \"admitted_reads\": %llu, \"aligned_bases\": %llu, \"wall_s\": %.6f, \"decode_s\": %.6f, \"inflate_s\": %.6f, "
                         "\"threads\": %u, \"admission_s\": %.6f, \"decoder_waited_for_batch_s\": %.6f, \"device_kernels_s\": %.6f, \"h2d_s\": %.6f, "
                         "\"reference_load_s\": %.6f, \"unique_names_s\": %.6f, \"bed_and_plots_s\": %.6f, \"device_thread_waited_s\": %.6f}\n",
-                    tids.size(), (unsigned long long)total_admitted, (unsigned long long)total_cells, wall_s, decode_total_s - decode_wait_s, bam.inflate_seconds(),
-                    opt.threads, admit_s, decode_wait_s, device_ms * 1e-3, h2d_ms * 1e-3, ref_s, names_s, bed_s, device_wait_s);
+                    n_contigs, (unsigned long long)t.total_admitted, (unsigned long long)t.total_cells, t.wall_s, t.decode_total_s - t.decode_wait_s, inflate_s,
+                    opt.threads, t.admit_s, t.decode_wait_s, t.device_ms * 1e-3, t.h2d_ms * 1e-3, t.ref_s, t.names_s, t.bed_s, t.device_wait_s);
             fclose(ft);
         }
     }
-    if (clb_bed_writer_close(bed) != 0) die("failed to write " + opt.out_bed);
-    clb_destroy(ctx);
+}
 
-    // build_coverage_export (report.rs:15-134)
+// build_coverage_export (report.rs:15-134): writes summary.json and returns what the HTML page shows (the summary; rows gets
+// one row per contig in natural order)
+report::Summary write_summary_json(const Options &opt, const std::string &header_text, const report::BamStats &bs,
+                                   const std::map<int32_t, ContigStats> &stats, std::vector<report::ContigRow> &rows) {
     std::vector<const ContigStats *> order;
     for (auto &kv : stats) order.push_back(&kv.second);
     std::stable_sort(order.begin(), order.end(), [](const ContigStats *a, const ContigStats *b) { return contig_less(a->name, b->name); });
     uint64_t total_bases = 0, callable = 0, q30_bases = 0, total_qpos = 0, total_unique = 0;
     double total_depth = 0, total_mapq = 0, total_baseq = 0;
     std::string cj;
-    std::vector<report::ContigRow> rows;
     auto exists = [](const std::string &p) { FILE *f = fopen(p.c_str(), "rb"); if (f) fclose(f); return f != nullptr; };
     for (size_t i = 0; i < order.size(); i++) {
         const ContigStats &s = *order[i];
@@ -489,8 +511,8 @@ int run(int argc, char **argv) {
         if (exists(p)) plots += std::string(plots.empty() ? "\n      " : ",\n      ") + jstr(p);
     }
     if (!plots.empty()) plots += "\n    ";
-    std::string js = "{\n  \"export\": {\n    \"summary\": {\n      \"aligner\": " + jstr(detect_aligner(H.text)) + ",\n      \"reference_build\": " +
-        jstr(reference_build(H.text)) + ",\n      \"sequencing_platform\": " + jstr(bs.infer_platform()) + ",\n      \"read_length\": " + std::to_string(bs.average_read_length()) +
+    std::string js = "{\n  \"export\": {\n    \"summary\": {\n      \"aligner\": " + jstr(detect_aligner(header_text)) + ",\n      \"reference_build\": " +
+        jstr(reference_build(header_text)) + ",\n      \"sequencing_platform\": " + jstr(bs.infer_platform()) + ",\n      \"read_length\": " + std::to_string(bs.average_read_length()) +
         ",\n      \"total_bases\": " + std::to_string(total_bases) + ",\n      \"callable_bases\": " + std::to_string(callable) +
         ",\n      \"callable_percentage\": " + fmt_f64(call_pct) + ",\n      \"average_depth\": " + fmt_f64(avg_depth) + ",\n      \"contigs_analyzed\": " +
         std::to_string(stats.size()) + "\n    },\n    \"contigs\": [" + (order.empty() ? "" : "\n" + cj + "\n    ") + "],\n    \"quality_metrics\": {\n      \"average_mapq\": " +
@@ -498,22 +520,73 @@ int run(int argc, char **argv) {
         ",\n      \"q30_percentage\": " + fmt_f64(total_qpos ? ((double)q30_bases / (double)total_qpos) * 100.0 : 0.0) + "\n    },\n    \"total_unique_reads\": " +
         std::to_string(total_unique) + "\n  },\n  \"files\": {\n    \"bed_file\": " + jstr(opt.out_bed) + ",\n    \"summary_html\": " + jstr(opt.summary) +
         ",\n    \"coverage_plots\": [" + plots + "]\n  }\n}";
-    FILE *fj = fopen("summary.json", "wb");                                  // main.rs:68: always in the CWD
-    if (!fj) die("cannot create summary.json");
-    fwrite(js.data(), 1, js.size(), fj); fclose(fj);
+    if (!write_file("summary.json", js)) die("cannot create summary.json");   // main.rs:68: always in the CWD
+    return report::Summary{reference_build(header_text), detect_aligner(header_text), bs.infer_platform(), bs.average_read_length(), total_unique, total_bases,
+                           callable, (uint64_t)stats.size(), bs.max_samples, call_pct, avg_depth, total_qpos ? total_mapq / (double)total_qpos : 0.0,
+                           total_qpos ? total_baseq / (double)total_qpos : 0.0};
+}
 
-    // write_html_report (report.rs:136-160)
+// write_html_report (report.rs:136-160)
+void write_html_report(const Options &opt, const report::Summary &sm, const std::vector<report::ContigRow> &rows) {
     auto slurp = [](const std::string &p) { std::ifstream f(p, std::ios::binary); if (!f) die("cannot read " + p); return std::string((std::istreambuf_iterator<char>(f)), std::istreambuf_iterator<char>()); };
     const std::string header = opt.templates.empty() ? report::default_header() : slurp(opt.templates + "/report_header.html");
     const std::string footer = opt.templates.empty() ? report::default_footer() : slurp(opt.templates + "/report_footer.html");
-    report::Summary sm{reference_build(H.text), detect_aligner(H.text), bs.infer_platform(), bs.average_read_length(), total_unique, total_bases, callable,
-                       (uint64_t)stats.size(), bs.max_samples, call_pct, avg_depth, total_qpos ? total_mapq / (double)total_qpos : 0.0,
-                       total_qpos ? total_baseq / (double)total_qpos : 0.0};
-    const std::string html = report::render_html_report(sm, rows, header, footer);
-    FILE *fh = fopen(opt.summary.c_str(), "wb");
-    if (!fh) die("cannot create " + opt.summary);
-    fwrite(html.data(), 1, html.size(), fh); fclose(fh);
-    progress("Completed", "");
+    if (!write_file(opt.summary, report::render_html_report(sm, rows, header, footer))) die("cannot create " + opt.summary);
+}
+
+int run(int argc, char **argv) {
+    const Options opt = parse_options(argc, argv);
+    BamReader bam(opt.bam, opt.threads);
+    const BamHeader &H = bam.header();
+    const auto fai = load_fai(opt.reference);
+
+    // initialize_contig_stats + validate_contig_selection (api/coverage.rs:149-204)
+    std::set<std::string> selected(opt.contigs.begin(), opt.contigs.end());
+    std::map<int32_t, ContigStats> stats;
+    for (size_t tid = 0; tid < H.names.size(); tid++) {
+        if (opt.have_contigs && !selected.count(H.names[tid])) continue;
+        ContigStats s; s.name = H.names[tid]; s.length = H.lens[tid];
+        stats[(int32_t)tid] = s;
+    }
+    if (opt.have_contigs && stats.empty()) {
+        std::string l; for (size_t i = 0; i < opt.contigs.size(); i++) l += (i ? ", " : "") + opt.contigs[i];
+        die("None of the specified contigs (" + l + ") were found in the BAM file");
+    }
+    uint32_t largest = 0;                                               // initialize_counter (api/coverage.rs:206-219)
+    for (auto &kv : stats) if (kv.second.name != "chrM") largest = std::max<uint32_t>(largest, (uint32_t)kv.second.length);
+
+    char err[512];
+    std::unique_ptr<clb_ctx, decltype(&clb_destroy)> ctx(clb_create(opt.device, &opt.o, err, sizeof err), clb_destroy);
+    if (!ctx) die(std::string("GPU context: ") + err);
+    std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
+    if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
+
+    // BamStats: its own pass over the first 10 000 records of the file, primary alignments only (bam_stats.rs:44-76)
+    report::BamStats bs;
+    {
+        BamReader head(opt.bam, std::min(opt.threads, 4u));
+        BamRecordView r;
+        while (!bs.full() && head.next(r)) bs.add_record(std::string(r.qname, r.l_qname ? r.l_qname - 1 : 0), r.flag, (uint64_t)std::max(0, r.l_seq));
+    }
+    // With a contig selection and a .bai next to the BAM the reader jumps to each contig (what bam.fetch does, mod.rs:54);
+    // otherwise the coordinate-sorted file is scanned once from the start.
+    BaiIndex bai;
+    const bool indexed = opt.have_contigs && load_bai(opt.bam, bai) && bai.first.size() == H.names.size();
+
+    progress(opt, "Started");
+    try {
+        const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get());
+        report_timing(opt, t, stats.size(), bam.inflate_seconds());
+        if (clb_bed_writer_close(bed.release()) != 0) die("failed to write " + opt.out_bed);
+        ctx.reset();
+        std::vector<report::ContigRow> rows;
+        const report::Summary sm = write_summary_json(opt, H.text, bs, stats, rows);
+        write_html_report(opt, sm, rows);
+    } catch (const std::exception &e) {
+        progress(opt, "Error", ",\"error\":" + jstr(e.what()));
+        throw;
+    }
+    progress(opt, "Completed");
     return 0;
 }
 

@@ -91,6 +91,43 @@ def test_cli_errors_like_the_reference(tmp_path):
     assert p.returncode != 0 and "None of the specified contigs (chrZ) were found in the BAM file" in p.stderr
 
 
+@pytest.mark.parametrize("case", ["unsorted", "truncated", "svg_collision_1_contig", "svg_collision_6_contigs"])
+def test_cli_failures_exit_1_with_the_error(tmp_path, case):
+    """Bad input files and unwritable outputs end in `Error: <message>` and exit code 1, whichever thread meets the failure
+    (decoder: unsorted or truncated BAM; device thread: a directory where a coverage plot goes, while the decoder is done
+    or still running).  With --progress the failure is also the last event, after Started."""
+    cs = [synth.synth_short("chr1", 120_000, seed=44)]
+    if case == "svg_collision_6_contigs":
+        cs += [synth.synth_short(f"chr{i}", 60_000, seed=44 + i) for i in range(2, 7)]
+    contigs = [(c.name, c.length, c.reads) for c in cs]
+    if case == "unsorted":                                   # the second half of the records in reverse order
+        n = cs[0].reads.n
+        contigs = [(cs[0].name, cs[0].length, cs[0].reads.select(np.concatenate([np.arange(n // 2), np.arange(n - 1, n // 2 - 1, -1)])))]
+        want = "Error processing contig: records are not coordinate sorted"
+    elif case == "truncated":
+        want = "truncated"
+    else:
+        (tmp_path / "chr1_coverage.svg").mkdir()
+        want = f"Error processing contig: cannot create {tmp_path / 'chr1_coverage.svg'}"
+    bam = str(tmp_path / "in.bam"); fa = str(tmp_path / "ref.fa")
+    bamio.write_bam(bam, contigs); bamio.write_fasta(fa, [(c.name, c.ref) for c in cs])
+    if case == "truncated":
+        raw = open(bam, "rb").read()
+        open(bam, "wb").write(raw[: len(raw) * 2 // 3])
+    for extra in ([], ["--progress"]):
+        p = subprocess.run([CLI, "coverage", bam, "-r", fa, "-o", str(tmp_path / "out.bed"), *extra], cwd=tmp_path,
+                           capture_output=True, text=True, timeout=120)
+        assert p.returncode == 1, p.stderr[-2000:]
+        last = p.stderr.splitlines()[-1]
+        assert last.startswith("Error: ") and want in last, p.stderr[-2000:]
+        events = [json.loads(line) for line in p.stderr.splitlines() if line.startswith("{")]
+        if extra:
+            assert events[0] == {"Started": {"task": "Coverage Analysis"}}
+            assert events[-1] == {"Error": {"task": "Coverage Analysis", "error": last[len("Error: "):]}}
+        else:
+            assert events == []
+
+
 def test_cli_report_outputs_match_the_python_mirror(tmp_path):
     """Rows N2-N4: SVG plots from the device bins, HTML page, platform inference -- C++ (report_writer.hpp) against the
     Python mirror (report.py / bam_stats.py) fed with the ORACLE's bins and the JSON the CLI wrote."""

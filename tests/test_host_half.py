@@ -2,6 +2,7 @@
 No compute call touches a GPU here."""
 import os
 import re
+import threading
 
 import numpy as np
 import pytest
@@ -193,7 +194,8 @@ def test_nmask_packing():
 
 def test_bed_writer_large_contig_threads_and_file(tmp_path):
     """More than 65536 runs: the threaded formatter, in memory and through pwrite, against plain Python formatting;
-    a small contig afterwards checks the file offset is left at the end (and quirk Q1 across the two)."""
+    a small contig afterwards checks the file offset is left at the end (and quirk Q1 across the two).  Then the same through a
+    FIFO, and into /dev/full, which must fail with CLB_E_IO."""
     rng = np.random.default_rng(77)
     n = 150_000
     lens = rng.integers(1, 3000, size=n)
@@ -217,3 +219,31 @@ def test_bed_writer_large_contig_threads_and_file(tmp_path):
     f.add_contig("chrBig", L, iv, np.zeros(6), None, 0); f.add_contig("s", 7, small, np.zeros(6), None, 0)
     f.close()
     assert open(path, "rb").read() == want_all
+    # a pipe cannot seek: the parts are written in order
+    fifo = str(tmp_path / "bed.fifo")
+    os.mkfifo(fifo)
+    got = []
+    reader = threading.Thread(target=lambda: got.append(open(fifo, "rb").read()))
+    reader.start()
+    try:
+        p = CallableProfiler(fifo, L)
+        try:
+            p.add_contig("chrBig", L, iv, np.zeros(6), None, 0); p.add_contig("s", 7, small, np.zeros(6), None, 0)
+        finally:
+            p.close()
+    finally:
+        reader.join()
+    assert got == [want_all]
+    # a full disk is an error, whether it shows up in add_contig (large contig) or only when the buffer is flushed at close
+    full = CallableProfiler("/dev/full", L)
+    with pytest.raises(_lib.ClbError) as e:
+        full.add_contig("chrBig", L, iv, np.zeros(6), None, 0)
+    assert e.value.code == _lib.CLB_E_IO and "cannot write /dev/full" in str(e.value)
+    with pytest.raises(_lib.ClbError) as e:
+        full.close()
+    assert e.value.code == _lib.CLB_E_IO
+    full = CallableProfiler("/dev/full", L)
+    full.add_contig("s", 7, small, np.zeros(6), None, 0)
+    with pytest.raises(_lib.ClbError) as e:
+        full.close()
+    assert e.value.code == _lib.CLB_E_IO
