@@ -223,7 +223,7 @@ int launch_compaction(clb_ctx *ctx) {
     }
     const uint32_t n_blk = (ctx->n_windows + 1023) / 1024;
     k_scan_windows_local<<<n_blk, 1024, 0, ctx->s_compute>>>((const uint2 *)ctx->win_tab.p, ctx->n_windows, (uint32_t *)ctx->win_out.p,
-                                                            (uint32_t *)ctx->blk_tot.p);
+                                                            (uint32_t *)ctx->blk_tot.p, (const uint32_t *)ctx->misc.p + M_ERR);
     k_scan_blocks<<<1, 1024, 0, ctx->s_compute>>>((uint32_t *)ctx->blk_tot.p, n_blk, (uint32_t *)ctx->misc.p + M_NTOTAL);
     const uint32_t warps_per_block = 8;
     k_gather_intervals<<<(ctx->n_windows + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, ctx->s_compute>>>(

@@ -53,6 +53,9 @@ constexpr int STAT_STRIDE = 16;       // one 128-byte line per global counter (u
 enum { ST_REF_N = 0, ST_CALLABLE = 1, ST_NO_COVERAGE = 2, ST_LOW_COVERAGE = 3, ST_EXCESSIVE = 4, ST_POOR_MAPQ = 5 };
 enum { S_COUNT0 = 0, S_COVERED = 6, S_SUMCOV = 7, S_SUMBQ = 8, S_SUMMAPQ = 9, S_QBASES = 10, S_RESERVED = 11, N_STATS = 12 };
 enum { ERR_QUAL_SPAN = 1, ERR_REC_OVERFLOW = 2, ERR_UNSORTED = 8, ERR_OFFSETS = 16 };
+// the kernels after the pileup do not touch win_tab / rec once one of these is set: k_validate_batch refused the columns (the
+// pileup kernels returned before writing win_tab[w]) or a window could not be run; the host reports the error instead
+constexpr uint32_t ERR_RESULT_INVALID = ERR_UNSORTED | ERR_OFFSETS | ERR_QUAL_SPAN;
 
 struct KParams {
     // packed read columns (device)
@@ -933,6 +936,7 @@ __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P
 // a fixed small grid walks the queue; with an empty queue the launch costs a few microseconds.
 template <bool BQ_HI, bool DBG>
 __global__ void __launch_bounds__(NT, 1) k_pileup_classify_deep(const KParams P) {
+    if (*P.err & ERR_RESULT_INVALID) return;
     const uint32_t n = *P.deep_count;
     for (uint32_t i = blockIdx.x; i < n; i += gridDim.x) {
         pileup_classify_window<BQ_HI, true, DBG>(P, P.deep_list[i]);
@@ -1163,9 +1167,11 @@ __device__ __forceinline__ uint32_t win_drop_first(const uint2 *win_tab, uint32_
 }
 
 // step 1: every block scans 1024 windows locally and publishes its total
-__global__ void __launch_bounds__(1024) k_scan_windows_local(const uint2 *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot) {
+__global__ void __launch_bounds__(1024) k_scan_windows_local(const uint2 *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot,
+                                                             const uint32_t *err) {
     __shared__ uint32_t sW[32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (*err & ERR_RESULT_INVALID) return;                    // win_tab was not written: nothing to scan
     const uint32_t i = blockIdx.x * 1024u + tid;
     const uint32_t v = i < n_w ? (win_tab[i].y & 0xfffu) - win_drop_first(win_tab, i) : 0u;
     uint32_t inc = v;
@@ -1205,12 +1211,13 @@ __global__ void __launch_bounds__(1024) k_scan_blocks(uint32_t *blk_tot, uint32_
 
 // one warp per window: move its records to their sorted place (start/state/soft; end filled next)
 // (nothing to gather when the record buffer overflowed: the records past its capacity were never written and the
-// interval array is just as small; the host grows both and re-runs the contig)
+// interval array is just as small; the host grows both and re-runs the contig.  Nothing either when the input was refused:
+// win_tab and the scan hold whatever an earlier contig, or no contig, left there)
 __global__ void k_gather_intervals(const unsigned long long *rec, const uint2 *win_tab, const uint32_t *win_out, const uint32_t *blk_off,
                                    uint32_t n_w, IntervalOut *out, const uint32_t *err) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    if (w >= n_w || (*err & ERR_REC_OVERFLOW)) return;
+    if (w >= n_w || (*err & (ERR_REC_OVERFLOW | ERR_RESULT_INVALID))) return;
     const uint2 t = win_tab[w];
     const uint32_t skip = win_drop_first(win_tab, w);
     const uint32_t o = blk_off[w >> 10] + win_out[w], cnt = (t.y & 0xfffu) - skip;
@@ -1222,7 +1229,7 @@ __global__ void k_gather_intervals(const unsigned long long *rec, const uint2 *w
 }
 
 __global__ void k_fill_ends(IntervalOut *out, const uint32_t *n_total, uint32_t region_end, const uint32_t *err) {
-    if (*err & ERR_REC_OVERFLOW) return;
+    if (*err & (ERR_REC_OVERFLOW | ERR_RESULT_INVALID)) return;
     const uint32_t n = *n_total;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
         out[i].end = (i + 1 < n) ? out[i + 1].start : region_end;
