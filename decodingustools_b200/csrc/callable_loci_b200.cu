@@ -158,6 +158,15 @@ KParams make_params(clb_ctx *c) {
     return P;
 }
 
+// The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
+// with the per-base dump (parity tests).  f is called with two std::integral_constant<bool, ...>.
+template <typename F>
+void with_variant(bool bq_hi, bool dbg, F &&f) {
+    using T = std::true_type; using N = std::false_type;
+    if (bq_hi) { if (dbg) f(T{}, T{}); else f(T{}, N{}); }
+    else { if (dbg) f(N{}, T{}); else f(N{}, N{}); }
+}
+
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
 // queue of windows the other two handed over) for windows [w0, w1) on the compute stream
 int launch_windows(clb_ctx *ctx, uint32_t w0, uint32_t w1, EvPair *time_pileup = nullptr, EvPair *time_fast = nullptr) {
@@ -175,24 +184,16 @@ int launch_windows(clb_ctx *ctx, uint32_t w0, uint32_t w1, EvPair *time_pileup =
     const bool hi = ctx->opt.min_base_quality >= 128;
     if (!all_general) {
         if (time_fast) CU(cudaEventRecord(time_fast->a, ctx->s_compute));
-        if (ctx->dbg) {                                  // per-base dump requested (parity tests): separate instantiation
-            if (hi) k_pileup_fast<true, true><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
-            else k_pileup_fast<false, true><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
-        } else {
-            if (hi) k_pileup_fast<true, false><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
-            else k_pileup_fast<false, false><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
-        }
+        with_variant(hi, ctx->dbg, [&](auto h, auto d) {
+            k_pileup_fast<decltype(h)::value, decltype(d)::value><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
+        });
         if (time_fast) CU(cudaEventRecord(time_fast->b, ctx->s_compute));
         ctx->launches += 1;
     }
     const uint32_t g = (uint32_t)std::min<uint64_t>((uint64_t)ctx->n_sm * std::max(1, ctx->max_ctas_per_sm), all_general ? n : 0xffffffffu);
-    if (ctx->dbg) {
-        if (hi) k_pileup_general<true, true><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
-        else k_pileup_general<false, true><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
-    } else {
-        if (hi) k_pileup_general<true, false><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
-        else k_pileup_general<false, false><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
-    }
+    with_variant(hi, ctx->dbg, [&](auto h, auto d) {
+        k_pileup_general<decltype(h)::value, decltype(d)::value><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
+    });
     if (time_pileup) CU(cudaEventRecord(time_pileup->b, ctx->s_compute));
     ctx->launches += 2;
     CU(cudaGetLastError());
@@ -211,14 +212,9 @@ int launch_compaction(clb_ctx *ctx) {
     {
         // windows with more than 65535 candidate reads were queued by the general kernel (normally none)
         const KParams P = make_params(ctx);
-        const bool hi = ctx->opt.min_base_quality >= 128;
-        if (ctx->dbg) {
-            if (hi) k_pileup_classify_deep<true, true><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
-            else k_pileup_classify_deep<false, true><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
-        } else {
-            if (hi) k_pileup_classify_deep<true, false><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
-            else k_pileup_classify_deep<false, false><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
-        }
+        with_variant(ctx->opt.min_base_quality >= 128, ctx->dbg, [&](auto h, auto d) {
+            k_pileup_classify_deep<decltype(h)::value, decltype(d)::value><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
+        });
         ctx->launches += 1;
     }
     const uint32_t n_blk = (ctx->n_windows + 1023) / 1024;
@@ -371,16 +367,15 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-#define CLB_SMEM_ATTR(kernel, bytes) \
-    if ((e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(bytes))) != cudaSuccess) { \
-        clb_destroy(ctx); return bail("cudaFuncSetAttribute(" #kernel ")", e); }
-    CLB_SMEM_ATTR((k_pileup_general<false, false>), SMEM_BYTES) CLB_SMEM_ATTR((k_pileup_general<true, false>), SMEM_BYTES)
-    CLB_SMEM_ATTR((k_pileup_general<false, true>), SMEM_BYTES) CLB_SMEM_ATTR((k_pileup_general<true, true>), SMEM_BYTES)
-    CLB_SMEM_ATTR((k_pileup_classify_deep<false, false>), SMEM_BYTES_DEEP) CLB_SMEM_ATTR((k_pileup_classify_deep<true, false>), SMEM_BYTES_DEEP)
-    CLB_SMEM_ATTR((k_pileup_classify_deep<false, true>), SMEM_BYTES_DEEP) CLB_SMEM_ATTR((k_pileup_classify_deep<true, true>), SMEM_BYTES_DEEP)
-    CLB_SMEM_ATTR((k_pileup_fast<false, false>), F_SMEM) CLB_SMEM_ATTR((k_pileup_fast<true, false>), F_SMEM)
-    CLB_SMEM_ATTR((k_pileup_fast<false, true>), F_SMEM) CLB_SMEM_ATTR((k_pileup_fast<true, true>), F_SMEM)
-#undef CLB_SMEM_ATTR
+    for (int v = 0; v < 4; v++)                              // every instantiation of the pileup kernels
+        with_variant(v & 1, v & 2, [&](auto h, auto d) {
+            constexpr bool H = decltype(h)::value, D = decltype(d)::value;
+            const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_general<H, D>, smem, (int)SMEM_BYTES);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_classify_deep<H, D>, smem, (int)SMEM_BYTES_DEEP);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_fast<H, D>, smem, (int)F_SMEM);
+        });
+    if (e != cudaSuccess) { clb_destroy(ctx); return bail("cudaFuncSetAttribute (pileup kernels)", e); }
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->max_ctas_per_sm, k_pileup_general<false, false>, NT, SMEM_BYTES);
     cudaDeviceGetAttribute(&ctx->n_sm, cudaDevAttrMultiProcessorCount, device);
     if ((e = cudaMalloc((void **)&ctx->d_first_tab, 65536 * 4 + WIN_TABLE_BYTES + 256)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaMalloc", e); }

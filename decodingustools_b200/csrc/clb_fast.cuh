@@ -55,11 +55,6 @@ static_assert(F_OFF_WSTATS + NWARPS * N_STATS * 8 <= F_OFF_X, "phase C scratch f
 static_assert(CLB_F_MINB * (F_SMEM + 1024) <= 228 * 1024, "shared memory per SM");
 enum { FC_BAIL = 0, FC_XCNT = 1 };
 
-// window table word y: record count | first state << 12 | window-soft first record << 16 | last state << 20
-__device__ __forceinline__ uint32_t pack_win_y(uint32_t count, uint32_t first_state, uint32_t wsoft, uint32_t last_state) {
-    return count | (first_state << 12) | (wsoft << 16) | (last_state << 20);
-}
-
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -100,70 +95,44 @@ __device__ __forceinline__ uint32_t bytes_ge(uint32_t x, uint32_t t_low) {
     return (BQ_HI ? (x & d) : (x | d)) & H;
 }
 
-// One 16-byte chunk whose bytes all belong to the segment: 6 instructions per word (LOP3, IMAD, LOP3, SHF, IDP.4A, ATOMS).
-// acc collects 128 x the sum of the passing qualities (the 0x80 flags are the dot-product weights).
-template <bool BQ_HI>
-__device__ __forceinline__ void count_chunk(const uint4 v, uint32_t dst, uint32_t t_low, uint32_t &acc) {
-    const uint32_t l0 = bytes_ge<BQ_HI>(v.x, t_low), l1 = bytes_ge<BQ_HI>(v.y, t_low);
-    const uint32_t l2 = bytes_ge<BQ_HI>(v.z, t_low), l3 = bytes_ge<BQ_HI>(v.w, t_low);
-    acc = __dp4a(v.x, l0, __dp4a(v.y, l1, __dp4a(v.z, l2, __dp4a(v.w, l3, acc))));
-    red_shared(dst, l0 >> 7); red_shared(dst + 4, l1 >> 7); red_shared(dst + 8, l2 >> 7); red_shared(dst + 12, l3 >> 7);
-}
-template <bool BQ_HI>
-__device__ __forceinline__ void chunk_plain(uint32_t src, uint32_t dst, uint32_t t_low, uint32_t &acc) {
-    count_chunk<BQ_HI>(lds128(src), dst, t_low, acc);
-}
-// First / last chunk of a segment: bytes outside [lo, hi) are taken out of the pass flags.
-template <bool BQ_HI>
-__device__ __forceinline__ void chunk_edge(uint32_t src, uint32_t dst, uint32_t lo, uint32_t hi, const uint4 *sMaskLo, const uint4 *sMaskHi,
-                                           uint32_t t_low, uint32_t &acc) {
-    const uint4 v = lds128(src);
-    const uint4 ml = sMaskLo[lo], mh = sMaskHi[hi];       // 0xFF in bytes outside [lo, hi)
-    const uint32_t l0 = bytes_ge<BQ_HI>(v.x, t_low) & ~(ml.x | mh.x), l1 = bytes_ge<BQ_HI>(v.y, t_low) & ~(ml.y | mh.y);
-    const uint32_t l2 = bytes_ge<BQ_HI>(v.z, t_low) & ~(ml.z | mh.z), l3 = bytes_ge<BQ_HI>(v.w, t_low) & ~(ml.w | mh.w);
-    acc = __dp4a(v.x, l0, __dp4a(v.y, l1, __dp4a(v.z, l2, __dp4a(v.w, l3, acc))));
-    red_shared(dst, l0 >> 7); red_shared(dst + 4, l1 >> 7); red_shared(dst + 8, l2 >> 7); red_shared(dst + 12, l3 >> 7);
-}
+__device__ __forceinline__ uint4 or4(const uint4 a, const uint4 b) { return make_uint4(a.x | b.x, a.y | b.y, a.z | b.z, a.w | b.w); }
 
-// First chunk of a segment of two or more chunks (bytes below lo are not part of it) / its last chunk (bytes from hi on are not):
-// one mask load each instead of the two of chunk_edge.
+// One 16-byte chunk: pass flags of the bytes not in drop (0xFF in bytes outside the segment), acc += 128 x the sum of the
+// passing qualities (the 0x80 flags are the dot-product weights), the four flag words added to dst .. dst + 12.  An interior
+// chunk passes a zero drop mask: 6 instructions per word (LOP3, IMAD, LOP3, SHF, IDP.4A, ATOMS).
 template <bool BQ_HI>
-__device__ __forceinline__ void chunk_first(uint32_t src, uint32_t dst, uint32_t lo, const uint4 *sMaskLo, uint32_t t_low, uint32_t &acc) {
-    const uint4 v = lds128(src);
-    const uint4 ml = sMaskLo[lo];
-    const uint32_t l0 = bytes_ge<BQ_HI>(v.x, t_low) & ~ml.x, l1 = bytes_ge<BQ_HI>(v.y, t_low) & ~ml.y;
-    const uint32_t l2 = bytes_ge<BQ_HI>(v.z, t_low) & ~ml.z, l3 = bytes_ge<BQ_HI>(v.w, t_low) & ~ml.w;
+__device__ __forceinline__ void count_words(const uint4 v, const uint4 drop, uint32_t dst, uint32_t t_low, uint32_t &acc) {
+    const uint32_t l0 = bytes_ge<BQ_HI>(v.x, t_low) & ~drop.x, l1 = bytes_ge<BQ_HI>(v.y, t_low) & ~drop.y;
+    const uint32_t l2 = bytes_ge<BQ_HI>(v.z, t_low) & ~drop.z, l3 = bytes_ge<BQ_HI>(v.w, t_low) & ~drop.w;
     acc = __dp4a(v.x, l0, __dp4a(v.y, l1, __dp4a(v.z, l2, __dp4a(v.w, l3, acc))));
     red_shared(dst, l0 >> 7); red_shared(dst + 4, l1 >> 7); red_shared(dst + 8, l2 >> 7); red_shared(dst + 12, l3 >> 7);
-}
-template <bool BQ_HI>
-__device__ __forceinline__ void chunk_last(uint32_t src, uint32_t dst, uint32_t hi, const uint4 *sMaskHi, uint32_t t_low, uint32_t &acc) {
-    chunk_first<BQ_HI>(src, dst, hi, sMaskHi, t_low, acc);
 }
 
 // Stream one M-segment: qs = byte offset of its first quality inside the stage (the stage keeps the 16-byte phase of
 // the global column), len bases, rrel = window entry of the first base.  Entry e of class a lives at byte e + 16 - a of
 // array a, so a chunk whose byte 0 is entry e0 adds its four words to words (e0 >> 2) + 4 .. + 7 of array e0 & 3.
+// A segment of two or more chunks needs one mask for its first chunk (bytes below head) and one for its last.
 template <bool BQ_HI>
 __device__ __forceinline__ void stream_segment(uint32_t stage_s, uint32_t sC_s, uint32_t qs, uint32_t len, uint32_t rrel,
                                                const uint4 *sMaskLo, const uint4 *sMaskHi, uint32_t t_low, uint32_t &acc) {
+    const uint4 none = make_uint4(0, 0, 0, 0);
     const uint32_t head = qs & 15u;
     const uint32_t nc = (head + len + 15u) >> 4;
     uint32_t src = stage_s + (qs & ~15u);
     const int e0 = (int)rrel - (int)head;                                  // >= -15
     uint32_t dst = sC_s + ((uint32_t)e0 & 3u) * (uint32_t)(F_CW * 4) + (uint32_t)(((e0 >> 2) + 4) * 4);
-    if (nc == 1u) { chunk_edge<BQ_HI>(src, dst, head, head + len, sMaskLo, sMaskHi, t_low, acc); return; }
-    chunk_first<BQ_HI>(src, dst, head, sMaskLo, t_low, acc);
+    if (nc == 1u) { count_words<BQ_HI>(lds128(src), or4(sMaskLo[head], sMaskHi[head + len]), dst, t_low, acc); return; }
+    count_words<BQ_HI>(lds128(src), sMaskLo[head], dst, t_low, acc);
     uint32_t n_int = nc - 2u;                                              // interior chunks: no masks
     src += 16; dst += 16;
 #pragma unroll 1
     for (; n_int >= 2u; n_int -= 2u) {
         const uint4 v0 = lds128(src), v1 = lds128(src + 16);               // both loads in flight before the first count
-        count_chunk<BQ_HI>(v0, dst, t_low, acc); count_chunk<BQ_HI>(v1, dst + 16, t_low, acc);
+        count_words<BQ_HI>(v0, none, dst, t_low, acc); count_words<BQ_HI>(v1, none, dst + 16, t_low, acc);
         src += 32; dst += 32;
     }
-    if (n_int) { chunk_plain<BQ_HI>(src, dst, t_low, acc); src += 16; dst += 16; }
-    chunk_last<BQ_HI>(src, dst, head + len - 16u * (nc - 1u), sMaskHi, t_low, acc);
+    if (n_int) { count_words<BQ_HI>(lds128(src), none, dst, t_low, acc); src += 16; dst += 16; }
+    count_words<BQ_HI>(lds128(src), sMaskHi[head + len - 16u * (nc - 1u)], dst, t_low, acc);
 }
 
 // Same from global memory (the few second-and-later M-segments of a window: their qualities are in L2, one 16-byte
@@ -179,15 +148,9 @@ __device__ __forceinline__ void stream_segment_global(const uint8_t *src0, uint3
     const uint32_t dst0 = sC_s + ((uint32_t)e0 & 3u) * (uint32_t)(F_CW * 4) + (uint32_t)(((e0 >> 2) + 4) * 4);
 #pragma unroll 1
     for (uint32_t c = c_first; c < nc; c += c_step) {              // the caller spreads the chunks of a segment over c_step threads
-        const uint32_t dst = dst0 + 16u * c;
         if (!CLB_GMEM_OK(src + c, q_lo, q_hi)) continue;
-        const uint4 v = ldg_stream(src + c);
         const uint32_t lo = c == 0 ? head : 0u, hi = min(16u, head + len - 16u * c);
-        const uint4 ml = sMaskLo[lo], mh = sMaskHi[hi];
-        const uint32_t l0 = bytes_ge<BQ_HI>(v.x, t_low) & ~(ml.x | mh.x), l1 = bytes_ge<BQ_HI>(v.y, t_low) & ~(ml.y | mh.y);
-        const uint32_t l2 = bytes_ge<BQ_HI>(v.z, t_low) & ~(ml.z | mh.z), l3 = bytes_ge<BQ_HI>(v.w, t_low) & ~(ml.w | mh.w);
-        acc = __dp4a(v.x, l0, __dp4a(v.y, l1, __dp4a(v.z, l2, __dp4a(v.w, l3, acc))));
-        red_shared(dst, l0 >> 7); red_shared(dst + 4, l1 >> 7); red_shared(dst + 8, l2 >> 7); red_shared(dst + 12, l3 >> 7);
+        count_words<BQ_HI>(ldg_stream(src + c), or4(sMaskLo[lo], sMaskHi[hi]), dst0 + 16u * c, t_low, acc);
     }
 }
 
@@ -219,13 +182,8 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     const ulonglong2 wq = *reinterpret_cast<const ulonglong2 *>(P.win_rec + 3 * (size_t)w + 1);
     const uint32_t G = wg.x;
     if (G == 0) return;
-    if (*P.err & (ERR_UNSORTED | ERR_OFFSETS)) return;                     // k_validate_batch refused the columns: do not walk them
-#ifdef CLB_PHASE_TIMING      // developer builds only (scripts/phase_timing.py)
-#define CLB_FSTAMP(i) do { if (P.timing && threadIdx.x == 0) P.timing[(size_t)w * 8 + (i)] = clock64(); } while (0)
-#else
-#define CLB_FSTAMP(i) do { } while (0)
-#endif
-    CLB_FSTAMP(0);
+    if (*P.err & ERR_INPUT_REFUSED) return;                                // do not walk refused columns
+    CLB_STAMP(0);
 
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_A);
     uint32_t *sC = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_C);
@@ -274,7 +232,7 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
         if (lane == 0) mbar_init(bar, 1);
     }
     __syncthreads();
-    CLB_FSTAMP(1);
+    CLB_STAMP(1);
     if (j < n_sub) fmeta_ops(P, M);
 
     const uint32_t t_low = (P.min_bq & 0x7fu) * 0x01010101u;
@@ -346,15 +304,15 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
             }
         }
         // this warp's next sub-batch: its columns are in flight while the current one is streamed
-        if (j == 0) CLB_FSTAMP(2);
+        if (j == 0) CLB_STAMP(2);
         const bool has_next = j + NWARPS < n_sub;
         if (has_next) fmeta_load(P, M, min(r_lo + (j + NWARPS) * G + (uint32_t)lane, r_hi - 1u), wq.x);
         if (fits && bytes) { mbar_wait(bar, parity); parity ^= 1u; }       // the staged qualities have landed
-        if (j == 0) CLB_FSTAMP(3);
+        if (j == 0) CLB_STAMP(3);
         if (has_next) fmeta_ops(P, M);
         // ---------------------------------------------------------------- phase B: stream from shared memory
         if (has0 && fits) stream_segment<BQ_HI>(stage_s, sC_s, s_qs, s_len, s_rr, sMaskLo, sMaskHi, t_low, acc128);
-        if (j == 0) CLB_FSTAMP(4);
+        if (j == 0) CLB_STAMP(4);
         acc_sum += acc128 >> 7; acc128 = 0;                                // at most 2047 bases x 255 x 128 per sub-batch: no overflow
     }
     __syncthreads();                                                       // every warp's pushes / counters
@@ -377,7 +335,7 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
         }
     }
 
-    CLB_FSTAMP(5);
+    CLB_STAMP(5);
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert(PPT == 8, "phase C of the fast kernel is written for 8 entries per thread");
     uint32_t a[PPT], qcv[PPT];
@@ -413,150 +371,22 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
         for (int k = 0; k < PPT; k++) a[k] += oa;
     }
     const uint32_t nbits = __funnelshift_r(nm0, nm1, (wb0 + ebase) & 31u);
-    const uint32_t k_end = n_ent > ebase ? min((uint32_t)PPT, n_ent - ebase) : 0u;
-    const uint32_t vmask = (1u << k_end) - 1u;                              // entries this thread reports
-    uint32_t stp = 0;                                                       // 4 bits of state per entry
-    uint32_t cnt_pack = 0, covered = 0, sraw = 0, sqc = 0;
-    const uint32_t min_dflm = P.min_depth_for_low_mapq, min_depth = P.min_depth;
-    const uint32_t max_depth = P.max_depth ? P.max_depth : 0xffffffffu;    // max_depth == 0 disables EXCESSIVE_COVERAGE
+    Entries<uint32_t> e = entries_of<uint32_t>(ebase, 0u, n_ent);          // no halo entry
+    const StateLimits lim = state_limits(P);
 #pragma unroll
     for (int k = 0; k < PPT; k++) {
-        const uint32_t raw = a[k] & 0xffffu, low = a[k] >> 16;
-        const uint32_t qc = qcv[k];
-        const uint32_t fst = sFirst[raw];                                   // one byte per depth: raw <= 254 (depth proof)
-        const bool is_low = raw >= min_dflm && low >= fst;
-        uint32_t s = qc > max_depth ? ST_EXCESSIVE : ST_CALLABLE;
-        s = qc < min_depth ? ST_LOW_COVERAGE : s;
-        s = is_low ? ST_POOR_MAPQ : s;
-        s = raw == 0 ? ST_NO_COVERAGE : s;
-        s = ((nbits >> k) & 1u) ? ST_REF_N : s;
-        stp |= s << (4 * k);
-        cnt_pack += 1u << (5 * s);
-        covered += raw > 0 ? 1u : 0u;
-        sraw += raw; sqc += qc;
+        const uint32_t raw = a[k] & 0xffffu;
+        classify_entry(e, k, raw, a[k] >> 16, qcv[k], sFirst[raw], (nbits >> k) & 1u, lim);   // one byte per depth: raw <= 254 (depth proof)
     }
-    constexpr uint32_t ALL_ENTRIES = (1u << PPT) - 1u;
-    if (vmask != ALL_ENTRIES) {
-        // entries past the region end carry no depth (reads are clipped there) but were counted as states: take them out
-        uint32_t inv = ~vmask & ALL_ENTRIES;
-        while (inv) {
-            const int k = __ffs(inv) - 1; inv &= inv - 1;
-            cnt_pack -= 1u << (5 * ((stp >> (4 * k)) & 15u));
-        }
-    }
-    if (DBG && P.dbg_raw) {
-#pragma unroll
-        for (int k = 0; k < PPT; k++) if ((vmask >> k) & 1u) {
-            const uint32_t o = wb0 + ebase + k - P.region_start;
-            P.dbg_raw[o] = a[k] & 0xffffu; P.dbg_qc[o] = qcv[k]; P.dbg_low[o] = a[k] >> 16; P.dbg_state[o] = (uint8_t)((stp >> (4 * k)) & 15u);
-        }
-    }
-    sLast[tid] = (uint8_t)(stp >> (4 * (PPT - 1)));
-    if (k_end && ebase + k_end == n_ent) sScan[3 * NWARPS + 1] = (stp >> (4 * (k_end - 1))) & 15u;   // state of the window's last position
-    {
-        uint32_t v[10];
-#pragma unroll
-        for (int s = 0; s < 6; s++) v[s] = (cnt_pack >> (5 * s)) & 31u;
-        v[6] = covered; v[7] = sraw; v[8] = acc_sum; v[9] = sqc;
-#pragma unroll
-        for (int i = 0; i < 10; i++) v[i] = __reduce_add_sync(FULL, v[i]);
-        const uint32_t mqs = __reduce_add_sync(FULL, acc_mapq), bqs = v[8];
-        if (lane == 0) {
-            unsigned long long *ws = sWStats + warp * N_STATS;
-#pragma unroll
-            for (int s = 0; s < 6; s++) ws[S_COUNT0 + s] = v[s];
-            ws[S_COVERED] = v[6]; ws[S_SUMCOV] = v[7]; ws[S_SUMBQ] = bqs; ws[S_QBASES] = v[9];
-            ws[S_RESERVED] = 0; ws[S_SUMMAPQ] = mqs;
-        }
-    }
-    __syncthreads();
-    if (tid < N_STATS) {
-        unsigned long long t = 0;
-#pragma unroll
-        for (int j = 0; j < NWARPS; j++) t += sWStats[j * N_STATS + tid];
-        if (t) atomicAdd(&P.stats[tid * STAT_STRIDE], t);
-    }
-    // run boundaries: entry e starts a run iff its state differs from entry e - 1; entry 0 always does (window soft)
-    uint32_t bmask;
-    {
-        const uint32_t prev_last = tid > 0 ? sLast[tid - 1] : ((stp & 15u) ^ 1u);
-        const uint32_t shifted = (stp << 4) | prev_last;
-        uint32_t diff = stp ^ shifted;
-        diff |= diff >> 1; diff |= diff >> 2;
-        bmask = 0;
-#pragma unroll
-        for (int k = 0; k < PPT; k++) bmask |= ((diff >> (4 * k)) & 1u) << k;
-        bmask &= vmask;
-    }
-    {
-        const uint32_t nb = __popc(bmask);
-        uint32_t inb = nb;
-#pragma unroll
-        for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inb, dd); if (lane >= dd) inb += t; }
-        if (lane == 31) sScan[2 * NWARPS + warp] = inb;
-        __syncthreads();
-        const uint32_t wt = lane < NWARPS ? sScan[2 * NWARPS + lane] : 0u;
-        const uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
-        if (tid == 0) {
-            const uint32_t base = atomicAdd(P.rec_cursor, total);           // total >= 1
-            sScan[3 * NWARPS] = base;
-            P.win_tab[w] = make_uint2(base, pack_win_y(total, stp & 15u, w > 0 ? 1u : 0u, sScan[3 * NWARPS + 1]));
-            if ((unsigned long long)base + total > P.rec_cap) atomicOr(P.err, ERR_REC_OVERFLOW);
-        }
-        __syncthreads();
-        uint32_t o = sScan[3 * NWARPS] + off;
-        uint32_t m = bmask;
-        while (m) {
-            const int k = __ffs(m) - 1; m &= m - 1;
-            const uint32_t s = (stp >> (4 * k)) & 15u;
-            const bool wsoft = w > 0 && tid == 0 && k == 0;
-            if (o < P.rec_cap)
-                P.rec[o] = (unsigned long long)(wb0 + ebase + k) | ((unsigned long long)s << 32)
-                         | ((unsigned long long)(wsoft ? 1u : 0u) << 41);
-            o++;
-        }
-    }
-    // bins: positions of CALLABLE / POOR_MAPPING_QUALITY / REF_N per stride-sized bin
-    if (P.n_bins) {
-        const uint32_t c_call = (cnt_pack >> (5 * ST_CALLABLE)) & 31u, c_poor = (cnt_pack >> (5 * ST_POOR_MAPQ)) & 31u, c_refn = cnt_pack & 31u;
-        const uint32_t we0 = (uint32_t)(warp * 32 * PPT), we1 = min(n_ent, (uint32_t)((warp + 1) * 32 * PPT));
-        if (we1 > we0) {                                                   // warp-uniform
-            const uint32_t fb = wr.z, nbe = wr.w - 1u;                     // first bin; entry where the next bin starts (k_window_ranges counts from the halo)
-            uint32_t wbin0, wbin1;
-            if (we1 <= nbe) { wbin0 = wbin1 = fb; }
-            else if (we0 >= nbe && we1 - nbe <= P.stride) { wbin0 = wbin1 = fb + 1; }
-            else { wbin0 = (wb0 + we0) / P.stride; wbin1 = (wb0 + we1 - 1) / P.stride; }
-            if (wbin0 == wbin1) {
-                const uint32_t s0 = __reduce_add_sync(FULL, c_call), s1 = __reduce_add_sync(FULL, c_poor), s2 = __reduce_add_sync(FULL, c_refn);
-                if (lane == 0) {
-                    if (s0) atomicAdd(&P.bins[wbin0], (unsigned long long)s0);
-                    if (s1) atomicAdd(&P.bins[P.n_bins + wbin0], (unsigned long long)s1);
-                    if (s2) atomicAdd(&P.bins[2 * P.n_bins + wbin0], (unsigned long long)s2);
-                }
-            } else if (k_end) {
-                const uint32_t tb0 = (wb0 + ebase) / P.stride, tb1 = (wb0 + ebase + k_end - 1) / P.stride;
-                if (tb0 == tb1) {
-                    if (c_call) atomicAdd(&P.bins[tb0], (unsigned long long)c_call);
-                    if (c_poor) atomicAdd(&P.bins[P.n_bins + tb0], (unsigned long long)c_poor);
-                    if (c_refn) atomicAdd(&P.bins[2 * P.n_bins + tb0], (unsigned long long)c_refn);
-                } else {
-#pragma unroll 1
-                    for (uint32_t k = 0; k < k_end; k++) {
-                        const uint32_t bi = (wb0 + ebase + k) / P.stride;
-                        const uint32_t s = (stp >> (4 * k)) & 15u;
-                        if (s == ST_CALLABLE) atomicAdd(&P.bins[bi], 1ull);
-                        else if (s == ST_POOR_MAPQ) atomicAdd(&P.bins[P.n_bins + bi], 1ull);
-                        else if (s == ST_REF_N) atomicAdd(&P.bins[2 * P.n_bins + bi], 1ull);
-                    }
-                }
-            }
-        }
-    }
-    CLB_FSTAMP(6);
-#ifdef CLB_PHASE_TIMING
-    if (P.timing && tid == 0) P.timing[(size_t)w * 8 + 7] = (long long)(r_hi - r_lo);
-#endif
-#undef CLB_FSTAMP
+    close_entries(e, n_ent, sLast, sScan);
+    dbg_dump<DBG>(e, w * (uint32_t)WREAL, [&](int k) { return make_uint3(a[k] & 0xffffu, qcv[k], a[k] >> 16); }, P);
+    reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
+    // the window's first position always starts a record (window soft: the interval gather drops it when the previous
+    // window ended in the same state)
+    write_records(e, wb0, 0u, 0u, w > 0 ? 1u : 0u, sLast, sScan, w, P);
+    add_bins(e, wb0, 0u, n_ent, wr.z, wr.w - 1u, P);                       // k_window_ranges counts the next bin's entry from the halo
+    CLB_STAMP(6);
+    CLB_STAMP_VALUE(7, r_hi - r_lo);
 }
 
 }  // namespace clb

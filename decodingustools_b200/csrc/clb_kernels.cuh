@@ -53,9 +53,11 @@ constexpr int STAT_STRIDE = 16;       // one 128-byte line per global counter (u
 enum { ST_REF_N = 0, ST_CALLABLE = 1, ST_NO_COVERAGE = 2, ST_LOW_COVERAGE = 3, ST_EXCESSIVE = 4, ST_POOR_MAPQ = 5 };
 enum { S_COUNT0 = 0, S_COVERED = 6, S_SUMCOV = 7, S_SUMBQ = 8, S_SUMMAPQ = 9, S_QBASES = 10, S_RESERVED = 11, N_STATS = 12 };
 enum { ERR_QUAL_SPAN = 1, ERR_REC_OVERFLOW = 2, ERR_UNSORTED = 8, ERR_OFFSETS = 16 };
-// the kernels after the pileup do not touch win_tab / rec once one of these is set: k_validate_batch refused the columns (the
-// pileup kernels returned before writing win_tab[w]) or a window could not be run; the host reports the error instead
-constexpr uint32_t ERR_RESULT_INVALID = ERR_UNSORTED | ERR_OFFSETS | ERR_QUAL_SPAN;
+// k_validate_batch refused the columns: the pileup kernels do not walk them and return before writing win_tab[w]
+constexpr uint32_t ERR_INPUT_REFUSED = ERR_UNSORTED | ERR_OFFSETS;
+// the kernels after the pileup do not touch win_tab / rec once one of these is set: the input was refused or a window could
+// not be run; the host reports the error instead
+constexpr uint32_t ERR_RESULT_INVALID = ERR_INPUT_REFUSED | ERR_QUAL_SPAN;
 
 struct KParams {
     // packed read columns (device)
@@ -89,10 +91,10 @@ struct KParams {
     unsigned long long *stats;     // [N_STATS * STAT_STRIDE]
     unsigned long long *bins;      // [3][n_bins]
     uint32_t n_bins, stride;
-    unsigned long long *rec;       // boundary records: pos | state << 32 | soft << 40
+    unsigned long long *rec;       // boundary records (pack_rec)
     uint32_t rec_cap;
     uint32_t *rec_cursor;
-    uint2 *win_tab;                // per window: (first record, record count)
+    uint2 *win_tab;                // per window: (first record, pack_win_y word)
     uint32_t *err;
     uint32_t *deep_count, *deep_list;   // windows with more than 65535 candidate reads, left to k_pileup_classify_deep
     uint32_t *gen_list, *gen_count, *gen_taken;   // queue of general-path windows (k_pileup_general takes tickets)
@@ -102,6 +104,15 @@ struct KParams {
     uint8_t *dbg_state;
     long long *timing;             // optional (developer builds): 8 clock64 stamps per window
 };
+
+// Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
+// kernel with P and w in scope.  The stamps cost instruction-cache space, so production builds compile them out.
+#ifdef CLB_PHASE_TIMING
+#define CLB_STAMP_VALUE(i, v) do { if (P.timing && threadIdx.x == 0) P.timing[(size_t)w * 8 + (i)] = (long long)(v); } while (0)
+#else
+#define CLB_STAMP_VALUE(i, v) do { } while (0)
+#endif
+#define CLB_STAMP(i) CLB_STAMP_VALUE(i, clock64())
 
 // One bulk L2 prefetch of bytes [lo, hi) of a device array (rounded out to 16 bytes: allocations are 256-byte granular).
 __device__ __forceinline__ void l2_prefetch(const void *base, uint64_t lo, uint64_t hi, uint32_t max_bytes) {
@@ -435,6 +446,230 @@ constexpr size_t WIN_TABLE_BYTES = 2 * 17 * 16 + NFIRST * 4 + NRCP * 4;   // sMa
 static_assert(WIN_TABLE_BYTES % 16 == 0, "window tables are copied with 16-byte loads");
 static_assert(SMEM_COUNTER_WORDS % 4 == 0 && LQ_SLAB % 4 == 0, "counter region is zeroed with 16-byte stores");
 
+// ---------------------------------------------------------------------------------------------
+// What a window leaves for the interval compaction: records of its run starts and one window-table word
+// ---------------------------------------------------------------------------------------------
+struct IntervalOut { uint32_t start, end; uint8_t state, soft; uint16_t pad; };
+
+// Boundary record: position where a run starts | its state << 32 | soft << 40 (the run merely continues the previous shard's).
+__device__ __forceinline__ unsigned long long pack_rec(uint32_t pos, uint32_t state, uint32_t soft) {
+    return (unsigned long long)pos | ((unsigned long long)state << 32) | ((unsigned long long)soft << 40);
+}
+__device__ __forceinline__ IntervalOut unpack_rec(unsigned long long r) {        // end: filled in by k_fill_ends
+    IntervalOut iv; iv.start = (uint32_t)r; iv.end = 0; iv.state = (uint8_t)(r >> 32); iv.soft = (uint8_t)((r >> 40) & 1u); iv.pad = 0;
+    return iv;
+}
+
+// Window table word y: record count | state of entry 0 << 12 | window soft << 16 | state of the last entry << 20.
+// "Window soft": the first record was emitted for the window's first position whatever its state (k_pileup_fast has no halo
+// entry); the state of entry 0 is only read then.
+__device__ __forceinline__ uint32_t pack_win_y(uint32_t count, uint32_t first_state, uint32_t wsoft, uint32_t last_state) {
+    return count | (first_state << 12) | (wsoft << 16) | (last_state << 20);
+}
+__device__ __forceinline__ uint32_t win_count(uint32_t y) { return y & 0xfffu; }
+// Records a window contributes to the sorted interval list: its count, minus the window-soft first record when the previous
+// window ended in the same state.
+__device__ __forceinline__ uint32_t win_drop_first(const uint2 *win_tab, uint32_t w) {
+    const uint32_t y = win_tab[w].y;
+    if (!((y >> 16) & 1u) || w == 0) return 0u;
+    return ((y >> 12) & 15u) == ((win_tab[w - 1].y >> 20) & 15u) ? 1u : 0u;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Phase C of both pileup kernels (k_pileup_fast, pileup_classify_window): classify the scanned depths, reduce the counters,
+// write the run boundaries and the bins.  Thread t holds window entries t * PPT .. t * PPT + PPT - 1.
+// ---------------------------------------------------------------------------------------------
+using stp_t = typename std::conditional<(PPT > 8), unsigned long long, uint32_t>::type;
+
+// One thread's entries.  Those outside [k_first, k_end) are classified with the rest but do not belong to the window: the
+// general kernel's halo (entry 0 of thread 0) and entries past the region end.  Sum: the type of the depth sums (64 bits
+// in deep windows, where 32-bit partial sums could overflow).
+template <typename Sum>
+struct Entries {
+    uint32_t ebase, k_first, k_end, vmask;   // vmask: bits [k_first, k_end)
+    stp_t stp;                               // 4 bits of state per entry
+    uint32_t cnt_pack, covered;              // entries per state (5 bits each), entries with raw depth > 0
+    Sum sraw, sqc;
+    __device__ __forceinline__ uint32_t state(int k) const { return (uint32_t)(stp >> (4 * k)) & 15u; }
+};
+template <typename Sum>
+__device__ __forceinline__ Entries<Sum> entries_of(uint32_t ebase, uint32_t k_first, uint32_t n_ent) {
+    Entries<Sum> e;
+    e.ebase = ebase; e.k_first = k_first;
+    e.k_end = n_ent > ebase ? min((uint32_t)PPT, n_ent - ebase) : 0u;
+    e.vmask = ((1u << e.k_end) - 1u) & ~((1u << k_first) - 1u);          // k_end >= k_first: a window has >= 2 entries
+    e.stp = 0; e.cnt_pack = 0; e.covered = 0; e.sraw = 0; e.sqc = 0;
+    return e;
+}
+
+// The options' depth thresholds, read once per window
+struct StateLimits { uint32_t min_depth_for_low_mapq, min_depth, max_depth; };
+__device__ __forceinline__ StateLimits state_limits(const KParams &P) {
+    return StateLimits{P.min_depth_for_low_mapq, P.min_depth, P.max_depth ? P.max_depth : 0xffffffffu};   // max_depth == 0 disables EXCESSIVE_COVERAGE
+}
+
+// State of entry k (callable_profiler.rs:89-120).  fst: the smallest low-MAPQ depth that makes raw depth POOR_MAPPING_QUALITY.
+template <typename Sum>
+__device__ __forceinline__ void classify_entry(Entries<Sum> &e, int k, uint32_t raw, uint32_t low, uint32_t qc, uint32_t fst, uint32_t ref_n,
+                                               const StateLimits &lim) {
+    const bool is_low = raw >= lim.min_depth_for_low_mapq && low >= fst;
+    uint32_t s = qc > lim.max_depth ? ST_EXCESSIVE : ST_CALLABLE;
+    s = qc < lim.min_depth ? ST_LOW_COVERAGE : s;
+    s = is_low ? ST_POOR_MAPQ : s;
+    s = raw == 0 ? ST_NO_COVERAGE : s;
+    s = ref_n ? ST_REF_N : s;
+    e.stp |= (stp_t)s << (4 * k);
+    e.cnt_pack += 1u << (5 * s);
+    e.covered += raw > 0 ? 1u : 0u;
+    e.sraw += raw; e.sqc += qc;
+}
+
+// Entries outside [k_first, k_end) were counted as states: take them out again.  Then publish what the boundary pass reads
+// from other threads: the state of this thread's last entry and that of the window's last position.
+template <typename Sum>
+__device__ __forceinline__ void close_entries(Entries<Sum> &e, uint32_t n_ent, uint8_t *sLast, uint32_t *sScan) {
+    uint32_t inv = ~e.vmask & ((1u << PPT) - 1u);
+    while (inv) {
+        const int k = __ffs(inv) - 1; inv &= inv - 1;
+        e.cnt_pack -= 1u << (5 * e.state(k));
+    }
+    sLast[threadIdx.x] = (uint8_t)e.state(PPT - 1);
+    if (e.k_end > e.k_first && e.ebase + e.k_end == n_ent) sScan[3 * NWARPS + 1] = e.state(e.k_end - 1);
+}
+
+// Per-base dump for the parity tests (own instantiation).  o0: offset of entry 0 from the region start; entry(k) = (raw, qc, low).
+template <bool DBG, typename Sum, typename Entry>
+__device__ __forceinline__ void dbg_dump(const Entries<Sum> &e, uint32_t o0, Entry entry, const KParams &P) {
+    if (DBG && P.dbg_raw) {
+#pragma unroll
+        for (int k = 0; k < PPT; k++) if ((e.vmask >> k) & 1u) {
+            const uint3 v = entry(k);
+            const uint32_t o = o0 + e.ebase + k;
+            P.dbg_raw[o] = v.x; P.dbg_qc[o] = v.y; P.dbg_low[o] = v.z; P.dbg_state[o] = (uint8_t)e.state(k);
+        }
+    }
+}
+
+__device__ __forceinline__ uint32_t warp_sum(uint32_t v) { return __reduce_add_sync(FULL, v); }
+__device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
+#pragma unroll
+    for (int dd = 16; dd > 0; dd >>= 1) v += __shfl_xor_sync(FULL, v, dd);
+    return v;
+}
+
+// Counters: per-warp sums in plain stores (no 64-bit shared atomics), summed after a barrier into one global atomic per
+// counter.  acc_sum / acc_mapq: the thread's base-quality and MAPQ sums (MapqSum: 64 bits unless the window's sum fits 32).
+template <typename Sum, typename MapqSum>
+__device__ __forceinline__ void reduce_stats(const Entries<Sum> &e, uint32_t acc_sum, MapqSum acc_mapq, unsigned long long *sWStats,
+                                             const KParams &P) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint32_t v[7];
+#pragma unroll
+    for (int s = 0; s < 6; s++) v[s] = (e.cnt_pack >> (5 * s)) & 31u;
+    v[6] = e.covered;
+#pragma unroll
+    for (int i = 0; i < 7; i++) v[i] = __reduce_add_sync(FULL, v[i]);
+    const Sum sraw = warp_sum(e.sraw), sqc = warp_sum(e.sqc), sbq = warp_sum((Sum)acc_sum);
+    const MapqSum smq = warp_sum(acc_mapq);
+    if (lane == 0) {
+        unsigned long long *ws = sWStats + warp * N_STATS;
+#pragma unroll
+        for (int s = 0; s < 6; s++) ws[S_COUNT0 + s] = v[s];
+        ws[S_COVERED] = v[6]; ws[S_SUMCOV] = sraw; ws[S_SUMBQ] = sbq; ws[S_QBASES] = sqc;
+        ws[S_RESERVED] = 0; ws[S_SUMMAPQ] = smq;
+    }
+    __syncthreads();
+    if (tid < N_STATS) {
+        unsigned long long t = 0;
+#pragma unroll
+        for (int j = 0; j < NWARPS; j++) t += sWStats[j * N_STATS + tid];
+        if (t) atomicAdd(&P.stats[tid * STAT_STRIDE], t);
+    }
+}
+
+// Run boundaries -> records.  Entry k starts a run iff its state differs from entry k - 1's; thread 0's entry 0 always does.
+// The entries in force start a record regardless; those in soft (a subset of force) that merely continue a run are flagged
+// soft.  pos0: position of entry 0; win_soft: see pack_win_y.
+template <typename Sum>
+__device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t pos0, uint32_t force, uint32_t soft, uint32_t win_soft,
+                                              const uint8_t *sLast, uint32_t *sScan, uint32_t w, const KParams &P) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint32_t bmask, softmask;
+    {
+        const uint32_t prev_last = tid > 0 ? sLast[tid - 1] : 0xfu;       // no state is 15
+        const stp_t shifted = (e.stp << 4) | (stp_t)prev_last;            // state of entry k-1 in nibble k
+        stp_t diff = e.stp ^ shifted;                                      // non-zero nibble <=> boundary
+        diff |= diff >> 1; diff |= diff >> 2;                              // bit 4k collects the nibble
+        bmask = 0;
+#pragma unroll
+        for (int k = 0; k < PPT; k++) bmask |= ((uint32_t)(diff >> (4 * k)) & 1u) << k;
+        softmask = soft & ~bmask;
+        bmask = (bmask | force) & e.vmask;
+    }
+    const uint32_t nb = __popc(bmask);
+    uint32_t inb = nb;
+#pragma unroll
+    for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inb, dd); if (lane >= dd) inb += t; }
+    if (lane == 31) sScan[2 * NWARPS + warp] = inb;
+    __syncthreads();
+    const uint32_t wt = lane < NWARPS ? sScan[2 * NWARPS + lane] : 0u;             // lane j: boundaries in warp j
+    const uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
+    if (tid == 0) {
+        const uint32_t base = atomicAdd(P.rec_cursor, total);                 // total may be 0 (general kernel): base is not read then
+        sScan[3 * NWARPS] = base;
+        P.win_tab[w] = make_uint2(base, pack_win_y(total, e.state(0), win_soft, sScan[3 * NWARPS + 1]));
+        if ((unsigned long long)base + total > P.rec_cap) atomicOr(P.err, ERR_REC_OVERFLOW);
+    }
+    __syncthreads();
+    uint32_t o = sScan[3 * NWARPS] + off;
+    uint32_t m = bmask;
+    while (m) {
+        const int k = __ffs(m) - 1; m &= m - 1;
+        if (o < P.rec_cap) P.rec[o] = pack_rec(pos0 + e.ebase + k, e.state(k), (softmask >> k) & 1u);
+        o++;
+    }
+}
+
+// Bins: positions of CALLABLE / POOR_MAPPING_QUALITY / REF_N per stride-sized bin.  pos0: position of entry 0; e_first: the
+// window's first own entry (1 with a halo, else 0); fb, nbe: the window's first bin and the entry where the next bin starts.
+template <typename Sum>
+__device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, uint32_t e_first, uint32_t n_ent, uint32_t fb, uint32_t nbe,
+                                         const KParams &P) {
+    if (!P.n_bins) return;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t c_call = (e.cnt_pack >> (5 * ST_CALLABLE)) & 31u, c_poor = (e.cnt_pack >> (5 * ST_POOR_MAPQ)) & 31u, c_refn = e.cnt_pack & 31u;
+    const uint32_t we0 = max(e_first, (uint32_t)(warp * 32 * PPT)), we1 = min(n_ent, (uint32_t)((warp + 1) * 32 * PPT));
+    if (we1 <= we0) return;                                                // warp-uniform
+    uint32_t wbin0, wbin1;
+    if (we1 <= nbe) { wbin0 = wbin1 = fb; }
+    else if (we0 >= nbe && we1 - nbe <= P.stride) { wbin0 = wbin1 = fb + 1; }
+    else { wbin0 = (pos0 + we0) / P.stride; wbin1 = (pos0 + we1 - 1) / P.stride; }
+    if (wbin0 == wbin1) {                                                  // whole warp inside one bin (the common case: stride >> 256)
+        const uint32_t s0 = __reduce_add_sync(FULL, c_call), s1 = __reduce_add_sync(FULL, c_poor), s2 = __reduce_add_sync(FULL, c_refn);
+        if (lane == 0) {
+            if (s0) atomicAdd(&P.bins[wbin0], (unsigned long long)s0);
+            if (s1) atomicAdd(&P.bins[P.n_bins + wbin0], (unsigned long long)s1);
+            if (s2) atomicAdd(&P.bins[2 * P.n_bins + wbin0], (unsigned long long)s2);
+        }
+    } else if (e.k_end > e.k_first) {
+        const uint32_t tb0 = (pos0 + e.ebase + e.k_first) / P.stride, tb1 = (pos0 + e.ebase + e.k_end - 1) / P.stride;
+        if (tb0 == tb1) {
+            if (c_call) atomicAdd(&P.bins[tb0], (unsigned long long)c_call);
+            if (c_poor) atomicAdd(&P.bins[P.n_bins + tb0], (unsigned long long)c_poor);
+            if (c_refn) atomicAdd(&P.bins[2 * P.n_bins + tb0], (unsigned long long)c_refn);
+        } else {
+#pragma unroll 1                                                // rare (a thread's entries straddle two bins): keep it small
+            for (uint32_t k = e.k_first; k < e.k_end; k++) {
+                const uint32_t bi = (pos0 + e.ebase + k) / P.stride;
+                const uint32_t s = e.state(k);
+                if (s == ST_CALLABLE) atomicAdd(&P.bins[bi], 1ull);
+                else if (s == ST_POOR_MAPQ) atomicAdd(&P.bins[P.n_bins + bi], 1ull);
+                else if (s == ST_REF_N) atomicAdd(&P.bins[2 * P.n_bins + bi], 1ull);
+            }
+        }
+    }
+}
+
 // One window.  WIDE = false packs the raw and low-MAPQ depths as 16 + 16 bits (windows with <= 65535 candidate reads, i.e.
 // practically all of them); WIDE = true keeps them in two 32-bit arrays and is only instantiated by k_pileup_classify_deep.
 template <bool BQ_HI, bool WIDE, bool DBG>
@@ -456,11 +691,6 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
 
     uint32_t *sLowD = reinterpret_cast<uint32_t *>(smem_raw + SMEM_BYTES);       // WIDE only
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-#ifdef CLB_PHASE_TIMING      // developer builds only (scripts/phase_timing.py): the stamps cost instruction-cache space
-#define CLB_STAMP(i) do { if (P.timing && tid == 0) P.timing[(size_t)w * 8 + (i)] = clock64(); } while (0)
-#else
-#define CLB_STAMP(i) do { } while (0)
-#endif
     CLB_STAMP(0);
 
     Win W;
@@ -718,15 +948,9 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
         if (p0 >= 0) { const uint32_t wi = (uint32_t)(p0 >> 5); nbits = __funnelshift_r(P.nmask[wi], P.nmask[wi + 1], (uint32_t)(p0 & 31)); }
         else nbits = P.nmask[0] << 1;
     }
-    const uint32_t k_first = ebase == 0 ? 1u : 0u;                       // entry 0 is the halo
-    const uint32_t k_end = n_ent > ebase ? min((uint32_t)PPT, n_ent - ebase) : 0u;
-    const uint32_t vmask = k_end > k_first ? (((1u << k_end) - 1u) & ~((1u << k_first) - 1u)) : 0u;   // entries this thread reports
-    using stp_t = typename std::conditional<(PPT > 8), unsigned long long, uint32_t>::type;
-    stp_t stp = 0;                                                         // 4 bits of state per entry
-    uint32_t cnt_pack = 0, covered = 0, sraw = 0, sqc = 0;
-    unsigned long long sraw_w = 0, sqc_w = 0;                              // deep windows: 32-bit partial sums could overflow
-    const uint32_t min_dflm = P.min_depth_for_low_mapq, min_depth = P.min_depth;
-    const uint32_t max_depth = P.max_depth ? P.max_depth : 0xffffffffu;   // max_depth == 0 disables EXCESSIVE_COVERAGE
+    using Sum = typename std::conditional<WIDE, unsigned long long, uint32_t>::type;   // deep windows: 32-bit partial sums could overflow
+    Entries<Sum> e = entries_of<Sum>(ebase, ebase == 0 ? 1u : 0u, n_ent);              // entry 0 is the halo
+    const StateLimits lim = state_limits(P);
     // Two copies of the per-entry classification, chosen per thread: when none of the thread's entries is deeper than
     // the shared-memory threshold table the lookup is a plain LDS; otherwise every entry may go to the global table
     // (kept apart because those loads, predicated off, would still cost six issue slots per ordinary entry).
@@ -743,17 +967,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
             } else {
                 fst = sFirst[raw];
             }
-            const bool is_low = raw >= min_dflm && low >= fst;
-            uint32_t s = qc > max_depth ? ST_EXCESSIVE : ST_CALLABLE;
-            s = qc < min_depth ? ST_LOW_COVERAGE : s;
-            s = is_low ? ST_POOR_MAPQ : s;
-            s = raw == 0 ? ST_NO_COVERAGE : s;
-            s = ((nbits >> k) & 1u) ? ST_REF_N : s;
-            stp |= (stp_t)s << (4 * k);
-            cnt_pack += 1u << (5 * s);
-            covered += raw > 0 ? 1u : 0u;
-            if (WIDE) { sraw_w += raw; sqc_w += qc; }
-            else { sraw += raw; sqc += qc; }
+            classify_entry(e, k, raw, low, qc, fst, (nbits >> k) & 1u, lim);
             b[k] = qc;                                                    // keep qc (entry 0 below, optional debug dump)
         }
     };
@@ -763,151 +977,25 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
         for (int k = 0; k < PPT; k++) deepest |= WIDE ? a[k] : a[k] & 0xffffu;
         if (deepest < (uint32_t)NFIRST) classify(std::false_type{}); else classify(std::true_type{});
     }
-    constexpr uint32_t ALL_ENTRIES = (1u << PPT) - 1u;
-    if (vmask != ALL_ENTRIES) {
-        // Few threads: the halo entry (thread 0) and entries past the region end were counted above; take them out again.
-        // Only entry 0 can carry depth (the halo is a real position); reads are clipped at the region end, so the
-        // entries past it have none.
-        uint32_t inv = ~vmask & ALL_ENTRIES;
-        if (inv & 1u) {
-            const uint32_t raw0 = WIDE ? a[0] : a[0] & 0xffffu;
-            covered -= raw0 > 0 ? 1u : 0u;
-            if (WIDE) { sraw_w -= raw0; sqc_w -= b[0]; } else { sraw -= raw0; sqc -= b[0]; }
-        }
-        while (inv) {
-            const int k = __ffs(inv) - 1; inv &= inv - 1;
-            cnt_pack -= 1u << (5 * ((uint32_t)(stp >> (4 * k)) & 15u));
-        }
+    if (!(e.vmask & 1u)) {
+        // the halo entry (thread 0) is a real position and carries depth: take it out of the sums again (reads are clipped
+        // at the region end, so entries past it have none)
+        const uint32_t raw0 = WIDE ? a[0] : a[0] & 0xffffu;
+        e.covered -= raw0 > 0 ? 1u : 0u; e.sraw -= raw0; e.sqc -= b[0];
     }
-    if (DBG && P.dbg_raw) {                                                // per-base dump for the parity tests (own instantiation)
-#pragma unroll
-        for (int k = 0; k < PPT; k++) if ((vmask >> k) & 1u) {
-            const uint32_t o = (uint32_t)(W.wb + (long long)(ebase + k) - P.region_start);
-            P.dbg_raw[o] = WIDE ? a[k] : a[k] & 0xffffu; P.dbg_qc[o] = b[k]; P.dbg_low[o] = WIDE ? lw[WIDE ? k : 0] : a[k] >> 16; P.dbg_state[o] = (uint8_t)((uint32_t)(stp >> (4 * k)) & 15u);
-        }
-    }
-    sLast[tid] = (uint8_t)((uint32_t)(stp >> (4 * (PPT - 1))) & 15u);
-    if (k_end > k_first && ebase + k_end == n_ent) sScan[3 * NWARPS + 1] = (uint32_t)(stp >> (4 * (k_end - 1))) & 15u;   // state of the window's last position
-    // per-warp partial sums of the additive counters (plain stores, summed after the barrier: no 64-bit smem atomics)
-    {
-        uint32_t v[10];
-#pragma unroll
-        for (int s = 0; s < 6; s++) v[s] = (cnt_pack >> (5 * s)) & 31u;
-        v[6] = covered; v[7] = sraw; v[8] = acc_sum; v[9] = sqc;
-#pragma unroll
-        for (int i = 0; i < 10; i++) v[i] = __reduce_add_sync(FULL, v[i]);
-        unsigned long long mqs = acc_mapq, bqs = acc_sum;
-#pragma unroll
-        for (int dd = 16; dd > 0; dd >>= 1) {
-            mqs += __shfl_xor_sync(FULL, mqs, dd);
-            if (WIDE) { sraw_w += __shfl_xor_sync(FULL, sraw_w, dd); sqc_w += __shfl_xor_sync(FULL, sqc_w, dd); bqs += __shfl_xor_sync(FULL, bqs, dd); }
-        }
-        if (lane == 0) {
-            unsigned long long *ws = sWStats + warp * N_STATS;
-#pragma unroll
-            for (int s = 0; s < 6; s++) ws[S_COUNT0 + s] = v[s];
-            ws[S_COVERED] = v[6]; ws[S_SUMCOV] = WIDE ? sraw_w : v[7]; ws[S_SUMBQ] = WIDE ? bqs : v[8]; ws[S_QBASES] = WIDE ? sqc_w : v[9];
-            ws[S_RESERVED] = 0; ws[S_SUMMAPQ] = mqs;
-        }
-    }
-    __syncthreads();
-    if (tid < N_STATS) {
-        unsigned long long t = 0;
-#pragma unroll
-        for (int j = 0; j < NWARPS; j++) t += sWStats[j * N_STATS + tid];
-        if (t) atomicAdd(&P.stats[tid * STAT_STRIDE], t);
-    }
+    close_entries(e, n_ent, sLast, sScan);
+    dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
+                  [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
+    reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
     CLB_STAMP(4);
-    // run boundaries: entry e starts a run iff its state differs from entry e-1 (the halo for e == 1); the first position
-    // of the region always does (soft when it merely continues the previous shard's run)
-    uint32_t bmask, softmask = 0;
-    {
-        const uint32_t prev_last = tid > 0 ? sLast[tid - 1] : 0xfu;
-        const stp_t shifted = (stp << 4) | (stp_t)prev_last;              // state of entry k-1 in nibble k
-        stp_t diff = stp ^ shifted;                                        // non-zero nibble <=> boundary
-        diff |= diff >> 1; diff |= diff >> 2;                              // bit 4k collects the nibble
-        bmask = 0;
-#pragma unroll
-        for (int k = 0; k < PPT; k++) bmask |= ((uint32_t)(diff >> (4 * k)) & 1u) << k;
-        if (w == 0 && tid == 0) {                                          // entry 1 of window 0 is the region's first position
-            if (!(bmask & 2u) && P.region_start != 0) softmask = 2u;
-            bmask |= 2u;
-        }
-        bmask &= vmask;
-    }
-    {
-        const uint32_t nb = __popc(bmask);
-        uint32_t inb = nb;
-#pragma unroll
-        for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inb, dd); if (lane >= dd) inb += t; }
-        if (lane == 31) sScan[2 * NWARPS + warp] = inb;
-        __syncthreads();
-        const uint32_t wt = lane < NWARPS ? sScan[2 * NWARPS + lane] : 0u;             // lane j: boundaries in warp j
-        const uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
-        if (tid == 0) {
-            const uint32_t base = total ? atomicAdd(P.rec_cursor, total) : 0u;
-            sScan[3 * NWARPS] = base;
-            P.win_tab[w] = make_uint2(base, total | (sScan[3 * NWARPS + 1] << 20));   // count | last state << 20 (see pack_win_y)
-            if (total && (unsigned long long)base + total > P.rec_cap) atomicOr(P.err, ERR_REC_OVERFLOW);
-        }
-        __syncthreads();
-        uint32_t o = sScan[3 * NWARPS] + off;
-        uint32_t m = bmask;
-        while (m) {
-            const int k = __ffs(m) - 1; m &= m - 1;
-            const uint32_t s = (uint32_t)(stp >> (4 * k)) & 15u;
-            if (o < P.rec_cap)
-                P.rec[o] = (unsigned long long)(uint32_t)(W.wb + (long long)(ebase + k)) | ((unsigned long long)s << 32)
-                         | ((unsigned long long)((softmask >> k) & 1u) << 40);
-            o++;
-        }
-    }
+    // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
+    // previous shard's run
+    const uint32_t region_first = w == 0 && tid == 0 ? 2u : 0u;
+    write_records(e, (uint32_t)W.wb, region_first, P.region_start != 0 ? region_first : 0u, 0u, sLast, sScan, w, P);
     CLB_STAMP(5);
-    // bins: positions of CALLABLE / POOR_MAPPING_QUALITY / REF_N per stride-sized bin
-    if (P.n_bins) {
-        const bool any = k_end > k_first;
-        const uint32_t c_call = (cnt_pack >> (5 * ST_CALLABLE)) & 31u, c_poor = (cnt_pack >> (5 * ST_POOR_MAPQ)) & 31u, c_refn = cnt_pack & 31u;
-        const uint32_t we0 = max(1u, (uint32_t)(warp * 32 * PPT)), we1 = min(n_ent, (uint32_t)((warp + 1) * 32 * PPT));
-        if (we1 > we0) {                                                   // warp-uniform
-            // the window's first bin and the entry where the next bin starts were divided out once by thread 0
-            const uint32_t fb = sCtl[10], nbe = sCtl[11];
-            uint32_t wbin0, wbin1;
-            if (we1 <= nbe) { wbin0 = wbin1 = fb; }
-            else if (we0 >= nbe && we1 - nbe <= P.stride) { wbin0 = wbin1 = fb + 1; }
-            else { wbin0 = (uint32_t)(W.wb + we0) / P.stride; wbin1 = (uint32_t)(W.wb + we1 - 1) / P.stride; }
-            if (wbin0 == wbin1) {        // whole warp inside one bin (the common case: stride >> 256)
-                const uint32_t s0 = __reduce_add_sync(FULL, c_call), s1 = __reduce_add_sync(FULL, c_poor), s2 = __reduce_add_sync(FULL, c_refn);
-                if (lane == 0) {
-                    if (s0) atomicAdd(&P.bins[wbin0], (unsigned long long)s0);
-                    if (s1) atomicAdd(&P.bins[P.n_bins + wbin0], (unsigned long long)s1);
-                    if (s2) atomicAdd(&P.bins[2 * P.n_bins + wbin0], (unsigned long long)s2);
-                }
-            } else if (any) {
-                const uint32_t tb0 = (uint32_t)(W.wb + ebase + k_first) / P.stride, tb1 = (uint32_t)(W.wb + ebase + k_end - 1) / P.stride;
-                if (tb0 == tb1) {
-                    if (c_call) atomicAdd(&P.bins[tb0], (unsigned long long)c_call);
-                    if (c_poor) atomicAdd(&P.bins[P.n_bins + tb0], (unsigned long long)c_poor);
-                    if (c_refn) atomicAdd(&P.bins[2 * P.n_bins + tb0], (unsigned long long)c_refn);
-                } else {
-#pragma unroll 1                                                // rare (a thread's entries straddle two bins): keep it small
-                    for (int k = 0; k < PPT; k++) {
-                        if ((uint32_t)k >= k_first && (uint32_t)k < k_end) {
-                            const uint32_t bi = (uint32_t)(W.wb + ebase + k) / P.stride;
-                            const uint32_t s = (uint32_t)(stp >> (4 * k)) & 15u;
-                            if (s == ST_CALLABLE) atomicAdd(&P.bins[bi], 1ull);
-                            else if (s == ST_POOR_MAPQ) atomicAdd(&P.bins[P.n_bins + bi], 1ull);
-                            else if (s == ST_REF_N) atomicAdd(&P.bins[2 * P.n_bins + bi], 1ull);
-                        }
-                    }
-                }
-            }
-        }
-    }
+    add_bins(e, (uint32_t)W.wb, 1u, n_ent, sCtl[10], sCtl[11], P);        // first bin, next bin's entry: divided out once by thread 0
     CLB_STAMP(6);
-#ifdef CLB_PHASE_TIMING
-    if (P.timing && tid == 0) { P.timing[(size_t)w * 8 + 7] = (long long)(r_hi - r_lo); }
-#endif
-#undef CLB_STAMP
+    CLB_STAMP_VALUE(7, r_hi - r_lo);
 }
 
 // General kernel: persistent CTAs take the windows queued by k_window_ranges / k_pileup_fast one ticket at a time.
@@ -917,7 +1005,7 @@ template <bool BQ_HI, bool DBG>
 __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P) {
     __shared__ uint32_t s_ticket;
     const uint32_t n = *P.gen_count;
-    const bool refused = (*P.err & (ERR_UNSORTED | ERR_OFFSETS)) != 0;   // k_validate_batch refused the columns: take the tickets, do not walk them
+    const bool refused = (*P.err & ERR_INPUT_REFUSED) != 0;             // take the tickets, do not walk the columns
     for (;;) {
         if (threadIdx.x == 0) {
             uint32_t t = atomicAdd(P.gen_taken, 1u);
@@ -1155,17 +1243,6 @@ __global__ void k_first_table(uint32_t *first_tab, uint8_t *first_tab8, double f
 // ---------------------------------------------------------------------------------------------
 // Interval compaction: per-window record chunks (arbitrary order) -> sorted clb_interval array
 // ---------------------------------------------------------------------------------------------
-struct IntervalOut { uint32_t start, end; uint8_t state, soft; uint16_t pad; };
-
-// Records a window contributes to the sorted interval list: its count, minus the first record when that one is only
-// "window soft" (fast kernel: emitted unconditionally for the window's first position) and the previous window ended
-// in the same state.  win_tab[w].y = count | first state << 12 | window soft << 16 | last state << 20.
-__device__ __forceinline__ uint32_t win_drop_first(const uint2 *win_tab, uint32_t w) {
-    const uint32_t y = win_tab[w].y;
-    if (!((y >> 16) & 1u) || w == 0) return 0u;
-    return ((y >> 12) & 15u) == ((win_tab[w - 1].y >> 20) & 15u) ? 1u : 0u;
-}
-
 // step 1: every block scans 1024 windows locally and publishes its total
 __global__ void __launch_bounds__(1024) k_scan_windows_local(const uint2 *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot,
                                                              const uint32_t *err) {
@@ -1173,7 +1250,7 @@ __global__ void __launch_bounds__(1024) k_scan_windows_local(const uint2 *win_ta
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (*err & ERR_RESULT_INVALID) return;                    // win_tab was not written: nothing to scan
     const uint32_t i = blockIdx.x * 1024u + tid;
-    const uint32_t v = i < n_w ? (win_tab[i].y & 0xfffu) - win_drop_first(win_tab, i) : 0u;
+    const uint32_t v = i < n_w ? win_count(win_tab[i].y) - win_drop_first(win_tab, i) : 0u;
     uint32_t inc = v;
 #pragma unroll
     for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inc, dd); if (lane >= dd) inc += t; }
@@ -1220,11 +1297,9 @@ __global__ void k_gather_intervals(const unsigned long long *rec, const uint2 *w
     if (w >= n_w || (*err & (ERR_REC_OVERFLOW | ERR_RESULT_INVALID))) return;
     const uint2 t = win_tab[w];
     const uint32_t skip = win_drop_first(win_tab, w);
-    const uint32_t o = blk_off[w >> 10] + win_out[w], cnt = (t.y & 0xfffu) - skip;
+    const uint32_t o = blk_off[w >> 10] + win_out[w], cnt = win_count(t.y) - skip;
     for (uint32_t i = lane; i < cnt; i += 32) {
-        const unsigned long long r = rec[t.x + skip + i];
-        IntervalOut iv; iv.start = (uint32_t)r; iv.end = 0; iv.state = (uint8_t)(r >> 32); iv.soft = (uint8_t)((r >> 40) & 1u); iv.pad = 0;
-        out[o + i] = iv;
+        out[o + i] = unpack_rec(rec[t.x + skip + i]);
     }
 }
 
