@@ -59,6 +59,10 @@ class ContigDeviceResult:
     fast_ms: float = 0.0
     general_windows: int = 0
     upload_ms: float = 0.0
+    # depth histograms (set_depth_histogram): uint64[n] each, None when off.  Bin d counts the positions that are not REF_N
+    # with raw / QC depth d; the last bin counts every depth >= n - 1.
+    depth_hist_raw: Optional[np.ndarray] = None
+    depth_hist_qc: Optional[np.ndarray] = None
 
 
 def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDeviceResult:
@@ -110,6 +114,18 @@ class CallableLociContext:
         if rc != 0:
             raise ClbError(rc, self._L.clb_last_error(self._h).decode())
 
+    def set_depth_histogram(self, n_bins: int):
+        """Raw- and QC-depth histograms of n_bins bins (2..65536; 0: off, the default) from the next begin_contig on."""
+        self._check(self._L.clb_set_depth_histogram(self._h, int(n_bins)))
+
+    def _with_hist(self, r: ContigDeviceResult) -> ContigDeviceResult:
+        raw = C.POINTER(C.c_uint64)(); qc = C.POINTER(C.c_uint64)(); n = C.c_uint32(0)
+        self._check(self._L.clb_depth_histogram(self._h, C.byref(raw), C.byref(qc), C.byref(n)))
+        if n.value:
+            r.depth_hist_raw = np.ctypeslib.as_array(raw, shape=(n.value,)).copy()
+            r.depth_hist_qc = np.ctypeslib.as_array(qc, shape=(n.value,)).copy()
+        return r
+
     def set_stream(self, cuda_stream: int):
         self._check(self._L.clb_set_stream(self._h, C.c_void_p(int(cuda_stream) or None)))
 
@@ -148,7 +164,7 @@ class CallableLociContext:
         res = _lib.ContigResult()
         self._check(self._L.clb_finish_contig(self._h, C.byref(res)))
         self._keep = self._keep[:1]
-        return _result(res, copy_intervals)
+        return self._with_hist(_result(res, copy_intervals))
 
     def finish_contig_raw(self) -> "_lib.ContigResult":
         """clb_finish_contig without copying anything out: the struct's pointers stay valid until the next begin_contig."""
@@ -169,7 +185,7 @@ class CallableLociContext:
         if fetch:
             res = _lib.ContigResult()
             self._check(self._L.clb_rerun_resident(self._h, C.byref(res), C.byref(ms)))
-            return float(ms.value), _result(res, copy_intervals)
+            return float(ms.value), self._with_hist(_result(res, copy_intervals))
         self._check(self._L.clb_rerun_resident(self._h, None, C.byref(ms)))
         return float(ms.value), None
 
@@ -181,7 +197,7 @@ class CallableLociContext:
     def refresh_counters(self) -> ContigDeviceResult:
         res = _lib.ContigResult()
         self._check(self._L.clb_refresh_counters(self._h, C.byref(res)))
-        return _result(res, True)
+        return self._with_hist(_result(res, True))
 
     def debug_per_base(self, n: int):
         raw = np.zeros(n, np.uint32); qc = np.zeros(n, np.uint32); low = np.zeros(n, np.uint32); st = np.zeros(n, np.uint8)

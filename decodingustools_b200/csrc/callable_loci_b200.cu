@@ -50,6 +50,8 @@ struct clb_ctx {
     uint32_t contig_len = 0, largest = 0, region_start = 0, region_end = 0;
     uint32_t n_windows = 0, windows_done = 0;
     uint32_t stride = 0, n_bins = 0;
+    uint32_t dh_next = 0, dh_n = 0;     // depth-histogram bins: set by clb_set_depth_histogram, in force for the current contig
+    uint32_t dh_fetched = 0;            // ... and in the result of the last fetch (clb_depth_histogram)
     bool long_mode = false, span_on_device = false;
     uint64_t n_reads = 0, n_cigar = 0, n_qual = 0;
     long long last_pos = -1;
@@ -57,7 +59,7 @@ struct clb_ctx {
     DevBuf pos, flag, mapq, cigar_off, cigar, qual_off, qual, read_end, cigar_ckpt;
     DevBuf nmask, ref_ascii;
     DevBuf stats_padded, counters, rec, win_tab, win_rec, win_out, deep_list, intervals, misc;
-    DevBuf gen_list, blk_tot;
+    DevBuf gen_list, blk_tot, dhist;
     DevBuf dbg_raw, dbg_qc, dbg_low, dbg_state, timing;
     uint32_t rec_cap = 0;
     bool dbg = false;
@@ -117,6 +119,9 @@ int ensure(clb_ctx *ctx, DevBuf &b, size_t bytes, bool keep, cudaStream_t s) {
 
 void release(DevBuf &b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
 
+// u64 words of the counter buffer: [N_STATS stats][3 x n_bins bins][n raw][n qc] (histograms only when on)
+size_t n_counters(const clb_ctx *c) { return (size_t)N_STATS + 3 * (size_t)c->n_bins + 2 * (size_t)c->dh_n; }
+
 int get_events(clb_ctx *ctx, EvPair &ep) {
     if (!ctx->ev_pool.empty()) { ep = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); return CLB_OK; }
     CU(cudaEventCreate(&ep.a)); CU(cudaEventCreate(&ep.b));
@@ -151,6 +156,7 @@ KParams make_params(clb_ctx *c) {
     P.max_span = (const uint32_t *)c->misc.p + M_MAXSPAN;
     P.max_low_mapq_fraction = c->opt.max_low_mapq_fraction;
     P.timing = (long long *)c->timing.p;
+    P.dhist = c->dh_n ? (unsigned long long *)c->dhist.p : nullptr; P.dh_n = c->dh_n;
     if (c->dbg) {
         P.dbg_raw = (uint32_t *)c->dbg_raw.p; P.dbg_qc = (uint32_t *)c->dbg_qc.p;
         P.dbg_low = (uint32_t *)c->dbg_low.p; P.dbg_state = (uint8_t *)c->dbg_state.p;
@@ -159,12 +165,14 @@ KParams make_params(clb_ctx *c) {
 }
 
 // The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
-// with the per-base dump (parity tests).  f is called with two std::integral_constant<bool, ...>.
+// with the per-base dump (parity tests), HIST the one that also counts the depth histograms (only launched when they are
+// on, so the others stay as they were).  f is called with three std::integral_constant<bool, ...>.
 template <typename F>
-void with_variant(bool bq_hi, bool dbg, F &&f) {
+void with_variant(bool bq_hi, bool dbg, bool hist, F &&f) {
     using T = std::true_type; using N = std::false_type;
-    if (bq_hi) { if (dbg) f(T{}, T{}); else f(T{}, N{}); }
-    else { if (dbg) f(N{}, T{}); else f(N{}, N{}); }
+    auto h = [&](auto b, auto d) { if (hist) f(b, d, T{}); else f(b, d, N{}); };
+    if (bq_hi) { if (dbg) h(T{}, T{}); else h(T{}, N{}); }
+    else { if (dbg) h(N{}, T{}); else h(N{}, N{}); }
 }
 
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
@@ -184,15 +192,15 @@ int launch_windows(clb_ctx *ctx, uint32_t w0, uint32_t w1, EvPair *time_pileup =
     const bool hi = ctx->opt.min_base_quality >= 128;
     if (!all_general) {
         if (time_fast) CU(cudaEventRecord(time_fast->a, ctx->s_compute));
-        with_variant(hi, ctx->dbg, [&](auto h, auto d) {
-            k_pileup_fast<decltype(h)::value, decltype(d)::value><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
+        with_variant(hi, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+            k_pileup_fast<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
         });
         if (time_fast) CU(cudaEventRecord(time_fast->b, ctx->s_compute));
         ctx->launches += 1;
     }
     const uint32_t g = (uint32_t)std::min<uint64_t>((uint64_t)ctx->n_sm * std::max(1, ctx->max_ctas_per_sm), all_general ? n : 0xffffffffu);
-    with_variant(hi, ctx->dbg, [&](auto h, auto d) {
-        k_pileup_general<decltype(h)::value, decltype(d)::value><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
+    with_variant(hi, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+        k_pileup_general<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
     });
     if (time_pileup) CU(cudaEventRecord(time_pileup->b, ctx->s_compute));
     ctx->launches += 2;
@@ -202,7 +210,8 @@ int launch_windows(clb_ctx *ctx, uint32_t w0, uint32_t w1, EvPair *time_pileup =
 
 int reset_accumulators(clb_ctx *ctx) {
     CU(cudaMemsetAsync(ctx->stats_padded.p, 0, (size_t)N_STATS * STAT_STRIDE * 8, ctx->s_compute));
-    CU(cudaMemsetAsync(ctx->counters.p, 0, ((size_t)N_STATS + 3 * (size_t)ctx->n_bins) * 8, ctx->s_compute));
+    CU(cudaMemsetAsync(ctx->counters.p, 0, n_counters(ctx) * 8, ctx->s_compute));
+    if (ctx->dh_n) CU(cudaMemsetAsync(ctx->dhist.p, 0, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, ctx->s_compute));
     CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_CURSOR, 0, M_RESET_WORDS * sizeof(uint32_t), ctx->s_compute));   // cursor, err, n_total, deep windows, general queue
     return CLB_OK;
 }
@@ -212,8 +221,8 @@ int launch_compaction(clb_ctx *ctx) {
     {
         // windows with more than 65535 candidate reads were queued by the general kernel (normally none)
         const KParams P = make_params(ctx);
-        with_variant(ctx->opt.min_base_quality >= 128, ctx->dbg, [&](auto h, auto d) {
-            k_pileup_classify_deep<decltype(h)::value, decltype(d)::value><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
+        with_variant(ctx->opt.min_base_quality >= 128, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+            k_pileup_classify_deep<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
         });
         ctx->launches += 1;
     }
@@ -230,6 +239,12 @@ int launch_compaction(clb_ctx *ctx) {
                                                                        (const uint32_t *)ctx->misc.p + M_ERR);
     k_pack_stats<<<1, 32, 0, ctx->s_compute>>>((const unsigned long long *)ctx->stats_padded.p, (unsigned long long *)ctx->counters.p);
     ctx->launches += 5;
+    if (ctx->dh_n) {
+        const uint32_t n2 = 2 * ctx->dh_n;
+        k_fold_depth_hist<<<(n2 + 255) / 256, 256, 0, ctx->s_compute>>>((const unsigned long long *)ctx->dhist.p, n2,
+                                                                     (unsigned long long *)ctx->counters.p + N_STATS + 3 * (size_t)ctx->n_bins);
+        ctx->launches += 1;
+    }
     CU(cudaGetLastError());
     return CLB_OK;
 }
@@ -250,7 +265,8 @@ int alloc_outputs(clb_ctx *ctx) {
 
 // copy counters + interval count, validate device error bits, then copy the intervals
 int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
-    const size_t n_cnt = (size_t)N_STATS + 3 * (size_t)ctx->n_bins;
+    const size_t n_cnt = n_counters(ctx);
+    ctx->dh_fetched = 0;
     ctx->h_counters.resize(n_cnt);
     CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, M_WORDS * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaMemcpyAsync(ctx->h_counters.data(), ctx->counters.p, n_cnt * 8, cudaMemcpyDeviceToHost, ctx->s_compute));
@@ -275,6 +291,7 @@ int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     ctx->d2h_bytes = M_WORDS * 4 + n_cnt * 8 + n_iv * sizeof(clb_interval);
     ctx->h_bins.resize(3 * (size_t)ctx->n_bins);
     for (size_t i = 0; i < ctx->h_bins.size(); i++) ctx->h_bins[i] = (uint32_t)ctx->h_counters[N_STATS + i];
+    ctx->dh_fetched = ctx->dh_n;                                             // the histograms stay in h_counters, after the bins
 
     float kms = 0, hms = 0, ums = 0;
     for (auto &ep : ctx->ev_upload) { float t = 0; cudaEventElapsedTime(&t, ep.a, ep.b); ums += t; ctx->ev_pool.push_back(ep); }
@@ -367,13 +384,13 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-    for (int v = 0; v < 4; v++)                              // every instantiation of the pileup kernels
-        with_variant(v & 1, v & 2, [&](auto h, auto d) {
-            constexpr bool H = decltype(h)::value, D = decltype(d)::value;
+    for (int v = 0; v < 8; v++)                              // every instantiation of the pileup kernels
+        with_variant(v & 1, v & 2, v & 4, [&](auto h, auto d, auto x) {
+            constexpr bool H = decltype(h)::value, D = decltype(d)::value, X = decltype(x)::value;
             const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_general<H, D>, smem, (int)SMEM_BYTES);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_classify_deep<H, D>, smem, (int)SMEM_BYTES_DEEP);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_fast<H, D>, smem, (int)F_SMEM);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_general<H, D, X>, smem, (int)SMEM_BYTES);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_classify_deep<H, D, X>, smem, (int)SMEM_BYTES_DEEP);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_fast<H, D, X>, smem, (int)F_SMEM);
         });
     if (e != cudaSuccess) { clb_destroy(ctx); return bail("cudaFuncSetAttribute (pileup kernels)", e); }
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->max_ctas_per_sm, k_pileup_general<false, false>, NT, SMEM_BYTES);
@@ -392,7 +409,7 @@ void clb_destroy(clb_ctx *ctx) {
     cudaDeviceSynchronize();
     for (DevBuf *b : {&ctx->pos, &ctx->flag, &ctx->mapq, &ctx->cigar_off, &ctx->cigar, &ctx->qual_off, &ctx->qual, &ctx->read_end, &ctx->cigar_ckpt,
                       &ctx->nmask, &ctx->ref_ascii, &ctx->stats_padded, &ctx->counters, &ctx->rec, &ctx->win_tab, &ctx->win_rec,
-                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
+                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dhist, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
         release(*b);
     if (ctx->d_first_tab) cudaFree(ctx->d_first_tab);
     if (ctx->h_intervals) cudaFreeHost(ctx->h_intervals);
@@ -439,6 +456,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     ctx->long_mode = false; ctx->span_on_device = (max_ref_span == 0);
     ctx->h2d_bytes = 0; ctx->d2h_bytes = 0; ctx->launches = 0; ctx->n_intervals = 0;
     ctx->dbg = false;
+    ctx->dh_n = ctx->dh_next; ctx->dh_fetched = 0;
     clb_bin_geometry(ctx->name.c_str(), contig_len, largest_contig_len, &ctx->stride, &ctx->n_bins);
 
     // reference -> bit-packed N mask, padded so every window can read two words past its last entry
@@ -475,7 +493,8 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
 
     if ((rc = ensure(ctx, ctx->misc, M_WORDS * 4, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->stats_padded, (size_t)N_STATS * STAT_STRIDE * 8, false, ctx->s_compute))) return rc;
-    if ((rc = ensure(ctx, ctx->counters, ((size_t)N_STATS + 3 * (size_t)ctx->n_bins) * 8, false, ctx->s_compute))) return rc;
+    if ((rc = ensure(ctx, ctx->counters, n_counters(ctx) * 8, false, ctx->s_compute))) return rc;
+    if (ctx->dh_n && (rc = ensure(ctx, ctx->dhist, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, false, ctx->s_compute))) return rc;
     const uint64_t rlen = region_end - region_start;
     ctx->rec_cap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(rlen / 4 + 4096, 1u << 16), (uint64_t)rlen + 16);
     if ((rc = alloc_outputs(ctx))) return rc;
@@ -652,7 +671,7 @@ int clb_wait_uploads(clb_ctx *ctx) {
 int clb_counters_device(clb_ctx *ctx, void **dev_ptr, uint64_t *n_u64) {
     if (!ctx || !ctx->in_contig) return fail(ctx, CLB_E_INVALID, "no contig");
     if (dev_ptr) *dev_ptr = ctx->counters.p;
-    if (n_u64) *n_u64 = (uint64_t)N_STATS + 3 * (uint64_t)ctx->n_bins;
+    if (n_u64) *n_u64 = (uint64_t)n_counters(ctx);
     return CLB_OK;
 }
 
@@ -661,6 +680,24 @@ int clb_refresh_counters(clb_ctx *ctx, clb_contig_result *out) {
     CU(cudaSetDevice(ctx->device));
     CU(cudaDeviceSynchronize());     // the reduction may have run on a stream we do not own
     return fetch_result(ctx, out);
+}
+
+int clb_set_depth_histogram(clb_ctx *ctx, uint32_t n_bins) {
+    if (!ctx) return CLB_E_INVALID;
+    if (ctx->in_contig && !ctx->finished) return fail(ctx, CLB_E_INVALID, "clb_set_depth_histogram while a contig is open");
+    if (n_bins != 0 && (n_bins < 2 || n_bins > 65536)) return fail(ctx, CLB_E_INVALID, "depth histogram bins %u: 0 (off) or 2..65536", n_bins);
+    ctx->dh_next = n_bins;
+    return CLB_OK;
+}
+
+int clb_depth_histogram(const clb_ctx *ctx, const uint64_t **raw, const uint64_t **qc, uint32_t *n_bins) {
+    if (!ctx) return CLB_E_INVALID;
+    const uint32_t n = ctx->dh_fetched;
+    const unsigned long long *h = n ? ctx->h_counters.data() + N_STATS + 3 * (size_t)ctx->n_bins : nullptr;
+    if (raw) *raw = (const uint64_t *)h;
+    if (qc) *qc = n ? (const uint64_t *)(h + n) : nullptr;
+    if (n_bins) *n_bins = n;
+    return CLB_OK;
 }
 
 static void *g_nccl_allreduce = nullptr;
@@ -680,7 +717,7 @@ int clb_allreduce_nccl(clb_ctx *ctx, void *nccl_comm) {
         if (!fn) return fail(ctx, CLB_E_UNSUPPORTED, "ncclAllReduce not found in this process");
     }
     CU(cudaSetDevice(ctx->device));
-    const size_t n = (size_t)N_STATS + 3 * (size_t)ctx->n_bins;
+    const size_t n = n_counters(ctx);
     const int ncclUint64 = 5, ncclSum = 0;       // nccl.h: ncclDataType_t / ncclRedOp_t (stable since NCCL 2.0)
     const int r = fn(ctx->counters.p, ctx->counters.p, n, ncclUint64, ncclSum, nccl_comm, ctx->s_compute);
     if (r != 0) return fail(ctx, CLB_E_CUDA, "ncclAllReduce returned %d", r);

@@ -49,9 +49,10 @@ constexpr size_t F_SMEM = F_OFF_BAR + NWARPS * 8;
 constexpr int F_OFF_SCAN = F_OFF_STAGE;                        // phase C scratch inside the stages
 constexpr int F_OFF_LAST = F_OFF_SCAN + 64 * 4;
 constexpr int F_OFF_WSTATS = F_OFF_LAST + NT;
+constexpr int F_OFF_HIST = F_OFF_WSTATS + NWARPS * N_STATS * 8;    // depth table (HIST instantiations), 2 x DH_TAB u32
 static_assert(F_OFF_STAGE % 16 == 0 && F_WSTAGE % 16 == 0, "bulk copies need 16-byte aligned destinations");
 static_assert(F_OFF_WSTATS % 8 == 0 && F_OFF_BAR % 8 == 0 && F_OFF_X % 8 == 0 && F_OFF_MASK % 16 == 0 && F_OFF_FIRST % 16 == 0, "alignment");
-static_assert(F_OFF_WSTATS + NWARPS * N_STATS * 8 <= F_OFF_X, "phase C scratch fits the stages");
+static_assert(F_OFF_HIST + 2 * DH_TAB * 4 <= F_OFF_X, "phase C scratch fits the stages");
 static_assert(CLB_F_MINB * (F_SMEM + 1024) <= 228 * 1024, "shared memory per SM");
 enum { FC_BAIL = 0, FC_XCNT = 1 };
 
@@ -172,7 +173,7 @@ __device__ __forceinline__ void fmeta_load(const KParams &P, FMeta &M, uint32_t 
     M.pback = P.pos[ic >= (uint32_t)F_LOOKBACK ? ic - (uint32_t)F_LOOKBACK : 0u];
 }
 
-template <bool BQ_HI, bool DBG>
+template <bool BQ_HI, bool DBG, bool HIST = false>
 __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint32_t w = P.win_first + blockIdx.x;
@@ -338,6 +339,11 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     CLB_STAMP(5);
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert(PPT == 8, "phase C of the fast kernel is written for 8 entries per thread");
+    // The stages are dead since the barrier after the main loop (each warp's last sub-batch has streamed) and nothing has
+    // gone to global memory (a window that bailed returned above): zero the depth table here, the scan barrier below orders
+    // it before the first count.
+    uint32_t *sHist = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_HIST);
+    if constexpr (HIST) zero_depth_table(sHist);
     uint32_t a[PPT], qcv[PPT];
     {
         const uint4 a0 = *reinterpret_cast<const uint4 *>(sA + ebase), a1 = *reinterpret_cast<const uint4 *>(sA + ebase + 4);
@@ -373,14 +379,19 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     const uint32_t nbits = __funnelshift_r(nm0, nm1, (wb0 + ebase) & 31u);
     Entries<uint32_t> e = entries_of<uint32_t>(ebase, 0u, n_ent);          // no halo entry
     const StateLimits lim = state_limits(P);
+    DepthHist dh{};
+    if constexpr (HIST) dh = depth_hist_of(smem_addr(sHist), P);
 #pragma unroll
     for (int k = 0; k < PPT; k++) {
         const uint32_t raw = a[k] & 0xffffu;
         classify_entry(e, k, raw, a[k] >> 16, qcv[k], sFirst[raw], (nbits >> k) & 1u, lim);   // one byte per depth: raw <= 254 (depth proof)
+        if constexpr (HIST) count_depth<true>(dh, e, k, raw, qcv[k]);      // qc <= raw <= 254: the table holds every depth
     }
+    if constexpr (HIST) close_depth_runs<true>(dh);
     close_entries(e, n_ent, sLast, sScan);
     dbg_dump<DBG>(e, w * (uint32_t)WREAL, [&](int k) { return make_uint3(a[k] & 0xffffu, qcv[k], a[k] >> 16); }, P);
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
+    if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
     // the window's first position always starts a record (window soft: the interval gather drops it when the previous
     // window ended in the same state)
     write_records(e, wb0, 0u, 0u, w > 0 ? 1u : 0u, sLast, sScan, w, P);

@@ -103,6 +103,10 @@ struct KParams {
     uint32_t *dbg_raw, *dbg_qc, *dbg_low;
     uint8_t *dbg_state;
     long long *timing;             // optional (developer builds): 8 clock64 stamps per window
+    // depth histograms (HIST instantiations only): DH_SLOTS copies of [raw n][qc n], CTA b adds to copy b % DH_SLOTS;
+    // k_fold_depth_hist sums them into the counter buffer
+    unsigned long long *dhist;
+    uint32_t dh_n;                 // bins per histogram, 2 .. 65536; the last one counts every depth >= dh_n - 1
 };
 
 // Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
@@ -524,6 +528,59 @@ __device__ __forceinline__ void classify_entry(Entries<Sum> &e, int k, uint32_t 
     e.sraw += raw; e.sqc += qc;
 }
 
+// Depth histograms (HIST instantiations; DESIGN.md §4).  Each CTA counts into a table of DH_TAB u32 bins per histogram in
+// shared memory (raw at s_tab, qc at s_tab + 4 * DH_TAB), zeroed at the start of phase C, and flushes it after the
+// reduce_stats barrier into its global slot copy; a clamped depth past the table (general and deep kernels only) goes to the
+// slot copy directly.  A thread merges runs of equal depth over its entries in registers first (depth changes at read ends
+// only, so at 30x a thread's 8 entries hold two or three runs): one predicated shared atomic per run instead of per entry.
+#ifndef CLB_DH_SLOTS
+#define CLB_DH_SLOTS 16
+#endif
+constexpr int DH_SLOTS = CLB_DH_SLOTS;   // global copies of the histograms (blockIdx.x % DH_SLOTS): spreads the flush atomics
+constexpr int DH_TAB = 256;              // shared bins per histogram: every depth the fast kernel can see (raw <= 254)
+struct DepthHist {
+    uint32_t s_tab, nm1;                 // shared table, n - 1
+    unsigned long long *g;               // this CTA's slot copy: [raw n][qc n]
+    uint32_t rd, rc, qd, qn;             // open runs: (depth, entries) of raw and qc
+};
+__device__ __forceinline__ DepthHist depth_hist_of(uint32_t s_tab, const KParams &P) {
+    return DepthHist{s_tab, P.dh_n - 1u, P.dhist + (size_t)(blockIdx.x % DH_SLOTS) * 2u * P.dh_n, 0u, 0u, 0u, 0u};
+}
+// TAB_ONLY: the caller's depths never exceed DH_TAB - 1 (k_pileup_fast's depth proof)
+template <bool TAB_ONLY>
+__device__ __forceinline__ void depth_hist_add(const DepthHist &h, uint32_t which, uint32_t d, uint32_t cnt) {
+    if (TAB_ONLY || d < (uint32_t)DH_TAB) red_shared_nz(h.s_tab + 4u * ((uint32_t)DH_TAB * which + d), cnt);
+    else if (cnt) atomicAdd(h.g + (size_t)which * (h.nm1 + 1u) + d, (unsigned long long)cnt);
+}
+// Entry k of the classification: counts when it is one of the window's own entries (vmask: not the general kernel's halo,
+// not past the region end) and not REF_N, at depth min(depth, n - 1).
+template <bool TAB_ONLY, typename Sum>
+__device__ __forceinline__ void count_depth(DepthHist &h, const Entries<Sum> &e, int k, uint32_t raw, uint32_t qc) {
+    const uint32_t one = (((e.vmask >> k) & 1u) && e.state(k) != ST_REF_N) ? 1u : 0u;
+    const uint32_t dr = min(raw, h.nm1), dq = min(qc, h.nm1);
+    const bool br = dr != h.rd, bq = dq != h.qd;
+    depth_hist_add<TAB_ONLY>(h, 0u, h.rd, br ? h.rc : 0u);          // a run ends: add it
+    depth_hist_add<TAB_ONLY>(h, 1u, h.qd, bq ? h.qn : 0u);
+    h.rc = (br ? 0u : h.rc) + one; h.rd = dr;
+    h.qn = (bq ? 0u : h.qn) + one; h.qd = dq;
+}
+template <bool TAB_ONLY>
+__device__ __forceinline__ void close_depth_runs(DepthHist &h) {
+    depth_hist_add<TAB_ONLY>(h, 0u, h.rd, h.rc);
+    depth_hist_add<TAB_ONLY>(h, 1u, h.qd, h.qn);
+}
+// Before the barrier that precedes the first count_depth; the table must be dead (no other phase uses it any more).
+__device__ __forceinline__ void zero_depth_table(uint32_t *tab) {
+    for (int i = threadIdx.x; i < 2 * DH_TAB; i += NT) tab[i] = 0u;
+}
+// After a barrier that follows every close_depth_runs: the table's non-zero bins to the CTA's slot copy.
+__device__ __forceinline__ void flush_depth_table(const DepthHist &h, const uint32_t *tab) {
+    for (int i = threadIdx.x; i < 2 * DH_TAB; i += NT) {
+        const uint32_t which = (uint32_t)i / DH_TAB, d = (uint32_t)i % DH_TAB, v = tab[i];
+        if (v && d <= h.nm1) atomicAdd(h.g + (size_t)which * (h.nm1 + 1u) + d, (unsigned long long)v);
+    }
+}
+
 // Entries outside [k_first, k_end) were counted as states: take them out again.  Then publish what the boundary pass reads
 // from other threads: the state of this thread's last entry and that of the window's last position.
 template <typename Sum>
@@ -672,7 +729,8 @@ __device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, u
 
 // One window.  WIDE = false packs the raw and low-MAPQ depths as 16 + 16 bits (windows with <= 65535 candidate reads, i.e.
 // practically all of them); WIDE = true keeps them in two 32-bit arrays and is only instantiated by k_pileup_classify_deep.
-template <bool BQ_HI, bool WIDE, bool DBG>
+// HIST: also count the depth histograms (the segment pool, dead in phase C, holds the shared table).
+template <bool BQ_HI, bool WIDE, bool DBG, bool HIST>
 __device__ __forceinline__ void pileup_classify_window(const KParams &P, const uint32_t w) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw);
@@ -885,6 +943,9 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     CLB_STAMP(3);
 
     // ------------------------------------------------------------------ phase C: scan, classify, segment
+    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4, "the depth table fits the segment pool");
+    uint32_t *sHist = reinterpret_cast<uint32_t *>(sPool);
+    if constexpr (HIST) zero_depth_table(sHist);                           // the scan barrier below orders it before the counts
     const uint32_t ebase = tid * PPT;
     uint32_t a[PPT], b[PPT], lqv[PPT], lw[WIDE ? PPT : 1];
     {
@@ -951,6 +1012,8 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     using Sum = typename std::conditional<WIDE, unsigned long long, uint32_t>::type;   // deep windows: 32-bit partial sums could overflow
     Entries<Sum> e = entries_of<Sum>(ebase, ebase == 0 ? 1u : 0u, n_ent);              // entry 0 is the halo
     const StateLimits lim = state_limits(P);
+    DepthHist dh{};
+    if constexpr (HIST) dh = depth_hist_of(smem_addr(sHist), P);
     // Two copies of the per-entry classification, chosen per thread: when none of the thread's entries is deeper than
     // the shared-memory threshold table the lookup is a plain LDS; otherwise every entry may go to the global table
     // (kept apart because those loads, predicated off, would still cost six issue slots per ordinary entry).
@@ -968,6 +1031,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
                 fst = sFirst[raw];
             }
             classify_entry(e, k, raw, low, qc, fst, (nbits >> k) & 1u, lim);
+            if constexpr (HIST) count_depth<false>(dh, e, k, raw, qc);
             b[k] = qc;                                                    // keep qc (entry 0 below, optional debug dump)
         }
     };
@@ -977,6 +1041,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
         for (int k = 0; k < PPT; k++) deepest |= WIDE ? a[k] : a[k] & 0xffffu;
         if (deepest < (uint32_t)NFIRST) classify(std::false_type{}); else classify(std::true_type{});
     }
+    if constexpr (HIST) close_depth_runs<false>(dh);
     if (!(e.vmask & 1u)) {
         // the halo entry (thread 0) is a real position and carries depth: take it out of the sums again (reads are clipped
         // at the region end, so entries past it have none)
@@ -987,6 +1052,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
                   [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
+    if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
     CLB_STAMP(4);
     // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
     // previous shard's run
@@ -1001,7 +1067,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
 // General kernel: persistent CTAs take the windows queued by k_window_ranges / k_pileup_fast one ticket at a time.
 // The queue only grows between launches (all pushes of a batch of windows happen before this kernel starts on the
 // same stream), so a CTA that draws a ticket past the end gives it back and leaves: gen_taken == gen_count afterwards.
-template <bool BQ_HI, bool DBG>
+template <bool BQ_HI, bool DBG, bool HIST = false>
 __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P) {
     __shared__ uint32_t s_ticket;
     const uint32_t n = *P.gen_count;
@@ -1015,19 +1081,19 @@ __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P
         __syncthreads();
         const uint32_t t = s_ticket;
         if (t == 0xffffffffu) break;
-        if (!refused) pileup_classify_window<BQ_HI, false, DBG>(P, P.gen_list[t]);
+        if (!refused) pileup_classify_window<BQ_HI, false, DBG, HIST>(P, P.gen_list[t]);
         __syncthreads();                                     // shared memory (and s_ticket) are reused by the next window
     }
 }
 
 // Second pass over the (rare) windows k_pileup_classify queued because they hold more than 65535 candidate reads:
 // a fixed small grid walks the queue; with an empty queue the launch costs a few microseconds.
-template <bool BQ_HI, bool DBG>
+template <bool BQ_HI, bool DBG, bool HIST = false>
 __global__ void __launch_bounds__(NT, 1) k_pileup_classify_deep(const KParams P) {
     if (*P.err & ERR_RESULT_INVALID) return;
     const uint32_t n = *P.deep_count;
     for (uint32_t i = blockIdx.x; i < n; i += gridDim.x) {
-        pileup_classify_window<BQ_HI, true, DBG>(P, P.deep_list[i]);
+        pileup_classify_window<BQ_HI, true, DBG, HIST>(P, P.deep_list[i]);
         __syncthreads();                                     // shared memory is reused by the next window
     }
 }
@@ -1313,6 +1379,16 @@ __global__ void k_fill_ends(IntervalOut *out, const uint32_t *n_total, uint32_t 
 // padded per-counter lines -> compact [N_STATS] prefix of the counter buffer (bins follow it)
 __global__ void k_pack_stats(const unsigned long long *stats_padded, unsigned long long *counters) {
     if (threadIdx.x < N_STATS) counters[threadIdx.x] = stats_padded[threadIdx.x * STAT_STRIDE];
+}
+
+// the DH_SLOTS copies of the depth histograms ([raw n][qc n] each, n2 = 2n words) -> their place in the counter buffer
+__global__ void k_fold_depth_hist(const unsigned long long *slots, uint32_t n2, unsigned long long *out) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += gridDim.x * blockDim.x) {
+        unsigned long long t = 0;
+#pragma unroll
+        for (int k = 0; k < DH_SLOTS; k++) t += slots[(size_t)k * n2 + i];
+        out[i] = t;
+    }
 }
 
 }  // namespace clb

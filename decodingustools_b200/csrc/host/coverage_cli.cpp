@@ -306,13 +306,15 @@ struct Options {
     unsigned threads = std::max(1u, std::thread::hardware_concurrency());
     int device = 0;
     bool verbose = false, progress = false; std::string timing_json;
+    std::string depth_hist; uint32_t depth_hist_max = 1000;      // --depth-histogram FILE: rows for depths 0 .. depth_hist_max (last: >=)
 };
 
 void usage() {
     fprintf(stderr, "Usage: decodingus-tools-b200 coverage <BAM_FILE> -r <REFERENCE> [-o callable_regions.bed] [-s summary.html] [-L contig]...\n"
                     "       [--min-depth 4] [--max-depth 500] [--min-mapping-quality 10] [--min-base-quality 20]\n"
                     "       [--min-depth-for-low-mapq 10] [--max-low-mapq 1] [--max-low-mapq-fraction 0.1] [--threads N] [--device D]\n"
-                    "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n");
+                    "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n"
+                    "       [--depth-histogram FILE] [--depth-histogram-max 1000]\n");
     exit(2);
 }
 
@@ -339,6 +341,12 @@ Options parse_options(int argc, char **argv) {
         else if (a == "--verbose") opt.verbose = true;
         else if (a == "--progress") opt.progress = true;
         else if (a == "--timing-json") opt.timing_json = val();
+        else if (a == "--depth-histogram") opt.depth_hist = val();
+        else if (a == "--depth-histogram-max") {
+            const unsigned long d = std::stoul(val());
+            if (d < 1 || d > 65535) usage();
+            opt.depth_hist_max = (uint32_t)d;
+        }
         else if (!a.empty() && a[0] != '-' && opt.bam.empty()) opt.bam = a;
         else usage();
     }
@@ -351,6 +359,25 @@ Options parse_options(int argc, char **argv) {
 void progress(const Options &opt, const char *kind, const std::string &extra = "") {
     if (opt.progress) fprintf(stderr, "{\"%s\":{\"task\":\"Coverage Analysis\"%s}}\n", kind, extra.c_str());
 }
+
+// --depth-histogram: "#contig\tdepth\traw_bases\tqc_bases", then per contig one row per depth from 0 to its last non-zero bin
+// (the last bin of the histogram counts that depth or more), and last the sum over all contigs under the name "*".
+struct DepthHistTsv {
+    std::string text = "#contig\tdepth\traw_bases\tqc_bases\n";
+    std::vector<uint64_t> raw_total, qc_total;
+    void add_rows(const std::string &name, const uint64_t *raw, const uint64_t *qc, uint32_t n) {
+        uint32_t last = n;
+        while (last > 0 && raw[last - 1] == 0 && qc[last - 1] == 0) last--;
+        for (uint32_t d = 0; d < last; d++)
+            text += name + "\t" + std::to_string(d) + "\t" + std::to_string(raw[d]) + "\t" + std::to_string(qc[d]) + "\n";
+    }
+    void add_contig(const std::string &name, const uint64_t *raw, const uint64_t *qc, uint32_t n) {
+        raw_total.resize(n, 0); qc_total.resize(n, 0);
+        for (uint32_t d = 0; d < n; d++) { raw_total[d] += raw[d]; qc_total[d] += qc[d]; }
+        add_rows(name, raw, qc, n);
+    }
+    std::string finish() { add_rows("*", raw_total.data(), qc_total.data(), (uint32_t)raw_total.size()); return text; }
+};
 
 bool write_file(const std::string &path, const std::string &data) {
     FILE *f = fopen(path.c_str(), "wb");
@@ -371,7 +398,7 @@ struct Timing {
 // this thread   : clb_begin_contig / clb_push_reads per batch (copies overlap the kernels of earlier windows and the
 //                 decoding of the next batch) / clb_finish_contig, BED text, plots
 Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, const std::map<std::string, FaiEntry> &fai,
-                       std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed) {
+                       std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed, DepthHistTsv *hist) {
     auto check = [&](int rc, const char *what) { if (rc != 0) die(std::string("Error processing contig: ") + what + ": " + clb_last_error(ctx)); };
     // coverage plots land next to the BED file (callable_profiler.rs:24-27,80-83)
     const size_t slash = opt.out_bed.find_last_of('/');
@@ -425,6 +452,11 @@ Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, 
             st.n_covered = res.n_covered_bases; st.sum_cov = res.summed_coverage; st.sum_bq = res.summed_baseq;
             st.sum_mapq = res.summed_mapq; st.qbases = res.quality_bases;
             t.total_admitted += admitted; t.total_cells += res.summed_coverage;
+            if (hist) {
+                const uint64_t *raw = nullptr, *qc = nullptr; uint32_t n = 0;
+                check(clb_depth_histogram(ctx, &raw, &qc, &n), "depth histogram");
+                hist->add_contig(st.name, raw, qc, n);
+            }
             const auto tb = std::chrono::steady_clock::now();
             std::vector<uint32_t> bins(res.bins, res.bins + 3 * (size_t)res.n_bins);
             int has_bins = 0;
@@ -558,6 +590,8 @@ int run(int argc, char **argv) {
     char err[512];
     std::unique_ptr<clb_ctx, decltype(&clb_destroy)> ctx(clb_create(opt.device, &opt.o, err, sizeof err), clb_destroy);
     if (!ctx) die(std::string("GPU context: ") + err);
+    if (!opt.depth_hist.empty() && clb_set_depth_histogram(ctx.get(), opt.depth_hist_max + 1) != 0)
+        die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
     if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
 
@@ -575,9 +609,12 @@ int run(int argc, char **argv) {
 
     progress(opt, "Started");
     try {
-        const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get());
+        DepthHistTsv hist;
+        const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get(),
+                                         opt.depth_hist.empty() ? nullptr : &hist);
         report_timing(opt, t, stats.size(), bam.inflate_seconds());
         if (clb_bed_writer_close(bed.release()) != 0) die("failed to write " + opt.out_bed);
+        if (!opt.depth_hist.empty() && !write_file(opt.depth_hist, hist.finish())) die("cannot write " + opt.depth_hist);
         ctx.reset();
         std::vector<report::ContigRow> rows;
         const report::Summary sm = write_summary_json(opt, H.text, bs, stats, rows);

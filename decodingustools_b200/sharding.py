@@ -71,17 +71,27 @@ COUNTER_FIELDS = ("n_covered_bases", "summed_coverage", "summed_baseq", "summed_
 
 
 def pack_counters(res: ContigDeviceResult) -> np.ndarray:
-    """The additive part of a shard result as one int64 vector: 6 state counts, 5 sums, 3 * n_bins bins."""
+    """The additive part of a shard result as one int64 vector: 6 state counts, 5 sums, 3 * n_bins bins, then the raw and
+    QC depth histograms when they are on (the order of the device's counter buffer)."""
     head = np.array(list(res.state_counts) + [getattr(res, k) for k in COUNTER_FIELDS], dtype=np.uint64)
-    return np.concatenate([head, res.bins.astype(np.uint64).ravel()]).view(np.int64)
+    parts = [head, res.bins.astype(np.uint64).ravel()]
+    if res.depth_hist_raw is not None:
+        parts += [np.asarray(res.depth_hist_raw, np.uint64), np.asarray(res.depth_hist_qc, np.uint64)]
+    return np.concatenate(parts).view(np.int64)
 
 
 def unpack_counters(vec: np.ndarray, res: ContigDeviceResult) -> ContigDeviceResult:
+    """Inverse of pack_counters; whether `res` has depth histograms (and their length) says how the tail splits."""
     v = np.asarray(vec).view(np.uint64)
     res.state_counts = v[:6].copy()
     for i, k in enumerate(COUNTER_FIELDS):
         setattr(res, k, int(v[6 + i]))
-    res.bins = v[11:].reshape(3, -1).astype(np.uint32)
+    n = 0 if res.depth_hist_raw is None else len(res.depth_hist_raw)
+    end = v.shape[0] - 2 * n
+    res.bins = v[11:end].reshape(3, -1).astype(np.uint32)
+    if n:
+        res.depth_hist_raw = v[end:end + n].copy()
+        res.depth_hist_qc = v[end + n:].copy()
     return res
 
 

@@ -169,6 +169,17 @@ int clb_refresh_counters(clb_ctx *ctx, clb_contig_result *out);
 int clb_set_nccl_allreduce(void *nccl_allreduce_fn);
 int clb_allreduce_nccl(clb_ctx *ctx, void *nccl_comm);
 
+/* Depth histograms (not in the reference; off by default).  n_bins = 0: off; else 2..65536.  Bin d counts the region's
+ * positions that are not REF_N with depth d; the last bin counts depth >= n_bins - 1.  Takes effect at the next
+ * clb_begin_contig; CLB_E_INVALID while a contig is open or when out of range.
+ * Raw depth is the depth of summed_coverage (deletions and ref-skips included), QC depth the one of quality_bases (MAPQ >=
+ * min_mapping_quality and base quality >= min_base_quality).  When on, both follow the bins in the counter buffer
+ * ([12 counters][3 x n_bins bins][raw][qc], all counted by clb_counters_device), so region shards sum like the bins. */
+int clb_set_depth_histogram(clb_ctx *ctx, uint32_t n_bins);
+/* Raw-depth and QC-depth histograms of the last clb_finish_contig / clb_rerun_resident / clb_refresh_counters, [n_bins]
+ * each, owned by the context like the other results.  When off: *n_bins = 0 and NULL pointers. */
+int clb_depth_histogram(const clb_ctx *ctx, const uint64_t **raw, const uint64_t **qc, uint32_t *n_bins);
+
 /* Debug/parity: copy the per-base counters of [region_start, region_end) (computed by a separate
  * un-fused launch of the same pileup code).  Each pointer may be NULL. */
 int clb_debug_per_base(clb_ctx *ctx, uint32_t *raw, uint32_t *qc, uint32_t *low, uint8_t *state);
