@@ -63,6 +63,14 @@ class ContigDeviceResult:
     # with raw / QC depth d; the last bin counts every depth >= n - 1.
     depth_hist_raw: Optional[np.ndarray] = None
     depth_hist_qc: Optional[np.ndarray] = None
+    # depth tiles (set_depth_tiles): uint64[n_tiles] each, None when off.  Tile t covers contig positions
+    # [t * tile_len, min((t + 1) * tile_len, length)); territory counts its positions that are not REF_N, callable the
+    # CALLABLE ones, raw_sum / qc_sum the raw / QC depth summed over the territory (mean depth: sum / territory).
+    tile_len: int = 0
+    tile_territory: Optional[np.ndarray] = None
+    tile_callable: Optional[np.ndarray] = None
+    tile_raw_sum: Optional[np.ndarray] = None
+    tile_qc_sum: Optional[np.ndarray] = None
 
 
 def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDeviceResult:
@@ -78,6 +86,15 @@ def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDevice
                               iv, bins, int(res.stride), int(res.region_start), int(res.region_end), float(res.kernel_ms),
                               float(res.h2d_ms), float(res.pileup_ms), int(res.h2d_bytes), int(res.d2h_bytes), int(res.gpu_launches),
                               float(res.fast_ms), int(res.general_windows), float(res.upload_ms))
+
+
+def depth_tile_ranges(length: int, tile_len: int) -> Tuple[np.ndarray, np.ndarray]:
+    """(start, end) of the depth tiles of a contig of `length` positions (set_depth_tiles): tile t covers
+    [t * tile_len, min((t + 1) * tile_len, length)), so the last tile may be partial and a tile longer than the contig is
+    one tile covering all of it."""
+    n = -(-int(length) // int(tile_len))
+    start = np.arange(n, dtype=np.int64) * int(tile_len)
+    return start, np.minimum(start + int(tile_len), int(length))
 
 
 class CallableLociContext:
@@ -118,12 +135,23 @@ class CallableLociContext:
         """Raw- and QC-depth histograms of n_bins bins (2..65536; 0: off, the default) from the next begin_contig on."""
         self._check(self._L.clb_set_depth_histogram(self._h, int(n_bins)))
 
-    def _with_hist(self, r: ContigDeviceResult) -> ContigDeviceResult:
+    def set_depth_tiles(self, tile_len: int):
+        """Per-tile territory, callable count and raw / QC depth sums over tiles of tile_len positions (256..2^31; 0: off,
+        the default) from the next begin_contig on."""
+        self._check(self._L.clb_set_depth_tiles(self._h, int(tile_len)))
+
+    def _with_optional_counts(self, r: ContigDeviceResult) -> ContigDeviceResult:
         raw = C.POINTER(C.c_uint64)(); qc = C.POINTER(C.c_uint64)(); n = C.c_uint32(0)
         self._check(self._L.clb_depth_histogram(self._h, C.byref(raw), C.byref(qc), C.byref(n)))
         if n.value:
             r.depth_hist_raw = np.ctypeslib.as_array(raw, shape=(n.value,)).copy()
             r.depth_hist_qc = np.ctypeslib.as_array(qc, shape=(n.value,)).copy()
+        arrs = [C.POINTER(C.c_uint64)() for _ in range(4)]; nt = C.c_uint32(0); tl = C.c_uint32(0)
+        self._check(self._L.clb_depth_tiles(self._h, *[C.byref(a) for a in arrs], C.byref(nt), C.byref(tl)))
+        if nt.value:
+            r.tile_len = int(tl.value)
+            r.tile_territory, r.tile_callable, r.tile_raw_sum, r.tile_qc_sum = (
+                np.ctypeslib.as_array(a, shape=(nt.value,)).copy() for a in arrs)
         return r
 
     def set_stream(self, cuda_stream: int):
@@ -164,7 +192,7 @@ class CallableLociContext:
         res = _lib.ContigResult()
         self._check(self._L.clb_finish_contig(self._h, C.byref(res)))
         self._keep = self._keep[:1]
-        return self._with_hist(_result(res, copy_intervals))
+        return self._with_optional_counts(_result(res, copy_intervals))
 
     def finish_contig_raw(self) -> "_lib.ContigResult":
         """clb_finish_contig without copying anything out: the struct's pointers stay valid until the next begin_contig."""
@@ -185,7 +213,7 @@ class CallableLociContext:
         if fetch:
             res = _lib.ContigResult()
             self._check(self._L.clb_rerun_resident(self._h, C.byref(res), C.byref(ms)))
-            return float(ms.value), self._with_hist(_result(res, copy_intervals))
+            return float(ms.value), self._with_optional_counts(_result(res, copy_intervals))
         self._check(self._L.clb_rerun_resident(self._h, None, C.byref(ms)))
         return float(ms.value), None
 
@@ -197,7 +225,7 @@ class CallableLociContext:
     def refresh_counters(self) -> ContigDeviceResult:
         res = _lib.ContigResult()
         self._check(self._L.clb_refresh_counters(self._h, C.byref(res)))
-        return self._with_hist(_result(res, True))
+        return self._with_optional_counts(_result(res, True))
 
     def debug_per_base(self, n: int):
         raw = np.zeros(n, np.uint32); qc = np.zeros(n, np.uint32); low = np.zeros(n, np.uint32); st = np.zeros(n, np.uint8)

@@ -52,6 +52,9 @@ struct clb_ctx {
     uint32_t stride = 0, n_bins = 0;
     uint32_t dh_next = 0, dh_n = 0;     // depth-histogram bins: set by clb_set_depth_histogram, in force for the current contig
     uint32_t dh_fetched = 0;            // ... and in the result of the last fetch (clb_depth_histogram)
+    uint32_t tl_next = 0, tl_len = 0;   // depth-tile length: set by clb_set_depth_tiles, in force for the current contig
+    uint32_t n_tiles = 0;               // ceil(contig_len / tl_len) while on
+    uint32_t tl_fetched = 0;            // tiles in the result of the last fetch (clb_depth_tiles)
     bool long_mode = false, span_on_device = false;
     uint64_t n_reads = 0, n_cigar = 0, n_qual = 0;
     long long last_pos = -1;
@@ -119,8 +122,10 @@ int ensure(clb_ctx *ctx, DevBuf &b, size_t bytes, bool keep, cudaStream_t s) {
 
 void release(DevBuf &b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
 
-// u64 words of the counter buffer: [N_STATS stats][3 x n_bins bins][n raw][n qc] (histograms only when on)
-size_t n_counters(const clb_ctx *c) { return (size_t)N_STATS + 3 * (size_t)c->n_bins + 2 * (size_t)c->dh_n; }
+// u64 words of the counter buffer: [N_STATS stats][3 x n_bins bins][n raw][n qc][territory T][callable T][raw_sum T][qc_sum T]
+// (histograms and tiles only when on)
+size_t tiles_offset(const clb_ctx *c) { return (size_t)N_STATS + 3 * (size_t)c->n_bins + 2 * (size_t)c->dh_n; }
+size_t n_counters(const clb_ctx *c) { return tiles_offset(c) + 4 * (size_t)c->n_tiles; }
 
 int get_events(clb_ctx *ctx, EvPair &ep) {
     if (!ctx->ev_pool.empty()) { ep = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); return CLB_OK; }
@@ -157,6 +162,7 @@ KParams make_params(clb_ctx *c) {
     P.max_low_mapq_fraction = c->opt.max_low_mapq_fraction;
     P.timing = (long long *)c->timing.p;
     P.dhist = c->dh_n ? (unsigned long long *)c->dhist.p : nullptr; P.dh_n = c->dh_n;
+    P.tiles = c->tl_len ? (unsigned long long *)c->counters.p + tiles_offset(c) : nullptr; P.tile_len = c->tl_len; P.n_tiles = c->n_tiles;
     if (c->dbg) {
         P.dbg_raw = (uint32_t *)c->dbg_raw.p; P.dbg_qc = (uint32_t *)c->dbg_qc.p;
         P.dbg_low = (uint32_t *)c->dbg_low.p; P.dbg_state = (uint8_t *)c->dbg_state.p;
@@ -165,15 +171,24 @@ KParams make_params(clb_ctx *c) {
 }
 
 // The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
-// with the per-base dump (parity tests), HIST the one that also counts the depth histograms (only launched when they are
-// on, so the others stay as they were).  f is called with three std::integral_constant<bool, ...>.
+// with the per-base dump (parity tests), FEAT the optional counts that are on (FEAT_HIST: depth histograms, FEAT_TILES: depth
+// tiles; only launched when on, so the others stay as they were).  f is called with two std::integral_constant<bool, ...>
+// and one std::integral_constant<unsigned, FEAT>.
 template <typename F>
-void with_variant(bool bq_hi, bool dbg, bool hist, F &&f) {
+void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
     using T = std::true_type; using N = std::false_type;
-    auto h = [&](auto b, auto d) { if (hist) f(b, d, T{}); else f(b, d, N{}); };
+    auto h = [&](auto b, auto d) {
+        switch (feat) {
+        case 0: f(b, d, std::integral_constant<unsigned, 0u>{}); break;
+        case FEAT_HIST: f(b, d, std::integral_constant<unsigned, FEAT_HIST>{}); break;
+        case FEAT_TILES: f(b, d, std::integral_constant<unsigned, FEAT_TILES>{}); break;
+        default: f(b, d, std::integral_constant<unsigned, FEAT_HIST | FEAT_TILES>{}); break;
+        }
+    };
     if (bq_hi) { if (dbg) h(T{}, T{}); else h(T{}, N{}); }
     else { if (dbg) h(N{}, T{}); else h(N{}, N{}); }
 }
+unsigned features(const clb_ctx *c) { return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u); }
 
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
 // queue of windows the other two handed over) for windows [w0, w1) on the compute stream
@@ -192,14 +207,14 @@ int launch_windows(clb_ctx *ctx, uint32_t w0, uint32_t w1, EvPair *time_pileup =
     const bool hi = ctx->opt.min_base_quality >= 128;
     if (!all_general) {
         if (time_fast) CU(cudaEventRecord(time_fast->a, ctx->s_compute));
-        with_variant(hi, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+        with_variant(hi, ctx->dbg, features(ctx), [&](auto h, auto d, auto x) {
             k_pileup_fast<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<n, NT, F_SMEM, ctx->s_compute>>>(P);
         });
         if (time_fast) CU(cudaEventRecord(time_fast->b, ctx->s_compute));
         ctx->launches += 1;
     }
     const uint32_t g = (uint32_t)std::min<uint64_t>((uint64_t)ctx->n_sm * std::max(1, ctx->max_ctas_per_sm), all_general ? n : 0xffffffffu);
-    with_variant(hi, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+    with_variant(hi, ctx->dbg, features(ctx), [&](auto h, auto d, auto x) {
         k_pileup_general<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<g, NT, SMEM_BYTES, ctx->s_compute>>>(P);
     });
     if (time_pileup) CU(cudaEventRecord(time_pileup->b, ctx->s_compute));
@@ -221,7 +236,7 @@ int launch_compaction(clb_ctx *ctx) {
     {
         // windows with more than 65535 candidate reads were queued by the general kernel (normally none)
         const KParams P = make_params(ctx);
-        with_variant(ctx->opt.min_base_quality >= 128, ctx->dbg, ctx->dh_n != 0, [&](auto h, auto d, auto x) {
+        with_variant(ctx->opt.min_base_quality >= 128, ctx->dbg, features(ctx), [&](auto h, auto d, auto x) {
             k_pileup_classify_deep<decltype(h)::value, decltype(d)::value, decltype(x)::value><<<ctx->n_sm, NT, SMEM_BYTES_DEEP, ctx->s_compute>>>(P);
         });
         ctx->launches += 1;
@@ -266,7 +281,7 @@ int alloc_outputs(clb_ctx *ctx) {
 // copy counters + interval count, validate device error bits, then copy the intervals
 int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     const size_t n_cnt = n_counters(ctx);
-    ctx->dh_fetched = 0;
+    ctx->dh_fetched = 0; ctx->tl_fetched = 0;
     ctx->h_counters.resize(n_cnt);
     CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, M_WORDS * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaMemcpyAsync(ctx->h_counters.data(), ctx->counters.p, n_cnt * 8, cudaMemcpyDeviceToHost, ctx->s_compute));
@@ -292,6 +307,7 @@ int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     ctx->h_bins.resize(3 * (size_t)ctx->n_bins);
     for (size_t i = 0; i < ctx->h_bins.size(); i++) ctx->h_bins[i] = (uint32_t)ctx->h_counters[N_STATS + i];
     ctx->dh_fetched = ctx->dh_n;                                             // the histograms stay in h_counters, after the bins
+    ctx->tl_fetched = ctx->n_tiles;                                          // ... and the tiles after them
 
     float kms = 0, hms = 0, ums = 0;
     for (auto &ep : ctx->ev_upload) { float t = 0; cudaEventElapsedTime(&t, ep.a, ep.b); ums += t; ctx->ev_pool.push_back(ep); }
@@ -384,9 +400,9 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-    for (int v = 0; v < 8; v++)                              // every instantiation of the pileup kernels
-        with_variant(v & 1, v & 2, v & 4, [&](auto h, auto d, auto x) {
-            constexpr bool H = decltype(h)::value, D = decltype(d)::value, X = decltype(x)::value;
+    for (int v = 0; v < 16; v++)                             // every instantiation of the pileup kernels
+        with_variant(v & 1, v & 2, (unsigned)v >> 2, [&](auto h, auto d, auto x) {
+            constexpr bool H = decltype(h)::value, D = decltype(d)::value; constexpr unsigned X = decltype(x)::value;
             const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
             if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_general<H, D, X>, smem, (int)SMEM_BYTES);
             if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pileup_classify_deep<H, D, X>, smem, (int)SMEM_BYTES_DEEP);
@@ -457,6 +473,8 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     ctx->h2d_bytes = 0; ctx->d2h_bytes = 0; ctx->launches = 0; ctx->n_intervals = 0;
     ctx->dbg = false;
     ctx->dh_n = ctx->dh_next; ctx->dh_fetched = 0;
+    ctx->tl_len = ctx->tl_next; ctx->tl_fetched = 0;
+    ctx->n_tiles = ctx->tl_len ? (uint32_t)(((uint64_t)contig_len + ctx->tl_len - 1) / ctx->tl_len) : 0u;
     clb_bin_geometry(ctx->name.c_str(), contig_len, largest_contig_len, &ctx->stride, &ctx->n_bins);
 
     // reference -> bit-packed N mask, padded so every window can read two words past its last entry
@@ -697,6 +715,28 @@ int clb_depth_histogram(const clb_ctx *ctx, const uint64_t **raw, const uint64_t
     if (raw) *raw = (const uint64_t *)h;
     if (qc) *qc = n ? (const uint64_t *)(h + n) : nullptr;
     if (n_bins) *n_bins = n;
+    return CLB_OK;
+}
+
+int clb_set_depth_tiles(clb_ctx *ctx, uint32_t tile_len) {
+    if (!ctx) return CLB_E_INVALID;
+    if (ctx->in_contig && !ctx->finished) return fail(ctx, CLB_E_INVALID, "clb_set_depth_tiles while a contig is open");
+    if (tile_len != 0 && (tile_len < 256 || tile_len > 0x80000000u)) return fail(ctx, CLB_E_INVALID, "depth tile length %u: 0 (off) or 256..2^31", tile_len);
+    ctx->tl_next = tile_len;
+    return CLB_OK;
+}
+
+int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64_t **callable, const uint64_t **raw_sum,
+                    const uint64_t **qc_sum, uint32_t *n_tiles, uint32_t *tile_len) {
+    if (!ctx) return CLB_E_INVALID;
+    const uint32_t n = ctx->tl_fetched;
+    const uint64_t *t = n ? (const uint64_t *)ctx->h_counters.data() + tiles_offset(ctx) : nullptr;
+    if (territory) *territory = t;
+    if (callable) *callable = n ? t + n : nullptr;
+    if (raw_sum) *raw_sum = n ? t + 2 * (size_t)n : nullptr;
+    if (qc_sum) *qc_sum = n ? t + 3 * (size_t)n : nullptr;
+    if (n_tiles) *n_tiles = n;
+    if (tile_len) *tile_len = n ? ctx->tl_len : 0u;
     return CLB_OK;
 }
 

@@ -107,7 +107,15 @@ struct KParams {
     // k_fold_depth_hist sums them into the counter buffer
     unsigned long long *dhist;
     uint32_t dh_n;                 // bins per histogram, 2 .. 65536; the last one counts every depth >= dh_n - 1
+    // depth tiles (TILES instantiations only): [territory][callable][raw_sum][qc_sum], n_tiles u64 each, in the counter buffer.
+    // Tile t covers contig positions [t * tile_len, min((t + 1) * tile_len, contig length)); tile_len >= 256.
+    unsigned long long *tiles;
+    uint32_t tile_len, n_tiles;
 };
+
+// The optional counts of the pileup kernels (template argument FEAT); the instantiations with a feature are only launched
+// when it is on, so the ones without stay as they were.
+enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u };
 
 // Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
 // kernel with P and w in scope.  The stamps cost instruction-cache space, so production builds compile them out.
@@ -614,6 +622,64 @@ __device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
     return v;
 }
 
+// Depth tiles (TILES instantiations; DESIGN.md §4).  Per tile: the own positions that are not REF_N (territory), the
+// CALLABLE ones, and the raw and QC depth sums over the former.  A thread's entries cross at most one tile boundary and a
+// warp's 256 entries touch at most two tiles (tile_len >= 256): each warp sums into its two tiles and parks them in its
+// slot; after the reduce_stats barrier the CTA adds the slots up for the at most TL_MAX tiles of the window and flushes
+// them with one global atomic per non-zero (tile, counter).  The slots sit beside the depth table (both may be on).
+constexpr int TL_MAX = 9;                                   // tiles one window can touch: 2047 positions, tiles of >= 256
+constexpr int TL_SLOT_BYTES = NWARPS * (8 * 8 + 4);         // per warp [2 tiles][4 counters] u64, then per warp its first tile (u32)
+// After close_entries and the general kernel's halo correction: cnt_pack, sraw and sqc cover the own entries only (entries
+// past the region end carry no depth).  pos0: position of entry 0; depth(k) = (raw, qc) of entry k.
+template <typename Sum, typename Depth>
+__device__ __forceinline__ void count_tiles(const Entries<Sum> &e, uint32_t pos0, uint32_t nbits, Depth depth, unsigned long long *sTileSum,
+                                            uint32_t *sTileFirst, const KParams &P) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t L = P.tile_len;
+    const uint32_t p = pos0 + e.ebase + e.k_first;                        // the thread's first own entry (never the halo)
+    const uint32_t t = p / L;
+    const uint32_t split = e.k_first + min(L - (p - t * L), (uint32_t)PPT);   // entries below split lie in tile t, the rest in t + 1
+    const uint32_t own = e.vmask & ~nbits;                                // own entries that are not REF_N
+    uint32_t ter0 = __popc(own), cal0 = (e.cnt_pack >> (5 * ST_CALLABLE)) & 31u, ter1 = 0u, cal1 = 0u;
+    Sum raw0 = e.sraw, qc0 = e.sqc, raw1 = 0, qc1 = 0;
+    if (own != e.vmask || split < e.k_end) {                              // REF_N depth in the sums, or a tile boundary (rare)
+        ter0 = cal0 = 0u; raw0 = qc0 = 0;
+#pragma unroll
+        for (int k = 0; k < PPT; k++) {
+            const uint2 d = depth(k);
+            const uint32_t o = (own >> k) & 1u, c = o && e.state(k) == ST_CALLABLE ? 1u : 0u;
+            const Sum r = o ? (Sum)d.x : (Sum)0, q = o ? (Sum)d.y : (Sum)0;
+            if ((uint32_t)k < split) { ter0 += o; cal0 += c; raw0 += r; qc0 += q; }
+            else { ter1 += o; cal1 += c; raw1 += r; qc1 += q; }
+        }
+    }
+    const uint32_t T = __shfl_sync(FULL, t, 0);                           // the warp's first tile
+    if (t != T) { ter1 = ter0; cal1 = cal0; raw1 = raw0; qc1 = qc0; ter0 = cal0 = 0u; raw0 = qc0 = 0; }   // then nothing reached t + 1
+    const uint32_t s0 = warp_sum(ter0), s1 = warp_sum(cal0);
+    const Sum s2 = warp_sum(raw0), s3 = warp_sum(qc0);
+    uint32_t u0 = 0u, u1 = 0u; Sum u2 = 0, u3 = 0;
+    if (__any_sync(FULL, ter1 != 0u)) { u0 = warp_sum(ter1); u1 = warp_sum(cal1); u2 = warp_sum(raw1); u3 = warp_sum(qc1); }   // warp-uniform
+    if (lane == 0) {
+        unsigned long long *ws = sTileSum + warp * 8;
+        ws[0] = s0; ws[1] = s1; ws[2] = s2; ws[3] = s3; ws[4] = u0; ws[5] = u1; ws[6] = u2; ws[7] = u3;
+        sTileFirst[warp] = T;
+    }
+}
+// After a barrier that follows every count_tiles: thread c * TL_MAX + j adds counter c of the window's tile j.
+__device__ __forceinline__ void flush_tiles(const unsigned long long *sTileSum, const uint32_t *sTileFirst, const KParams &P) {
+    const uint32_t i = threadIdx.x;
+    if (i >= 4u * TL_MAX) return;
+    const uint32_t c = i / TL_MAX, j = i % TL_MAX, t0 = sTileFirst[0];
+    unsigned long long s = 0;
+#pragma unroll
+    for (int w = 0; w < NWARPS; w++) {
+        const uint32_t d = sTileFirst[w] - t0;
+        if (d == j) s += sTileSum[w * 8 + c];
+        if (d + 1u == j) s += sTileSum[w * 8 + 4 + c];
+    }
+    if (s && t0 + j < P.n_tiles) atomicAdd(P.tiles + (size_t)c * P.n_tiles + t0 + j, s);
+}
+
 // Counters: per-warp sums in plain stores (no 64-bit shared atomics), summed after a barrier into one global atomic per
 // counter.  acc_sum / acc_mapq: the thread's base-quality and MAPQ sums (MapqSum: 64 bits unless the window's sum fits 32).
 template <typename Sum, typename MapqSum>
@@ -729,9 +795,11 @@ __device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, u
 
 // One window.  WIDE = false packs the raw and low-MAPQ depths as 16 + 16 bits (windows with <= 65535 candidate reads, i.e.
 // practically all of them); WIDE = true keeps them in two 32-bit arrays and is only instantiated by k_pileup_classify_deep.
-// HIST: also count the depth histograms (the segment pool, dead in phase C, holds the shared table).
-template <bool BQ_HI, bool WIDE, bool DBG, bool HIST>
+// FEAT: also count the depth histograms and / or the depth tiles (the segment pool, dead in phase C, holds their shared
+// tables).
+template <bool BQ_HI, bool WIDE, bool DBG, unsigned FEAT>
 __device__ __forceinline__ void pileup_classify_window(const KParams &P, const uint32_t w) {
+    constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0;
     extern __shared__ __align__(16) uint8_t smem_raw[];
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw);
     uint32_t *sB = sA + WN;
@@ -944,7 +1012,10 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
 
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4, "the depth table fits the segment pool");
+    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES, "the tile slots fit the segment pool");
     uint32_t *sHist = reinterpret_cast<uint32_t *>(sPool);
+    unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(sHist + 2 * DH_TAB);
+    uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
     if constexpr (HIST) zero_depth_table(sHist);                           // the scan barrier below orders it before the counts
     const uint32_t ebase = tid * PPT;
     uint32_t a[PPT], b[PPT], lqv[PPT], lw[WIDE ? PPT : 1];
@@ -1051,8 +1122,11 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     close_entries(e, n_ent, sLast, sScan);
     dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
                   [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
+    if constexpr (TILES)
+        count_tiles(e, (uint32_t)W.wb, nbits, [&](int k) { return make_uint2(WIDE ? a[k] : a[k] & 0xffffu, b[k]); }, sTileSum, sTileFirst, P);
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
     if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
+    if constexpr (TILES) flush_tiles(sTileSum, sTileFirst, P);
     CLB_STAMP(4);
     // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
     // previous shard's run
@@ -1067,7 +1141,7 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
 // General kernel: persistent CTAs take the windows queued by k_window_ranges / k_pileup_fast one ticket at a time.
 // The queue only grows between launches (all pushes of a batch of windows happen before this kernel starts on the
 // same stream), so a CTA that draws a ticket past the end gives it back and leaves: gen_taken == gen_count afterwards.
-template <bool BQ_HI, bool DBG, bool HIST = false>
+template <bool BQ_HI, bool DBG, unsigned FEAT = 0u>
 __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P) {
     __shared__ uint32_t s_ticket;
     const uint32_t n = *P.gen_count;
@@ -1081,19 +1155,19 @@ __global__ void __launch_bounds__(NT, CLB_MINB) k_pileup_general(const KParams P
         __syncthreads();
         const uint32_t t = s_ticket;
         if (t == 0xffffffffu) break;
-        if (!refused) pileup_classify_window<BQ_HI, false, DBG, HIST>(P, P.gen_list[t]);
+        if (!refused) pileup_classify_window<BQ_HI, false, DBG, FEAT>(P, P.gen_list[t]);
         __syncthreads();                                     // shared memory (and s_ticket) are reused by the next window
     }
 }
 
 // Second pass over the (rare) windows k_pileup_classify queued because they hold more than 65535 candidate reads:
 // a fixed small grid walks the queue; with an empty queue the launch costs a few microseconds.
-template <bool BQ_HI, bool DBG, bool HIST = false>
+template <bool BQ_HI, bool DBG, unsigned FEAT = 0u>
 __global__ void __launch_bounds__(NT, 1) k_pileup_classify_deep(const KParams P) {
     if (*P.err & ERR_RESULT_INVALID) return;
     const uint32_t n = *P.deep_count;
     for (uint32_t i = blockIdx.x; i < n; i += gridDim.x) {
-        pileup_classify_window<BQ_HI, true, DBG, HIST>(P, P.deep_list[i]);
+        pileup_classify_window<BQ_HI, true, DBG, FEAT>(P, P.deep_list[i]);
         __syncthreads();                                     // shared memory is reused by the next window
     }
 }

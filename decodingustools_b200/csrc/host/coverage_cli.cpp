@@ -307,6 +307,7 @@ struct Options {
     int device = 0;
     bool verbose = false, progress = false; std::string timing_json;
     std::string depth_hist; uint32_t depth_hist_max = 1000;      // --depth-histogram FILE: rows for depths 0 .. depth_hist_max (last: >=)
+    std::string depth_tiles; uint32_t depth_tile_size = 1000;    // --depth-tiles FILE: one row per tile of depth_tile_size positions
 };
 
 void usage() {
@@ -314,7 +315,7 @@ void usage() {
                     "       [--min-depth 4] [--max-depth 500] [--min-mapping-quality 10] [--min-base-quality 20]\n"
                     "       [--min-depth-for-low-mapq 10] [--max-low-mapq 1] [--max-low-mapq-fraction 0.1] [--threads N] [--device D]\n"
                     "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n"
-                    "       [--depth-histogram FILE] [--depth-histogram-max 1000]\n");
+                    "       [--depth-histogram FILE] [--depth-histogram-max 1000] [--depth-tiles FILE] [--depth-tile-size 1000]\n");
     exit(2);
 }
 
@@ -346,6 +347,12 @@ Options parse_options(int argc, char **argv) {
             const unsigned long d = std::stoul(val());
             if (d < 1 || d > 65535) usage();
             opt.depth_hist_max = (uint32_t)d;
+        }
+        else if (a == "--depth-tiles") opt.depth_tiles = val();
+        else if (a == "--depth-tile-size") {
+            const unsigned long long l = std::stoull(val());
+            if (l < 256 || l > (1ull << 31)) usage();
+            opt.depth_tile_size = (uint32_t)l;
         }
         else if (!a.empty() && a[0] != '-' && opt.bam.empty()) opt.bam = a;
         else usage();
@@ -379,6 +386,23 @@ struct DepthHistTsv {
     std::string finish() { add_rows("*", raw_total.data(), qc_total.data(), (uint32_t)raw_total.size()); return text; }
 };
 
+// --depth-tiles: "#contig\tstart\tend\tterritory\tcallable\tmean_raw\tmean_qc", then one row per tile, contigs in tid order.
+// start / end: the tile's 0-based half-open range; mean_raw / mean_qc: depth sums over territory (0.00 when it is 0).
+struct DepthTilesTsv {
+    std::string text = "#contig\tstart\tend\tterritory\tcallable\tmean_raw\tmean_qc\n";
+    void add_contig(const std::string &name, uint32_t contig_len, uint32_t tile_len, const uint64_t *territory, const uint64_t *callable,
+                    const uint64_t *raw_sum, const uint64_t *qc_sum, uint32_t n) {
+        char buf[160];
+        for (uint32_t t = 0; t < n; t++) {
+            const uint64_t start = (uint64_t)t * tile_len, end = std::min<uint64_t>(start + tile_len, contig_len), ter = territory[t];
+            snprintf(buf, sizeof buf, "\t%llu\t%llu\t%llu\t%llu\t%.2f\t%.2f\n", (unsigned long long)start, (unsigned long long)end,
+                     (unsigned long long)ter, (unsigned long long)callable[t], ter ? (double)raw_sum[t] / (double)ter : 0.0,
+                     ter ? (double)qc_sum[t] / (double)ter : 0.0);
+            text += name; text += buf;
+        }
+    }
+};
+
 bool write_file(const std::string &path, const std::string &data) {
     FILE *f = fopen(path.c_str(), "wb");
     if (!f) return false;
@@ -398,7 +422,8 @@ struct Timing {
 // this thread   : clb_begin_contig / clb_push_reads per batch (copies overlap the kernels of earlier windows and the
 //                 decoding of the next batch) / clb_finish_contig, BED text, plots
 Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, const std::map<std::string, FaiEntry> &fai,
-                       std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed, DepthHistTsv *hist) {
+                       std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed, DepthHistTsv *hist,
+                       DepthTilesTsv *tiles) {
     auto check = [&](int rc, const char *what) { if (rc != 0) die(std::string("Error processing contig: ") + what + ": " + clb_last_error(ctx)); };
     // coverage plots land next to the BED file (callable_profiler.rs:24-27,80-83)
     const size_t slash = opt.out_bed.find_last_of('/');
@@ -456,6 +481,11 @@ Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, 
                 const uint64_t *raw = nullptr, *qc = nullptr; uint32_t n = 0;
                 check(clb_depth_histogram(ctx, &raw, &qc, &n), "depth histogram");
                 hist->add_contig(st.name, raw, qc, n);
+            }
+            if (tiles) {
+                const uint64_t *ter = nullptr, *cal = nullptr, *raw = nullptr, *qc = nullptr; uint32_t n = 0, len = 0;
+                check(clb_depth_tiles(ctx, &ter, &cal, &raw, &qc, &n, &len), "depth tiles");
+                tiles->add_contig(st.name, clen, len, ter, cal, raw, qc, n);
             }
             const auto tb = std::chrono::steady_clock::now();
             std::vector<uint32_t> bins(res.bins, res.bins + 3 * (size_t)res.n_bins);
@@ -592,6 +622,8 @@ int run(int argc, char **argv) {
     if (!ctx) die(std::string("GPU context: ") + err);
     if (!opt.depth_hist.empty() && clb_set_depth_histogram(ctx.get(), opt.depth_hist_max + 1) != 0)
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
+    if (!opt.depth_tiles.empty() && clb_set_depth_tiles(ctx.get(), opt.depth_tile_size) != 0)
+        die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
     if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
 
@@ -610,11 +642,13 @@ int run(int argc, char **argv) {
     progress(opt, "Started");
     try {
         DepthHistTsv hist;
+        DepthTilesTsv tiles;
         const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get(),
-                                         opt.depth_hist.empty() ? nullptr : &hist);
+                                         opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles);
         report_timing(opt, t, stats.size(), bam.inflate_seconds());
         if (clb_bed_writer_close(bed.release()) != 0) die("failed to write " + opt.out_bed);
         if (!opt.depth_hist.empty() && !write_file(opt.depth_hist, hist.finish())) die("cannot write " + opt.depth_hist);
+        if (!opt.depth_tiles.empty() && !write_file(opt.depth_tiles, tiles.text)) die("cannot write " + opt.depth_tiles);
         ctx.reset();
         std::vector<report::ContigRow> rows;
         const report::Summary sm = write_summary_json(opt, H.text, bs, stats, rows);

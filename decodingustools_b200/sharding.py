@@ -68,30 +68,37 @@ def reads_for_region(reads: ReadColumns, start: int, end: int, max_ref_span: int
 
 
 COUNTER_FIELDS = ("n_covered_bases", "summed_coverage", "summed_baseq", "summed_mapq", "quality_bases")
+TILE_FIELDS = ("tile_territory", "tile_callable", "tile_raw_sum", "tile_qc_sum")
 
 
 def pack_counters(res: ContigDeviceResult) -> np.ndarray:
     """The additive part of a shard result as one int64 vector: 6 state counts, 5 sums, 3 * n_bins bins, then the raw and
-    QC depth histograms when they are on (the order of the device's counter buffer)."""
+    QC depth histograms when they are on, then the tiles' territory, callable, raw_sum and qc_sum when they are on (the
+    order of the device's counter buffer)."""
     head = np.array(list(res.state_counts) + [getattr(res, k) for k in COUNTER_FIELDS], dtype=np.uint64)
     parts = [head, res.bins.astype(np.uint64).ravel()]
     if res.depth_hist_raw is not None:
         parts += [np.asarray(res.depth_hist_raw, np.uint64), np.asarray(res.depth_hist_qc, np.uint64)]
+    if res.tile_territory is not None:
+        parts += [np.asarray(getattr(res, k), np.uint64) for k in TILE_FIELDS]
     return np.concatenate(parts).view(np.int64)
 
 
 def unpack_counters(vec: np.ndarray, res: ContigDeviceResult) -> ContigDeviceResult:
-    """Inverse of pack_counters; whether `res` has depth histograms (and their length) says how the tail splits."""
+    """Inverse of pack_counters; whether `res` has depth histograms and tiles (and their lengths) says how the tail splits."""
     v = np.asarray(vec).view(np.uint64)
     res.state_counts = v[:6].copy()
     for i, k in enumerate(COUNTER_FIELDS):
         setattr(res, k, int(v[6 + i]))
     n = 0 if res.depth_hist_raw is None else len(res.depth_hist_raw)
-    end = v.shape[0] - 2 * n
+    nt = 0 if res.tile_territory is None else len(res.tile_territory)
+    end = v.shape[0] - 2 * n - 4 * nt
     res.bins = v[11:end].reshape(3, -1).astype(np.uint32)
     if n:
         res.depth_hist_raw = v[end:end + n].copy()
-        res.depth_hist_qc = v[end + n:].copy()
+        res.depth_hist_qc = v[end + n:end + 2 * n].copy()
+    for i, k in enumerate(TILE_FIELDS if nt else ()):
+        setattr(res, k, v[end + 2 * n + i * nt:end + 2 * n + (i + 1) * nt].copy())
     return res
 
 

@@ -180,6 +180,20 @@ int clb_set_depth_histogram(clb_ctx *ctx, uint32_t n_bins);
  * each, owned by the context like the other results.  When off: *n_bins = 0 and NULL pointers. */
 int clb_depth_histogram(const clb_ctx *ctx, const uint64_t **raw, const uint64_t **qc, uint32_t *n_bins);
 
+/* Depth tiles (not in the reference; off by default): a fixed grid of tile_len positions in whole-contig coordinates, tile t
+ * = [t * tile_len, min((t + 1) * tile_len, contig_len)), n_tiles = ceil(contig_len / tile_len).  tile_len = 0: off; else
+ * 256..2^31.  Per tile, over the region's positions in it: territory (positions that are not REF_N), callable (positions
+ * classified CALLABLE), raw_sum and qc_sum (raw / QC depth summed over the positions that are not REF_N; depths as in the
+ * depth histograms).  Mean depths are sum / territory.  Takes effect at the next clb_begin_contig; CLB_E_INVALID while a
+ * contig is open or when out of range.  When on, the four arrays follow the histograms in the counter buffer
+ * ([12 counters][3 x n_bins bins][hist raw][hist qc][territory][callable][raw_sum][qc_sum], all counted by
+ * clb_counters_device), so region shards of one contig sum into the same tiles. */
+int clb_set_depth_tiles(clb_ctx *ctx, uint32_t tile_len);
+/* The tiles of the last clb_finish_contig / clb_rerun_resident / clb_refresh_counters, [n_tiles] each, owned by the context
+ * like the other results.  When off: *n_tiles = 0, *tile_len = 0 and NULL pointers. */
+int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64_t **callable, const uint64_t **raw_sum,
+                    const uint64_t **qc_sum, uint32_t *n_tiles, uint32_t *tile_len);
+
 /* Debug/parity: copy the per-base counters of [region_start, region_end) (computed by a separate
  * un-fused launch of the same pileup code).  Each pointer may be NULL. */
 int clb_debug_per_base(clb_ctx *ctx, uint32_t *raw, uint32_t *qc, uint32_t *low, uint8_t *state);
