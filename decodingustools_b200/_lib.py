@@ -56,9 +56,10 @@ SYMBOLS = [
     "clb_begin_contig", "clb_reserve", "clb_push_reads", "clb_finish_contig", "clb_host_alloc", "clb_host_free", "clb_wait_uploads",
     "clb_rerun_resident",
     "clb_counters_device", "clb_refresh_counters", "clb_set_nccl_allreduce", "clb_allreduce_nccl", "clb_debug_per_base",
-    "clb_set_depth_histogram", "clb_depth_histogram", "clb_set_depth_tiles", "clb_depth_tiles",
+    "clb_set_depth_histogram", "clb_depth_histogram", "clb_set_depth_tiles", "clb_depth_tiles", "clb_set_depth_runs", "clb_depth_runs",
     "clb_admit_reads", "clb_admit_reads_mt", "clb_admitter_new", "clb_admitter_push", "clb_admitter_free", "clb_compact_reads", "clb_bed_writer_open", "clb_bed_writer_add_contig", "clb_bed_writer_buffer",
     "clb_bed_writer_close", "clb_stitch_intervals", "clb_bin_geometry",
+    "clb_bedgraph_writer_open", "clb_bedgraph_writer_add_contig", "clb_bedgraph_writer_buffer", "clb_bedgraph_writer_close",
 ]
 
 _lib = None
@@ -97,6 +98,8 @@ def lib() -> C.CDLL:
     L.clb_depth_histogram.argtypes = [vp, C.POINTER(C.POINTER(u64)), C.POINTER(C.POINTER(u64)), C.POINTER(u32)]
     L.clb_set_depth_tiles.argtypes = [vp, u32]
     L.clb_depth_tiles.argtypes = [vp] + [C.POINTER(C.POINTER(u64))] * 4 + [C.POINTER(u32), C.POINTER(u32)]
+    L.clb_set_depth_runs.argtypes = [vp, C.c_int]
+    L.clb_depth_runs.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
     L.clb_admit_reads.argtypes = [i32, u32, u64, vp, vp, vp, vp, vp]
     L.clb_host_alloc.restype = vp
     L.clb_host_alloc.argtypes = [C.c_size_t]
@@ -114,6 +117,12 @@ def lib() -> C.CDLL:
     L.clb_bed_writer_buffer.restype = vp
     L.clb_bed_writer_buffer.argtypes = [vp, C.POINTER(u64)]
     L.clb_bed_writer_close.argtypes = [vp]
+    L.clb_bedgraph_writer_open.restype = vp
+    L.clb_bedgraph_writer_open.argtypes = [C.c_char_p]
+    L.clb_bedgraph_writer_add_contig.argtypes = [vp, C.c_char_p, u32, vp, u64]
+    L.clb_bedgraph_writer_buffer.restype = vp
+    L.clb_bedgraph_writer_buffer.argtypes = [vp, C.POINTER(u64)]
+    L.clb_bedgraph_writer_close.argtypes = [vp]
     L.clb_stitch_intervals.restype = u64
     L.clb_stitch_intervals.argtypes = [vp, vp, u32, vp]
     L.clb_bin_geometry.argtypes = [C.c_char_p, u32, u32, C.POINTER(u32), C.POINTER(u32)]

@@ -25,6 +25,8 @@ from .soa import ReadColumns
 
 INTERVAL_DTYPE = np.dtype([("start", "<u4"), ("end", "<u4"), ("state", "u1"), ("soft_start", "u1"), ("_pad", "<u2")])
 assert INTERVAL_DTYPE.itemsize == C.sizeof(_lib.Interval) == 12
+# clb_depth_run: a run of equal raw depth starts at `start` and ends where the next one starts (the last: at the region end)
+RUN_DTYPE = np.dtype([("start", "<u4"), ("depth", "<u4")])
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -71,6 +73,9 @@ class ContigDeviceResult:
     tile_callable: Optional[np.ndarray] = None
     tile_raw_sum: Optional[np.ndarray] = None
     tile_qc_sum: Optional[np.ndarray] = None
+    # depth runs (set_depth_runs): RUN_DTYPE[n], None when off.  The raw depth of every position of the region as runs of
+    # equal depth (depth_run_ends gives their ends); region shards join with stitch_depth_runs.
+    depth_runs: Optional[np.ndarray] = None
 
 
 def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDeviceResult:
@@ -86,6 +91,27 @@ def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDevice
                               iv, bins, int(res.stride), int(res.region_start), int(res.region_end), float(res.kernel_ms),
                               float(res.h2d_ms), float(res.pileup_ms), int(res.h2d_bytes), int(res.d2h_bytes), int(res.gpu_launches),
                               float(res.fast_ms), int(res.general_windows), float(res.upload_ms))
+
+
+def depth_run_ends(runs: np.ndarray, region_end: int) -> np.ndarray:
+    """End of each depth run: the next run's start, region_end for the last."""
+    starts = np.asarray(runs["start"], dtype=np.int64)
+    return np.append(starts[1:], np.int64(region_end)) if starts.size else np.zeros(0, np.int64)
+
+
+def stitch_depth_runs(shards: Sequence[np.ndarray]) -> np.ndarray:
+    """Concatenate the depth runs of region shards of one contig in genomic order, dropping a shard's first run when its
+    depth equals the previous shard's last (runs are defined by depth alone)."""
+    parts: List[np.ndarray] = []
+    last = None
+    for s in shards:
+        s = np.ascontiguousarray(s, dtype=RUN_DTYPE)
+        if s.size and last is not None and s["depth"][0] == last:
+            s = s[1:]
+        if s.size:
+            parts.append(s)
+            last = s["depth"][-1]
+    return np.concatenate(parts) if parts else np.zeros(0, RUN_DTYPE)
 
 
 def depth_tile_ranges(length: int, tile_len: int) -> Tuple[np.ndarray, np.ndarray]:
@@ -140,6 +166,10 @@ class CallableLociContext:
         the default) from the next begin_contig on."""
         self._check(self._L.clb_set_depth_tiles(self._h, int(tile_len)))
 
+    def set_depth_runs(self, on: bool):
+        """Runs of equal raw depth over every position of the region (off by default) from the next begin_contig on."""
+        self._check(self._L.clb_set_depth_runs(self._h, 1 if on else 0))
+
     def _with_optional_counts(self, r: ContigDeviceResult) -> ContigDeviceResult:
         raw = C.POINTER(C.c_uint64)(); qc = C.POINTER(C.c_uint64)(); n = C.c_uint32(0)
         self._check(self._L.clb_depth_histogram(self._h, C.byref(raw), C.byref(qc), C.byref(n)))
@@ -152,6 +182,12 @@ class CallableLociContext:
             r.tile_len = int(tl.value)
             r.tile_territory, r.tile_callable, r.tile_raw_sum, r.tile_qc_sum = (
                 np.ctypeslib.as_array(a, shape=(nt.value,)).copy() for a in arrs)
+        rp = C.c_void_p(0); nr = C.c_uint64(0)
+        self._check(self._L.clb_depth_runs(self._h, C.byref(rp), C.byref(nr)))
+        if rp.value:
+            n = int(nr.value)
+            r.depth_runs = (np.ctypeslib.as_array(C.cast(rp, C.POINTER(C.c_uint8)), shape=(n * 8,)).view(RUN_DTYPE).copy()
+                            if n else np.zeros(0, RUN_DTYPE))
         return r
 
     def set_stream(self, cuda_stream: int):
@@ -317,6 +353,41 @@ class ContigProfiler:
     n_reads: int = 0
     bins: Optional[np.ndarray] = None
     stride: int = 0
+
+
+class BedGraphWriter:
+    """Depth runs as bedGraph text (clb_bedgraph_writer): "name\tstart\tend\tdepth" lines, contigs in the order added."""
+
+    def __init__(self, path: Optional[str]):
+        self._L = _lib.lib()
+        self.path = path
+        self._w = self._L.clb_bedgraph_writer_open(path.encode() if path else None)
+        if not self._w:
+            raise ClbError(_lib.CLB_E_IO, f"cannot create {path}")
+
+    def add_contig(self, name: str, length: int, runs: np.ndarray):
+        r = np.ascontiguousarray(runs, dtype=RUN_DTYPE)
+        rc = self._L.clb_bedgraph_writer_add_contig(self._w, name.encode(), int(length), _ptr(r), r.shape[0])
+        if rc != 0:
+            raise ClbError(rc, f"cannot write {self.path}" if rc == _lib.CLB_E_IO else f"depth runs of {name} do not tile [0,{length})")
+
+    def text(self) -> bytes:
+        n = C.c_uint64(0)
+        p = self._L.clb_bedgraph_writer_buffer(self._w, C.byref(n))
+        return C.string_at(p, n.value) if n.value else b""
+
+    def close(self):
+        if self._w:
+            w, self._w = self._w, None
+            rc = self._L.clb_bedgraph_writer_close(w)
+            if rc != 0:
+                raise ClbError(rc, f"cannot write {self.path}")
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class CallableProfiler:

@@ -55,6 +55,8 @@ struct clb_ctx {
     uint32_t tl_next = 0, tl_len = 0;   // depth-tile length: set by clb_set_depth_tiles, in force for the current contig
     uint32_t n_tiles = 0;               // ceil(contig_len / tl_len) while on
     uint32_t tl_fetched = 0;            // tiles in the result of the last fetch (clb_depth_tiles)
+    bool runs_next = false, runs = false;   // depth runs: set by clb_set_depth_runs, in force for the current contig
+    bool runs_fetched = false;              // ... and in the result of the last fetch (clb_depth_runs)
     bool long_mode = false, span_on_device = false;
     uint64_t n_reads = 0, n_cigar = 0, n_qual = 0;
     long long last_pos = -1;
@@ -63,6 +65,7 @@ struct clb_ctx {
     DevBuf nmask, ref_ascii;
     DevBuf stats_padded, counters, rec, win_tab, win_rec, win_out, deep_list, intervals, misc;
     DevBuf gen_list, blk_tot, dhist;
+    DevBuf run_rec, run_win_tab, runs_out;   // depth runs: records, window table, compacted runs (region length each)
     DevBuf dbg_raw, dbg_qc, dbg_low, dbg_state, timing;
     uint32_t rec_cap = 0;
     bool dbg = false;
@@ -76,11 +79,16 @@ struct clb_ctx {
     uint64_t h2d_bytes = 0, d2h_bytes = 0;
     uint32_t launches = 0;
     uint64_t n_intervals = 0;
+    clb_depth_run *h_runs = nullptr;       // pinned
+    size_t h_runs_cap = 0;
+    uint64_t n_runs = 0;
 };
 
 // misc layout (uint32): record cursor, error bits, n_total intervals, deep-window count, general-queue count / tickets taken
-// (these six are reset per run), then the maximum reference span
-enum { M_CURSOR = 0, M_ERR = 1, M_NTOTAL = 2, M_DEEP = 3, M_GEN_COUNT = 4, M_GEN_TAKEN = 5, M_RESET_WORDS = 6, M_MAXSPAN = 7, M_MAXQLEN = 8, M_WORDS = 9 };
+// (these six are reset per run), then the maximum reference span; with depth runs on, the run cursor and run count follow
+// (reset per run too, and only copied then)
+enum { M_CURSOR = 0, M_ERR = 1, M_NTOTAL = 2, M_DEEP = 3, M_GEN_COUNT = 4, M_GEN_TAKEN = 5, M_RESET_WORDS = 6, M_MAXSPAN = 7, M_MAXQLEN = 8, M_WORDS = 9,
+       M_RUN_CURSOR = 9, M_RUN_NTOTAL = 10, M_WORDS_RUNS = 11 };
 
 namespace {
 
@@ -163,6 +171,10 @@ KParams make_params(clb_ctx *c) {
     P.timing = (long long *)c->timing.p;
     P.dhist = c->dh_n ? (unsigned long long *)c->dhist.p : nullptr; P.dh_n = c->dh_n;
     P.tiles = c->tl_len ? (unsigned long long *)c->counters.p + tiles_offset(c) : nullptr; P.tile_len = c->tl_len; P.n_tiles = c->n_tiles;
+    if (c->runs) {
+        P.run_rec = (uint2 *)c->run_rec.p; P.run_cursor = (uint32_t *)c->misc.p + M_RUN_CURSOR; P.run_win_tab = (uint4 *)c->run_win_tab.p;
+        P.run_cap = c->region_end - c->region_start;
+    }
     if (c->dbg) {
         P.dbg_raw = (uint32_t *)c->dbg_raw.p; P.dbg_qc = (uint32_t *)c->dbg_qc.p;
         P.dbg_low = (uint32_t *)c->dbg_low.p; P.dbg_state = (uint8_t *)c->dbg_state.p;
@@ -171,24 +183,29 @@ KParams make_params(clb_ctx *c) {
 }
 
 // The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
-// with the per-base dump (parity tests), FEAT the optional counts that are on (FEAT_HIST: depth histograms, FEAT_TILES: depth
-// tiles; only launched when on, so the others stay as they were).  f is called with two std::integral_constant<bool, ...>
-// and one std::integral_constant<unsigned, FEAT>.
+// with the per-base dump (parity tests), FEAT the optional outputs that are on (FEAT_HIST: depth histograms, FEAT_TILES:
+// depth tiles, FEAT_RUNS: depth runs; only launched when on, so the others stay as they were).  f is called with two
+// std::integral_constant<bool, ...> and one std::integral_constant<unsigned, FEAT>.
+template <unsigned X> using FeatC = std::integral_constant<unsigned, X>;
 template <typename F>
 void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
     using T = std::true_type; using N = std::false_type;
     auto h = [&](auto b, auto d) {
         switch (feat) {
-        case 0: f(b, d, std::integral_constant<unsigned, 0u>{}); break;
-        case FEAT_HIST: f(b, d, std::integral_constant<unsigned, FEAT_HIST>{}); break;
-        case FEAT_TILES: f(b, d, std::integral_constant<unsigned, FEAT_TILES>{}); break;
-        default: f(b, d, std::integral_constant<unsigned, FEAT_HIST | FEAT_TILES>{}); break;
+        case 0: f(b, d, FeatC<0u>{}); break;
+        case 1: f(b, d, FeatC<1u>{}); break;
+        case 2: f(b, d, FeatC<2u>{}); break;
+        case 3: f(b, d, FeatC<3u>{}); break;
+        case 4: f(b, d, FeatC<4u>{}); break;
+        case 5: f(b, d, FeatC<5u>{}); break;
+        case 6: f(b, d, FeatC<6u>{}); break;
+        default: f(b, d, FeatC<7u>{}); break;
         }
     };
     if (bq_hi) { if (dbg) h(T{}, T{}); else h(T{}, N{}); }
     else { if (dbg) h(N{}, T{}); else h(N{}, N{}); }
 }
-unsigned features(const clb_ctx *c) { return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u); }
+unsigned features(const clb_ctx *c) { return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u) | (c->runs ? FEAT_RUNS : 0u); }
 
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
 // queue of windows the other two handed over) for windows [w0, w1) on the compute stream
@@ -228,6 +245,7 @@ int reset_accumulators(clb_ctx *ctx) {
     CU(cudaMemsetAsync(ctx->counters.p, 0, n_counters(ctx) * 8, ctx->s_compute));
     if (ctx->dh_n) CU(cudaMemsetAsync(ctx->dhist.p, 0, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, ctx->s_compute));
     CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_CURSOR, 0, M_RESET_WORDS * sizeof(uint32_t), ctx->s_compute));   // cursor, err, n_total, deep windows, general queue
+    if (ctx->runs) CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_RUN_CURSOR, 0, 2 * sizeof(uint32_t), ctx->s_compute));   // run cursor, run count
     return CLB_OK;
 }
 
@@ -242,11 +260,11 @@ int launch_compaction(clb_ctx *ctx) {
         ctx->launches += 1;
     }
     const uint32_t n_blk = (ctx->n_windows + 1023) / 1024;
-    k_scan_windows_local<<<n_blk, 1024, 0, ctx->s_compute>>>((const uint2 *)ctx->win_tab.p, ctx->n_windows, (uint32_t *)ctx->win_out.p,
+    k_scan_windows_local<uint2><<<n_blk, 1024, 0, ctx->s_compute>>>((const uint2 *)ctx->win_tab.p, ctx->n_windows, (uint32_t *)ctx->win_out.p,
                                                             (uint32_t *)ctx->blk_tot.p, (const uint32_t *)ctx->misc.p + M_ERR);
     k_scan_blocks<<<1, 1024, 0, ctx->s_compute>>>((uint32_t *)ctx->blk_tot.p, n_blk, (uint32_t *)ctx->misc.p + M_NTOTAL);
     const uint32_t warps_per_block = 8;
-    k_gather_intervals<<<(ctx->n_windows + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, ctx->s_compute>>>(
+    k_gather_intervals<uint2, unsigned long long, IntervalOut><<<(ctx->n_windows + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, ctx->s_compute>>>(
         (const unsigned long long *)ctx->rec.p, (const uint2 *)ctx->win_tab.p, (const uint32_t *)ctx->win_out.p,
         (const uint32_t *)ctx->blk_tot.p, ctx->n_windows, (IntervalOut *)ctx->intervals.p, (const uint32_t *)ctx->misc.p + M_ERR);
     k_fill_ends<<<std::max(1, ctx->n_sm * 4), 256, 0, ctx->s_compute>>>((IntervalOut *)ctx->intervals.p,
@@ -259,6 +277,16 @@ int launch_compaction(clb_ctx *ctx) {
         k_fold_depth_hist<<<(n2 + 255) / 256, 256, 0, ctx->s_compute>>>((const unsigned long long *)ctx->dhist.p, n2,
                                                                      (unsigned long long *)ctx->counters.p + N_STATS + 3 * (size_t)ctx->n_bins);
         ctx->launches += 1;
+    }
+    if (ctx->runs) {
+        // the depth runs through the same scan and gather (win_out / blk_tot are free again: the interval gather is done)
+        k_scan_windows_local<uint4><<<n_blk, 1024, 0, ctx->s_compute>>>((const uint4 *)ctx->run_win_tab.p, ctx->n_windows, (uint32_t *)ctx->win_out.p,
+                                                                       (uint32_t *)ctx->blk_tot.p, (const uint32_t *)ctx->misc.p + M_ERR);
+        k_scan_blocks<<<1, 1024, 0, ctx->s_compute>>>((uint32_t *)ctx->blk_tot.p, n_blk, (uint32_t *)ctx->misc.p + M_RUN_NTOTAL);
+        k_gather_intervals<uint4, uint2, uint2><<<(ctx->n_windows + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, ctx->s_compute>>>(
+            (const uint2 *)ctx->run_rec.p, (const uint4 *)ctx->run_win_tab.p, (const uint32_t *)ctx->win_out.p,
+            (const uint32_t *)ctx->blk_tot.p, ctx->n_windows, (uint2 *)ctx->runs_out.p, (const uint32_t *)ctx->misc.p + M_ERR);
+        ctx->launches += 3;
     }
     CU(cudaGetLastError());
     return CLB_OK;
@@ -275,15 +303,23 @@ int alloc_outputs(clb_ctx *ctx) {
     if ((rc = ensure(ctx, ctx->blk_tot, ((nw + 1023) / 1024 + 1) * 4, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->rec, (size_t)ctx->rec_cap * 8, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->intervals, (size_t)ctx->rec_cap * sizeof(IntervalOut), false, ctx->s_compute))) return rc;
+    if (ctx->runs) {
+        // a position starts at most one run: the region length bounds the records and the runs, so they never overflow
+        const size_t rlen = ctx->region_end - ctx->region_start;
+        if ((rc = ensure(ctx, ctx->run_win_tab, nw * sizeof(uint4), false, ctx->s_compute))) return rc;
+        if ((rc = ensure(ctx, ctx->run_rec, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
+        if ((rc = ensure(ctx, ctx->runs_out, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
+    }
     return CLB_OK;
 }
 
 // copy counters + interval count, validate device error bits, then copy the intervals
 int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     const size_t n_cnt = n_counters(ctx);
-    ctx->dh_fetched = 0; ctx->tl_fetched = 0;
+    const size_t n_misc = ctx->runs ? M_WORDS_RUNS : M_WORDS;
+    ctx->dh_fetched = 0; ctx->tl_fetched = 0; ctx->runs_fetched = false;
     ctx->h_counters.resize(n_cnt);
-    CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, M_WORDS * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
+    CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, n_misc * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaMemcpyAsync(ctx->h_counters.data(), ctx->counters.p, n_cnt * 8, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaStreamSynchronize(ctx->s_compute));
     const uint32_t e = ctx->h_misc[M_ERR];
@@ -303,11 +339,26 @@ int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
         CU(cudaStreamSynchronize(ctx->s_compute));
     }
     ctx->n_intervals = n_iv;
-    ctx->d2h_bytes = M_WORDS * 4 + n_cnt * 8 + n_iv * sizeof(clb_interval);
+    const uint64_t n_runs = ctx->runs && ctx->n_windows ? ctx->h_misc[M_RUN_NTOTAL] : 0;
+    if (ctx->runs) {
+        if (n_runs > ctx->h_runs_cap || !ctx->h_runs) {
+            if (ctx->h_runs) cudaFreeHost(ctx->h_runs);
+            ctx->h_runs = nullptr;
+            ctx->h_runs_cap = std::max<size_t>(n_runs + n_runs / 4, 1024);
+            CU(cudaHostAlloc((void **)&ctx->h_runs, ctx->h_runs_cap * sizeof(clb_depth_run), cudaHostAllocDefault));
+        }
+        if (n_runs) {
+            CU(cudaMemcpyAsync(ctx->h_runs, ctx->runs_out.p, n_runs * sizeof(clb_depth_run), cudaMemcpyDeviceToHost, ctx->s_compute));
+            CU(cudaStreamSynchronize(ctx->s_compute));
+        }
+    }
+    ctx->n_runs = n_runs;
+    ctx->d2h_bytes = n_misc * 4 + n_cnt * 8 + n_iv * sizeof(clb_interval) + n_runs * sizeof(clb_depth_run);
     ctx->h_bins.resize(3 * (size_t)ctx->n_bins);
     for (size_t i = 0; i < ctx->h_bins.size(); i++) ctx->h_bins[i] = (uint32_t)ctx->h_counters[N_STATS + i];
     ctx->dh_fetched = ctx->dh_n;                                             // the histograms stay in h_counters, after the bins
     ctx->tl_fetched = ctx->n_tiles;                                          // ... and the tiles after them
+    ctx->runs_fetched = ctx->runs;
 
     float kms = 0, hms = 0, ums = 0;
     for (auto &ep : ctx->ev_upload) { float t = 0; cudaEventElapsedTime(&t, ep.a, ep.b); ums += t; ctx->ev_pool.push_back(ep); }
@@ -400,7 +451,7 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-    for (int v = 0; v < 16; v++)                             // every instantiation of the pileup kernels
+    for (int v = 0; v < 32; v++)                             // every instantiation of the pileup kernels
         with_variant(v & 1, v & 2, (unsigned)v >> 2, [&](auto h, auto d, auto x) {
             constexpr bool H = decltype(h)::value, D = decltype(d)::value; constexpr unsigned X = decltype(x)::value;
             const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
@@ -414,7 +465,7 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
     if ((e = cudaMalloc((void **)&ctx->d_first_tab, 65536 * 4 + WIN_TABLE_BYTES + 256)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaMalloc", e); }
     k_first_table<<<65536 / 256, 256, 0, ctx->s_compute>>>(ctx->d_first_tab, (uint8_t *)(ctx->d_first_tab + 65536) + WIN_TABLE_BYTES, opt->max_low_mapq_fraction);
     k_window_tables<<<1, 256, 0, ctx->s_compute>>>(ctx->d_first_tab + 65536, opt->max_low_mapq_fraction);
-    if ((e = cudaHostAlloc((void **)&ctx->h_misc, M_WORDS * 4, cudaHostAllocDefault)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaHostAlloc", e); }
+    if ((e = cudaHostAlloc((void **)&ctx->h_misc, M_WORDS_RUNS * 4, cudaHostAllocDefault)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaHostAlloc", e); }
     if ((e = cudaStreamSynchronize(ctx->s_compute)) != cudaSuccess) { clb_destroy(ctx); return bail("first-table kernel", e); }
     return ctx;
 }
@@ -425,10 +476,11 @@ void clb_destroy(clb_ctx *ctx) {
     cudaDeviceSynchronize();
     for (DevBuf *b : {&ctx->pos, &ctx->flag, &ctx->mapq, &ctx->cigar_off, &ctx->cigar, &ctx->qual_off, &ctx->qual, &ctx->read_end, &ctx->cigar_ckpt,
                       &ctx->nmask, &ctx->ref_ascii, &ctx->stats_padded, &ctx->counters, &ctx->rec, &ctx->win_tab, &ctx->win_rec,
-                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dhist, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
+                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dhist, &ctx->run_rec, &ctx->run_win_tab, &ctx->runs_out, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
         release(*b);
     if (ctx->d_first_tab) cudaFree(ctx->d_first_tab);
     if (ctx->h_intervals) cudaFreeHost(ctx->h_intervals);
+    if (ctx->h_runs) cudaFreeHost(ctx->h_runs);
     if (ctx->h_misc) cudaFreeHost(ctx->h_misc);
     for (auto &ep : ctx->ev_pool) { cudaEventDestroy(ep.a); cudaEventDestroy(ep.b); }
     for (auto &ep : ctx->ev_kernel) { cudaEventDestroy(ep.a); cudaEventDestroy(ep.b); }
@@ -474,6 +526,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     ctx->dbg = false;
     ctx->dh_n = ctx->dh_next; ctx->dh_fetched = 0;
     ctx->tl_len = ctx->tl_next; ctx->tl_fetched = 0;
+    ctx->runs = ctx->runs_next; ctx->runs_fetched = false; ctx->n_runs = 0;
     ctx->n_tiles = ctx->tl_len ? (uint32_t)(((uint64_t)contig_len + ctx->tl_len - 1) / ctx->tl_len) : 0u;
     clb_bin_geometry(ctx->name.c_str(), contig_len, largest_contig_len, &ctx->stride, &ctx->n_bins);
 
@@ -509,7 +562,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     CU(cudaEventRecord(ep.b, ctx->s_compute));
     ctx->ev_h2d.push_back(ep);
 
-    if ((rc = ensure(ctx, ctx->misc, M_WORDS * 4, false, ctx->s_compute))) return rc;
+    if ((rc = ensure(ctx, ctx->misc, M_WORDS_RUNS * 4, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->stats_padded, (size_t)N_STATS * STAT_STRIDE * 8, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->counters, n_counters(ctx) * 8, false, ctx->s_compute))) return rc;
     if (ctx->dh_n && (rc = ensure(ctx, ctx->dhist, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, false, ctx->s_compute))) return rc;
@@ -737,6 +790,20 @@ int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64
     if (qc_sum) *qc_sum = n ? t + 3 * (size_t)n : nullptr;
     if (n_tiles) *n_tiles = n;
     if (tile_len) *tile_len = n ? ctx->tl_len : 0u;
+    return CLB_OK;
+}
+
+int clb_set_depth_runs(clb_ctx *ctx, int on) {
+    if (!ctx) return CLB_E_INVALID;
+    if (ctx->in_contig && !ctx->finished) return fail(ctx, CLB_E_INVALID, "clb_set_depth_runs while a contig is open");
+    ctx->runs_next = on != 0;
+    return CLB_OK;
+}
+
+int clb_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_runs) {
+    if (!ctx) return CLB_E_INVALID;
+    if (runs) *runs = ctx->runs_fetched ? ctx->h_runs : nullptr;
+    if (n_runs) *n_runs = ctx->runs_fetched ? ctx->n_runs : 0;
     return CLB_OK;
 }
 

@@ -51,9 +51,10 @@ constexpr int F_OFF_LAST = F_OFF_SCAN + 64 * 4;
 constexpr int F_OFF_WSTATS = F_OFF_LAST + NT;
 constexpr int F_OFF_HIST = F_OFF_WSTATS + NWARPS * N_STATS * 8;    // depth table (HIST instantiations), 2 x DH_TAB u32
 constexpr int F_OFF_TILE = F_OFF_HIST + 2 * DH_TAB * 4;              // tile slots (TILES instantiations), TL_SLOT_BYTES
+constexpr int F_OFF_RUN = F_OFF_TILE + TL_SLOT_BYTES;                 // per warp its last raw depth (RUNS instantiations), u32
 static_assert(F_OFF_STAGE % 16 == 0 && F_WSTAGE % 16 == 0, "bulk copies need 16-byte aligned destinations");
 static_assert(F_OFF_WSTATS % 8 == 0 && F_OFF_BAR % 8 == 0 && F_OFF_X % 8 == 0 && F_OFF_MASK % 16 == 0 && F_OFF_FIRST % 16 == 0, "alignment");
-static_assert(F_OFF_TILE + TL_SLOT_BYTES <= F_OFF_X, "phase C scratch fits the stages");
+static_assert(F_OFF_RUN + NWARPS * 4 <= F_OFF_X, "phase C scratch fits the stages");
 static_assert(CLB_F_MINB * (F_SMEM + 1024) <= 228 * 1024, "shared memory per SM");
 enum { FC_BAIL = 0, FC_XCNT = 1 };
 
@@ -176,7 +177,7 @@ __device__ __forceinline__ void fmeta_load(const KParams &P, FMeta &M, uint32_t 
 
 template <bool BQ_HI, bool DBG, unsigned FEAT = 0u>
 __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P) {
-    constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0;
+    constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0, RUNS = (FEAT & FEAT_RUNS) != 0;
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint32_t w = P.win_first + blockIdx.x;
     // one table record per window, three independent 16-byte loads (no dependent round trip)
@@ -391,6 +392,9 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     }
     if constexpr (HIST) close_depth_runs<true>(dh);
     close_entries(e, n_ent, sLast, sScan);
+    const auto raw_of = [&](int k) { return a[k] & 0xffffu; };            // not the packed word: its high half is the low-MAPQ depth
+    uint32_t *sRunLast = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_RUN);
+    if constexpr (RUNS) publish_run_depth(e, n_ent, raw_of, sRunLast, sScan);
     dbg_dump<DBG>(e, w * (uint32_t)WREAL, [&](int k) { return make_uint3(a[k] & 0xffffu, qcv[k], a[k] >> 16); }, P);
     unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(smem_raw + F_OFF_TILE);
     uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
@@ -398,9 +402,10 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
     if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
     if constexpr (TILES) flush_tiles(sTileSum, sTileFirst, P);
-    // the window's first position always starts a record (window soft: the interval gather drops it when the previous
-    // window ended in the same state)
-    write_records(e, wb0, 0u, 0u, w > 0 ? 1u : 0u, sLast, sScan, w, P);
+    // the window's first position always starts a record and a depth run (window soft: the gather drops them when the
+    // previous window ended in the same state / at the same raw depth)
+    const uint32_t rmask = RUNS ? run_starts(e, raw_of, 0u, sRunLast) : 0u;
+    write_records<RUNS>(e, wb0, 0u, 0u, w > 0 ? 1u : 0u, sLast, sScan, w, P, rmask, raw_of);
     add_bins(e, wb0, 0u, n_ent, wr.z, wr.w - 1u, P);                       // k_window_ranges counts the next bin's entry from the halo
     CLB_STAMP(6);
     CLB_STAMP_VALUE(7, r_hi - r_lo);

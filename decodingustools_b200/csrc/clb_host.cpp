@@ -4,6 +4,7 @@
 //   clb_bed_writer_*       CallableProfiler::write_state / finish_contig incl. the cross-contig quirks,
 //                          /root/reference/src/callable_loci/profilers/callable_profiler.rs:39-87,122-155
 //   clb_stitch_intervals   region-shard stitching (multi-GPU, SURVEY.md section 8(e))
+//   clb_bedgraph_writer_*  depth runs as bedGraph text (not in the reference)
 #include "../../include/callable_loci_b200.h"
 
 #include <algorithm>
@@ -295,15 +296,12 @@ extern "C" uint64_t clb_stitch_intervals(const clb_interval *const *shards, cons
     return n;
 }
 
-struct clb_bed_writer {
+// Where a text writer's output goes (a stdio file or memory) and the text formatting of large contigs on several threads.
+struct TextSink {
     FILE *fp = nullptr;
     std::string mem;
     bool in_memory = false;
     bool io_failed = false;        // the first failed stdio / pwrite call; add_contig and close report it as CLB_E_IO
-    uint32_t largest = 0;
-    bool have_pending = false;     // CallableProfiler::current_state survives finish_contig (quirk Q1)
-    std::string pend_name;
-    clb_interval pend{};
     std::vector<char> buf;
     struct Part { std::unique_ptr<char[]> p; size_t cap = 0; };
     std::vector<Part> parts;                // per-thread formatting buffers (reused, never zero-filled)
@@ -317,6 +315,75 @@ struct clb_bed_writer {
     void flush() {
         if (fp && !buf.empty()) { if (fwrite(buf.data(), 1, buf.size(), fp) != buf.size()) io_failed = true; buf.clear(); }
     }
+    bool open(const char *path) {
+        if (!path) { in_memory = true; return true; }
+        fp = fopen(path, "wb");
+        return fp != nullptr;
+    }
+    int close() {
+        if (fp) { flush(); if (fclose(fp) != 0) io_failed = true; }
+        return io_failed ? CLB_E_IO : CLB_OK;
+    }
+    // Items [0, n) as text, in order: format(part, lo, hi) writes the text of items [lo, hi) into part (growing it) and
+    // returns its length.  From 65536 items on (the BED text of a 30x human chromosome is ~100 MB) nt threads format one
+    // slice each, then the parts are copied / pwritten to their final offsets in parallel (written in order to a pipe).
+    template <typename Format>
+    void put_items(uint64_t n, const char *what, Format format) {
+        const uint32_t nt = n < (1u << 16) ? 1 : clb_host_threads();
+        if (parts.size() < nt) parts.resize(nt);
+        if (nt == 1) { put(parts[0].p.get(), format(parts[0], (uint64_t)0, n)); return; }
+        const bool dbg_t = getenv("CLB_ADMIT_DEBUG") != nullptr;
+        auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+        const double t0 = now();
+        std::vector<size_t> sizes(nt, 0);
+        const uint64_t per = (n + nt - 1) / nt;
+        auto run_threads = [&](auto &&fn) {
+            std::vector<std::thread> th;
+            for (uint32_t t = 1; t < nt; t++) th.emplace_back(fn, t);
+            fn(0);
+            for (auto &x : th) x.join();
+        };
+        run_threads([&](uint32_t t) {
+            const uint64_t lo = std::min(n, t * per), hi = std::min(n, lo + per);
+            sizes[t] = format(parts[t], lo, hi);
+        });
+        const double t1 = now();
+        std::vector<size_t> off(nt + 1, 0);
+        for (uint32_t t = 0; t < nt; t++) off[t + 1] = off[t] + sizes[t];
+        if (in_memory) {
+            const size_t base = mem.size();
+            mem.resize(base + off[nt]);
+            run_threads([&](uint32_t t) { memcpy(&mem[base + off[t]], parts[t].p.get(), sizes[t]); });
+        } else {
+            flush();
+            if (fflush(fp) != 0) io_failed = true;
+            const off_t base = ftello(fp);
+            if (base >= 0) {                                     // a seekable file: every part goes straight to its offset
+                const int fd = fileno(fp);
+                std::atomic<bool> io_err{false};
+                run_threads([&](uint32_t t) {
+                    size_t done = 0;
+                    while (done < sizes[t]) {
+                        const ssize_t r = pwrite(fd, parts[t].p.get() + done, sizes[t] - done, base + (off_t)(off[t] + done));
+                        if (r <= 0) { io_err = true; break; }
+                        done += (size_t)r;
+                    }
+                });
+                if (io_err || fseeko(fp, base + (off_t)off[nt], SEEK_SET) != 0) io_failed = true;
+            } else {                                             // a pipe or a terminal: in order
+                for (uint32_t t = 0; t < nt; t++)
+                    if (fwrite(parts[t].p.get(), 1, sizes[t], fp) != sizes[t]) io_failed = true;
+            }
+        }
+        if (dbg_t) fprintf(stderr, "%s: %u threads, format %.3f s, output %.3f s (%zu bytes)\n", what, nt, t1 - t0, now() - t1, off[nt]);
+    }
+};
+
+struct clb_bed_writer : TextSink {
+    uint32_t largest = 0;
+    bool have_pending = false;     // CallableProfiler::current_state survives finish_contig (quirk Q1)
+    std::string pend_name;
+    clb_interval pend{};
 };
 
 static const uint8_t kStateLen[6] = {5, 8, 11, 12, 18, 20};
@@ -336,7 +403,7 @@ static inline bool binned_state(uint8_t s) { return s == CLB_CALLABLE || s == CL
 
 // The BED lines of iv[lo, hi) (states already validated) into out; returns their length.  *binned |= whether one of them
 // has a binned state.
-static size_t format_lines(clb_bed_writer::Part &out, const std::string &name, const clb_interval *iv, uint64_t lo, uint64_t hi, bool *binned) {
+static size_t format_lines(TextSink::Part &out, const std::string &name, const clb_interval *iv, uint64_t lo, uint64_t hi, bool *binned) {
     const size_t max_line = name.size() + 1 + 10 + 1 + 10 + 1 + 20 + 1;
     if (out.cap < (size_t)(hi - lo) * max_line) { out.cap = (size_t)(hi - lo) * max_line; out.p.reset(new char[out.cap]); }
     char *p = out.p.get();
@@ -355,9 +422,7 @@ static size_t format_lines(clb_bed_writer::Part &out, const std::string &name, c
 extern "C" clb_bed_writer *clb_bed_writer_open(const char *path, uint32_t largest_contig_len) {
     clb_bed_writer *w = new clb_bed_writer();
     w->largest = largest_contig_len;
-    if (!path) { w->in_memory = true; return w; }
-    w->fp = fopen(path, "wb");                                // File::create truncates: callable_profiler.rs:31
-    if (!w->fp) { delete w; return nullptr; }
+    if (!w->open(path)) { delete w; return nullptr; }         // File::create truncates: callable_profiler.rs:31
     return w;
 }
 
@@ -373,10 +438,8 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
     }
     if (expect != contig_len) return CLB_E_INPUT;
     const std::string nm(name);
-    // large contigs are formatted on several threads (BED text of a 30x human chromosome is ~100 MB)
-    const uint32_t nt = n_iv < (1u << 16) ? 1 : clb_host_threads();
-    if (w->parts.size() < nt) w->parts.resize(nt);
     bool any_range = false;
+    if (w->parts.empty()) w->parts.resize(1);
     // Q1: the first position of a contig (or finish_contig of an empty one) flushes the previous contig's
     // last run once more; Q2: that flush also pushes it into THIS contig's coverage_ranges.
     if (w->have_pending) {
@@ -397,58 +460,14 @@ extern "C" int clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, ui
             }
         }
     }
-    if (nt == 1) {
-        w->put(w->parts[0].p.get(), format_lines(w->parts[0], nm, iv, 0, n_iv, &any_range));
-    } else {
-        // each thread formats into its own reusable buffer, then the parts are copied / pwritten to their final offsets in parallel
-        const bool dbg_t = getenv("CLB_ADMIT_DEBUG") != nullptr;
-        auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-        const double t0 = now();
-        std::vector<size_t> sizes(nt, 0);
-        std::vector<int> binned(nt, 0);
-        const uint64_t per = (n_iv + nt - 1) / nt;
-        auto run_threads = [&](auto &&fn) {
-            std::vector<std::thread> th;
-            for (uint32_t t = 1; t < nt; t++) th.emplace_back(fn, t);
-            fn(0);
-            for (auto &x : th) x.join();
-        };
-        run_threads([&](uint32_t t) {
-            const uint64_t lo = std::min(n_iv, t * per), hi = std::min(n_iv, lo + per);
-            bool b = false;
-            sizes[t] = format_lines(w->parts[t], nm, iv, lo, hi, &b);
-            binned[t] = b;
-        });
-        const double t1 = now();
-        std::vector<size_t> off(nt + 1, 0);
-        for (uint32_t t = 0; t < nt; t++) { off[t + 1] = off[t] + sizes[t]; if (binned[t]) any_range = true; }
-        if (w->in_memory) {
-            const size_t base = w->mem.size();
-            w->mem.resize(base + off[nt]);
-            run_threads([&](uint32_t t) { memcpy(&w->mem[base + off[t]], w->parts[t].p.get(), sizes[t]); });
-        } else {
-            w->flush();
-            if (fflush(w->fp) != 0) w->io_failed = true;
-            const off_t base = ftello(w->fp);
-            if (base >= 0) {                                     // a seekable file: every part goes straight to its offset
-                const int fd = fileno(w->fp);
-                std::atomic<bool> io_err{false};
-                run_threads([&](uint32_t t) {
-                    size_t done = 0;
-                    while (done < sizes[t]) {
-                        const ssize_t r = pwrite(fd, w->parts[t].p.get() + done, sizes[t] - done, base + (off_t)(off[t] + done));
-                        if (r <= 0) { io_err = true; break; }
-                        done += (size_t)r;
-                    }
-                });
-                if (io_err || fseeko(w->fp, base + (off_t)off[nt], SEEK_SET) != 0) w->io_failed = true;
-            } else {                                             // a pipe or a terminal: in order
-                for (uint32_t t = 0; t < nt; t++)
-                    if (fwrite(w->parts[t].p.get(), 1, sizes[t], w->fp) != sizes[t]) w->io_failed = true;
-            }
-        }
-        if (dbg_t) fprintf(stderr, "clb_bed_writer_add_contig: %u threads, format %.3f s, output %.3f s (%zu bytes)\n", nt, t1 - t0, now() - t1, off[nt]);
-    }
+    std::atomic<bool> binned{false};
+    w->put_items(n_iv, "clb_bed_writer_add_contig", [&](TextSink::Part &part, uint64_t lo, uint64_t hi) {
+        bool b = false;
+        const size_t len = format_lines(part, nm, iv, lo, hi, &b);
+        if (b) binned = true;
+        return len;
+    });
+    if (binned) any_range = true;
     if (n_iv) { w->have_pending = true; w->pend_name = nm; w->pend = iv[n_iv - 1]; }
     if (has_bins) *has_bins = any_range ? 1 : 0;
     return w->io_failed ? CLB_E_IO : CLB_OK;
@@ -462,8 +481,58 @@ extern "C" const char *clb_bed_writer_buffer(clb_bed_writer *w, uint64_t *len) {
 
 extern "C" int clb_bed_writer_close(clb_bed_writer *w) {
     if (!w) return CLB_E_INVALID;
-    if (w->fp) { w->flush(); if (fclose(w->fp) != 0) w->io_failed = true; }
-    const int rc = w->io_failed ? CLB_E_IO : CLB_OK;
+    const int rc = w->close();
+    delete w;
+    return rc;
+}
+
+struct clb_bedgraph_writer : TextSink {};
+
+// The bedGraph lines of runs[lo, hi) (runs[hi] or contig_len ends run hi - 1) into out; returns their length.
+static size_t format_runs(TextSink::Part &out, const std::string &name, uint32_t contig_len, const clb_depth_run *runs, uint64_t n,
+                          uint64_t lo, uint64_t hi) {
+    const size_t max_line = name.size() + 1 + 10 + 1 + 10 + 1 + 10 + 1;
+    if (out.cap < (size_t)(hi - lo) * max_line) { out.cap = (size_t)(hi - lo) * max_line; out.p.reset(new char[out.cap]); }
+    char *p = out.p.get();
+    for (uint64_t i = lo; i < hi; i++) {
+        memcpy(p, name.data(), name.size()); p += name.size();
+        *p++ = '\t'; p = put_u32_fast(p, runs[i].start); *p++ = '\t'; p = put_u32_fast(p, i + 1 < n ? runs[i + 1].start : contig_len);
+        *p++ = '\t'; p = put_u32_fast(p, runs[i].depth); *p++ = '\n';
+    }
+    return (size_t)(p - out.p.get());
+}
+
+extern "C" clb_bedgraph_writer *clb_bedgraph_writer_open(const char *path) {
+    clb_bedgraph_writer *w = new clb_bedgraph_writer();
+    if (!w->open(path)) { delete w; return nullptr; }
+    return w;
+}
+
+extern "C" int clb_bedgraph_writer_add_contig(clb_bedgraph_writer *w, const char *name, uint32_t contig_len, const clb_depth_run *runs,
+                                              uint64_t n) {
+    if (!w || !name || (n && !runs)) return CLB_E_INVALID;
+    // runs must tile [0, contig_len): the first starts at 0, starts ascend strictly, the last starts before contig_len
+    if ((n == 0) != (contig_len == 0)) return CLB_E_INVALID;
+    for (uint64_t i = 0; i < n; i++) {
+        if (i == 0 ? runs[0].start != 0 : runs[i].start <= runs[i - 1].start) return CLB_E_INVALID;
+    }
+    if (n && runs[n - 1].start >= contig_len) return CLB_E_INVALID;
+    const std::string nm(name);
+    w->put_items(n, "clb_bedgraph_writer_add_contig", [&](TextSink::Part &part, uint64_t lo, uint64_t hi) {
+        return format_runs(part, nm, contig_len, runs, n, lo, hi);
+    });
+    return w->io_failed ? CLB_E_IO : CLB_OK;
+}
+
+extern "C" const char *clb_bedgraph_writer_buffer(clb_bedgraph_writer *w, uint64_t *len) {
+    if (!w) return nullptr;
+    if (len) *len = w->mem.size();
+    return w->mem.data();
+}
+
+extern "C" int clb_bedgraph_writer_close(clb_bedgraph_writer *w) {
+    if (!w) return CLB_E_INVALID;
+    const int rc = w->close();
     delete w;
     return rc;
 }

@@ -111,11 +111,18 @@ struct KParams {
     // Tile t covers contig positions [t * tile_len, min((t + 1) * tile_len, contig length)); tile_len >= 256.
     unsigned long long *tiles;
     uint32_t tile_len, n_tiles;
+    // depth runs (RUNS instantiations): (position, raw depth) of every run start, reserved per window from run_cursor;
+    // run_win_tab[w] = (first record, count | window soft << 16, raw depth of the first own entry, of the last one).  At most
+    // one record per position: run_cap = region length.
+    uint2 *run_rec;
+    uint32_t *run_cursor;
+    uint4 *run_win_tab;
+    uint32_t run_cap;
 };
 
-// The optional counts of the pileup kernels (template argument FEAT); the instantiations with a feature are only launched
+// The optional outputs of the pileup kernels (template argument FEAT); the instantiations with a feature are only launched
 // when it is on, so the ones without stay as they were.
-enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u };
+enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u, FEAT_RUNS = 4u };
 
 // Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
 // kernel with P and w in scope.  The stamps cost instruction-cache space, so production builds compile them out.
@@ -486,6 +493,18 @@ __device__ __forceinline__ uint32_t win_drop_first(const uint2 *win_tab, uint32_
     if (!((y >> 16) & 1u) || w == 0) return 0u;
     return ((y >> 12) & 15u) == ((win_tab[w - 1].y >> 20) & 15u) ? 1u : 0u;
 }
+__device__ __forceinline__ uint32_t win_count(uint2 t) { return win_count(t.y); }
+__device__ __forceinline__ IntervalOut gather_out(unsigned long long r) { return unpack_rec(r); }
+
+// The depth-run window table (KParams::run_win_tab) and records: the same compaction reads them.  A window-soft first run
+// (k_pileup_fast) is dropped when its raw depth equals the previous window's last.
+__device__ __forceinline__ uint32_t win_count(uint4 t) { return t.y & 0xffffu; }
+__device__ __forceinline__ uint32_t win_drop_first(const uint4 *win_tab, uint32_t w) {
+    const uint4 t = win_tab[w];
+    if (!((t.y >> 16) & 1u) || w == 0) return 0u;
+    return t.z == win_tab[w - 1].w ? 1u : 0u;
+}
+__device__ __forceinline__ uint2 gather_out(uint2 r) { return r; }
 
 // ---------------------------------------------------------------------------------------------
 // Phase C of both pileup kernels (k_pileup_fast, pileup_classify_window): classify the scanned depths, reduce the counters,
@@ -710,12 +729,43 @@ __device__ __forceinline__ void reduce_stats(const Entries<Sum> &e, uint32_t acc
     }
 }
 
+// Depth runs (RUNS instantiations; DESIGN.md §4).  Entry k starts a run iff its raw depth differs from entry k - 1's.  A
+// thread takes the previous thread's last raw depth by shuffle within the warp and, for lane 0, from the previous warp's
+// word in sRunLast.  raw(k): raw depth of entry k.
+static_assert(3 * NWARPS + 4 <= 4 * NWARPS && 3 * NWARPS + 4 <= 64, "sScan words 3 * NWARPS + 2 / + 3 (last raw depth, run base)");
+// Before reduce_stats' barrier: lane 31 parks the warp's last raw depth, the thread holding the window's last position that
+// position's raw depth.
+template <typename Sum, typename Raw>
+__device__ __forceinline__ void publish_run_depth(const Entries<Sum> &e, uint32_t n_ent, Raw raw, uint32_t *sRunLast, uint32_t *sScan) {
+    if ((threadIdx.x & 31) == 31) sRunLast[threadIdx.x >> 5] = raw(PPT - 1);
+    if (e.k_end > e.k_first && e.ebase + e.k_end == n_ent) {
+        uint32_t last = 0;
+#pragma unroll
+        for (int k = 0; k < PPT; k++) last = (uint32_t)k + 1u == e.k_end ? raw(k) : last;
+        sScan[3 * NWARPS + 2] = last;
+    }
+}
+// After that barrier: the thread's own entries that start a run, plus those in force.  Thread 0's entry 0 always starts one
+// (k_pileup_fast has no halo; the general kernel's entry 0 is the halo, outside vmask).
+template <typename Sum, typename Raw>
+__device__ __forceinline__ uint32_t run_starts(const Entries<Sum> &e, Raw raw, uint32_t force, const uint32_t *sRunLast) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t up = __shfl_up_sync(FULL, raw(PPT - 1), 1);
+    uint32_t prev = lane > 0 ? up : warp > 0 ? sRunLast[warp - 1] : 0xffffffffu;
+    uint32_t m = 0;
+#pragma unroll
+    for (int k = 0; k < PPT; k++) { const uint32_t d = raw(k); m |= (d != prev ? 1u : 0u) << k; prev = d; }
+    return (m | force) & e.vmask;
+}
+
 // Run boundaries -> records.  Entry k starts a run iff its state differs from entry k - 1's; thread 0's entry 0 always does.
 // The entries in force start a record regardless; those in soft (a subset of force) that merely continue a run are flagged
-// soft.  pos0: position of entry 0; win_soft: see pack_win_y.
-template <typename Sum>
+// soft.  pos0: position of entry 0; win_soft: see pack_win_y.  RUNS: the depth-run starts in rmask go to the run records in
+// the same scan (state count | run count << 16: both <= 2047 per window); raw(k) is entry k's raw depth.
+template <bool RUNS, typename Sum, typename Raw>
 __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t pos0, uint32_t force, uint32_t soft, uint32_t win_soft,
-                                              const uint8_t *sLast, uint32_t *sScan, uint32_t w, const KParams &P) {
+                                              const uint8_t *sLast, uint32_t *sScan, uint32_t w, const KParams &P, uint32_t rmask,
+                                              Raw raw) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     uint32_t bmask, softmask;
     {
@@ -729,19 +779,26 @@ __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t po
         softmask = soft & ~bmask;
         bmask = (bmask | force) & e.vmask;
     }
-    const uint32_t nb = __popc(bmask);
+    const uint32_t nb = RUNS ? __popc(bmask) | (__popc(rmask) << 16) : __popc(bmask);
     uint32_t inb = nb;
 #pragma unroll
     for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inb, dd); if (lane >= dd) inb += t; }
     if (lane == 31) sScan[2 * NWARPS + warp] = inb;
     __syncthreads();
     const uint32_t wt = lane < NWARPS ? sScan[2 * NWARPS + lane] : 0u;             // lane j: boundaries in warp j
-    const uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
+    uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
+    const uint32_t roff = off >> 16, rtotal = total >> 16;
+    if (RUNS) { off &= 0xffffu; total &= 0xffffu; }
     if (tid == 0) {
         const uint32_t base = atomicAdd(P.rec_cursor, total);                 // total may be 0 (general kernel): base is not read then
         sScan[3 * NWARPS] = base;
         P.win_tab[w] = make_uint2(base, pack_win_y(total, e.state(0), win_soft, sScan[3 * NWARPS + 1]));
         if ((unsigned long long)base + total > P.rec_cap) atomicOr(P.err, ERR_REC_OVERFLOW);
+        if (RUNS) {
+            const uint32_t rbase = atomicAdd(P.run_cursor, rtotal);
+            sScan[3 * NWARPS + 3] = rbase;
+            P.run_win_tab[w] = make_uint4(rbase, rtotal | (win_soft << 16), raw(0), sScan[3 * NWARPS + 2]);
+        }
     }
     __syncthreads();
     uint32_t o = sScan[3 * NWARPS] + off;
@@ -750,6 +807,16 @@ __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t po
         const int k = __ffs(m) - 1; m &= m - 1;
         if (o < P.rec_cap) P.rec[o] = pack_rec(pos0 + e.ebase + k, e.state(k), (softmask >> k) & 1u);
         o++;
+    }
+    if (RUNS) {
+        uint32_t ro = sScan[3 * NWARPS + 3] + roff;
+#pragma unroll
+        for (int k = 0; k < PPT; k++) {                                   // unrolled: raw(k) stays in registers
+            if ((rmask >> k) & 1u) {
+                if (ro < P.run_cap) P.run_rec[ro] = make_uint2(pos0 + e.ebase + k, raw(k));
+                ro++;
+            }
+        }
     }
 }
 
@@ -799,7 +866,7 @@ __device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, u
 // tables).
 template <bool BQ_HI, bool WIDE, bool DBG, unsigned FEAT>
 __device__ __forceinline__ void pileup_classify_window(const KParams &P, const uint32_t w) {
-    constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0;
+    constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0, RUNS = (FEAT & FEAT_RUNS) != 0;
     extern __shared__ __align__(16) uint8_t smem_raw[];
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw);
     uint32_t *sB = sA + WN;
@@ -1012,10 +1079,11 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
 
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4, "the depth table fits the segment pool");
-    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES, "the tile slots fit the segment pool");
+    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4, "the tile slots and run words fit the segment pool");
     uint32_t *sHist = reinterpret_cast<uint32_t *>(sPool);
     unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(sHist + 2 * DH_TAB);
     uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
+    uint32_t *sRunLast = sTileFirst + NWARPS;                              // per warp: its last raw depth (RUNS)
     if constexpr (HIST) zero_depth_table(sHist);                           // the scan barrier below orders it before the counts
     const uint32_t ebase = tid * PPT;
     uint32_t a[PPT], b[PPT], lqv[PPT], lw[WIDE ? PPT : 1];
@@ -1120,6 +1188,8 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
         e.covered -= raw0 > 0 ? 1u : 0u; e.sraw -= raw0; e.sqc -= b[0];
     }
     close_entries(e, n_ent, sLast, sScan);
+    const auto raw_of = [&](int k) { return WIDE ? a[k] : a[k] & 0xffffu; };   // not the packed word: its high half is the low-MAPQ depth
+    if constexpr (RUNS) publish_run_depth(e, n_ent, raw_of, sRunLast, sScan);
     dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
                   [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
     if constexpr (TILES)
@@ -1129,9 +1199,10 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     if constexpr (TILES) flush_tiles(sTileSum, sTileFirst, P);
     CLB_STAMP(4);
     // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
-    // previous shard's run
+    // previous shard's run; it always starts a depth run too (the halo is compared with for every other window)
     const uint32_t region_first = w == 0 && tid == 0 ? 2u : 0u;
-    write_records(e, (uint32_t)W.wb, region_first, P.region_start != 0 ? region_first : 0u, 0u, sLast, sScan, w, P);
+    const uint32_t rmask = RUNS ? run_starts(e, raw_of, region_first, sRunLast) : 0u;
+    write_records<RUNS>(e, (uint32_t)W.wb, region_first, P.region_start != 0 ? region_first : 0u, 0u, sLast, sScan, w, P, rmask, raw_of);
     CLB_STAMP(5);
     add_bins(e, (uint32_t)W.wb, 1u, n_ent, sCtl[10], sCtl[11], P);        // first bin, next bin's entry: divided out once by thread 0
     CLB_STAMP(6);
@@ -1383,14 +1454,16 @@ __global__ void k_first_table(uint32_t *first_tab, uint8_t *first_tab8, double f
 // ---------------------------------------------------------------------------------------------
 // Interval compaction: per-window record chunks (arbitrary order) -> sorted clb_interval array
 // ---------------------------------------------------------------------------------------------
+// The same three steps compact the depth runs (Tab = uint4: KParams::run_win_tab, records uint2, copied as they are).
 // step 1: every block scans 1024 windows locally and publishes its total
-__global__ void __launch_bounds__(1024) k_scan_windows_local(const uint2 *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot,
+template <typename Tab>
+__global__ void __launch_bounds__(1024) k_scan_windows_local(const Tab *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot,
                                                              const uint32_t *err) {
     __shared__ uint32_t sW[32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (*err & ERR_RESULT_INVALID) return;                    // win_tab was not written: nothing to scan
     const uint32_t i = blockIdx.x * 1024u + tid;
-    const uint32_t v = i < n_w ? win_count(win_tab[i].y) - win_drop_first(win_tab, i) : 0u;
+    const uint32_t v = i < n_w ? win_count(win_tab[i]) - win_drop_first(win_tab, i) : 0u;
     uint32_t inc = v;
 #pragma unroll
     for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inc, dd); if (lane >= dd) inc += t; }
@@ -1430,16 +1503,18 @@ __global__ void __launch_bounds__(1024) k_scan_blocks(uint32_t *blk_tot, uint32_
 // (nothing to gather when the record buffer overflowed: the records past its capacity were never written and the
 // interval array is just as small; the host grows both and re-runs the contig.  Nothing either when the input was refused:
 // win_tab and the scan hold whatever an earlier contig, or no contig, left there)
-__global__ void k_gather_intervals(const unsigned long long *rec, const uint2 *win_tab, const uint32_t *win_out, const uint32_t *blk_off,
-                                   uint32_t n_w, IntervalOut *out, const uint32_t *err) {
+// (the depth runs of a contig whose state records overflowed are not gathered either: the host re-runs it)
+template <typename Tab, typename Rec, typename Out>
+__global__ void k_gather_intervals(const Rec *rec, const Tab *win_tab, const uint32_t *win_out, const uint32_t *blk_off,
+                                   uint32_t n_w, Out *out, const uint32_t *err) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (w >= n_w || (*err & (ERR_REC_OVERFLOW | ERR_RESULT_INVALID))) return;
-    const uint2 t = win_tab[w];
+    const Tab t = win_tab[w];
     const uint32_t skip = win_drop_first(win_tab, w);
-    const uint32_t o = blk_off[w >> 10] + win_out[w], cnt = win_count(t.y) - skip;
+    const uint32_t o = blk_off[w >> 10] + win_out[w], cnt = win_count(t) - skip;
     for (uint32_t i = lane; i < cnt; i += 32) {
-        out[o + i] = unpack_rec(rec[t.x + skip + i]);
+        out[o + i] = gather_out(rec[t.x + skip + i]);
     }
 }
 

@@ -308,6 +308,7 @@ struct Options {
     bool verbose = false, progress = false; std::string timing_json;
     std::string depth_hist; uint32_t depth_hist_max = 1000;      // --depth-histogram FILE: rows for depths 0 .. depth_hist_max (last: >=)
     std::string depth_tiles; uint32_t depth_tile_size = 1000;    // --depth-tiles FILE: one row per tile of depth_tile_size positions
+    std::string depth_bedgraph;                                  // --depth-bedgraph FILE: runs of equal raw depth of every position
 };
 
 void usage() {
@@ -315,7 +316,8 @@ void usage() {
                     "       [--min-depth 4] [--max-depth 500] [--min-mapping-quality 10] [--min-base-quality 20]\n"
                     "       [--min-depth-for-low-mapq 10] [--max-low-mapq 1] [--max-low-mapq-fraction 0.1] [--threads N] [--device D]\n"
                     "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n"
-                    "       [--depth-histogram FILE] [--depth-histogram-max 1000] [--depth-tiles FILE] [--depth-tile-size 1000]\n");
+                    "       [--depth-histogram FILE] [--depth-histogram-max 1000] [--depth-tiles FILE] [--depth-tile-size 1000]\n"
+                    "       [--depth-bedgraph FILE]\n");
     exit(2);
 }
 
@@ -349,6 +351,7 @@ Options parse_options(int argc, char **argv) {
             opt.depth_hist_max = (uint32_t)d;
         }
         else if (a == "--depth-tiles") opt.depth_tiles = val();
+        else if (a == "--depth-bedgraph") opt.depth_bedgraph = val();
         else if (a == "--depth-tile-size") {
             const unsigned long long l = std::stoull(val());
             if (l < 256 || l > (1ull << 31)) usage();
@@ -423,7 +426,7 @@ struct Timing {
 //                 decoding of the next batch) / clb_finish_contig, BED text, plots
 Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, const std::map<std::string, FaiEntry> &fai,
                        std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed, DepthHistTsv *hist,
-                       DepthTilesTsv *tiles) {
+                       DepthTilesTsv *tiles, clb_bedgraph_writer *bedgraph) {
     auto check = [&](int rc, const char *what) { if (rc != 0) die(std::string("Error processing contig: ") + what + ": " + clb_last_error(ctx)); };
     // coverage plots land next to the BED file (callable_profiler.rs:24-27,80-83)
     const size_t slash = opt.out_bed.find_last_of('/');
@@ -493,6 +496,13 @@ Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, 
             const int rc = clb_bed_writer_add_contig(bed, st.name.c_str(), clen, res.intervals, res.n_intervals, bins.data(), res.n_bins, res.stride, &has_bins);
             if (rc == CLB_E_IO) die("Error processing contig: cannot write " + opt.out_bed);
             if (rc != 0) die("Error processing contig: interval list does not tile the contig");
+            if (bedgraph) {
+                const clb_depth_run *runs = nullptr; uint64_t n = 0;
+                check(clb_depth_runs(ctx, &runs, &n), "depth runs");
+                const int rg = clb_bedgraph_writer_add_contig(bedgraph, st.name.c_str(), clen, runs, n);
+                if (rg == CLB_E_IO) die("cannot write " + opt.depth_bedgraph);
+                if (rg != 0) die("Error processing contig: depth runs do not tile the contig");
+            }
             if (has_bins && res.stride) {                                        // finish_contig, callable_profiler.rs:64-86
                 const std::string path = out_dir + st.name + "_coverage.svg";
                 if (!write_file(path, report::render_coverage_svg(st.name, clen, res.stride, bins.data(), res.n_bins)))
@@ -624,8 +634,16 @@ int run(int argc, char **argv) {
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     if (!opt.depth_tiles.empty() && clb_set_depth_tiles(ctx.get(), opt.depth_tile_size) != 0)
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
+    if (!opt.depth_bedgraph.empty() && clb_set_depth_runs(ctx.get(), 1) != 0)
+        die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
     if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
+    // opened before the first contig (a FIFO blocks here until its reader is there), written per contig after its BED lines
+    std::unique_ptr<clb_bedgraph_writer, decltype(&clb_bedgraph_writer_close)> bedgraph(nullptr, clb_bedgraph_writer_close);
+    if (!opt.depth_bedgraph.empty()) {
+        bedgraph.reset(clb_bedgraph_writer_open(opt.depth_bedgraph.c_str()));
+        if (!bedgraph) die("cannot write " + opt.depth_bedgraph);
+    }
 
     // BamStats: its own pass over the first 10 000 records of the file, primary alignments only (bam_stats.rs:44-76)
     report::BamStats bs;
@@ -644,9 +662,10 @@ int run(int argc, char **argv) {
         DepthHistTsv hist;
         DepthTilesTsv tiles;
         const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get(),
-                                         opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles);
+                                         opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles, bedgraph.get());
         report_timing(opt, t, stats.size(), bam.inflate_seconds());
         if (clb_bed_writer_close(bed.release()) != 0) die("failed to write " + opt.out_bed);
+        if (bedgraph && clb_bedgraph_writer_close(bedgraph.release()) != 0) die("cannot write " + opt.depth_bedgraph);
         if (!opt.depth_hist.empty() && !write_file(opt.depth_hist, hist.finish())) die("cannot write " + opt.depth_hist);
         if (!opt.depth_tiles.empty() && !write_file(opt.depth_tiles, tiles.text)) die("cannot write " + opt.depth_tiles);
         ctx.reset();

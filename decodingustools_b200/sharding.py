@@ -15,7 +15,7 @@ from typing import List, Sequence, Tuple
 
 import numpy as np
 
-from .callable_loci import INTERVAL_DTYPE, ContigDeviceResult, stitch_intervals
+from .callable_loci import INTERVAL_DTYPE, RUN_DTYPE, ContigDeviceResult, stitch_depth_runs, stitch_intervals
 from .soa import ReadColumns
 
 
@@ -113,13 +113,24 @@ def allreduce_counters(res: ContigDeviceResult, group=None) -> ContigDeviceResul
     return unpack_counters(t.cpu().numpy(), res)
 
 
-def gather_and_stitch(local_intervals: np.ndarray, region_start: int, dst: int = 0, group=None):
-    """Collect the per-rank interval lists of one contig on `dst` and stitch them in genomic order."""
+def _gather_sorted(local: np.ndarray, dtype: np.dtype, region_start: int, dst: int, group):
+    """The per-rank arrays of one contig on `dst`, in genomic order (None elsewhere)."""
     import torch.distributed as dist
-    payload = (int(region_start), np.ascontiguousarray(local_intervals, dtype=INTERVAL_DTYPE).tobytes())
+    payload = (int(region_start), np.ascontiguousarray(local, dtype=dtype).tobytes())
     gathered = [None] * dist.get_world_size(group) if dist.get_rank(group) == dst else None
     dist.gather_object(payload, gathered, dst=dst, group=group)
     if gathered is None:
         return None
-    parts = sorted((p for p in gathered if len(p[1])), key=lambda p: p[0])
-    return stitch_intervals([np.frombuffer(b, dtype=INTERVAL_DTYPE) for _, b in parts])
+    return [np.frombuffer(b, dtype=dtype) for _, b in sorted((p for p in gathered if len(p[1])), key=lambda p: p[0])]
+
+
+def gather_and_stitch(local_intervals: np.ndarray, region_start: int, dst: int = 0, group=None):
+    """Collect the per-rank interval lists of one contig on `dst` and stitch them in genomic order."""
+    parts = _gather_sorted(local_intervals, INTERVAL_DTYPE, region_start, dst, group)
+    return None if parts is None else stitch_intervals(parts)
+
+
+def gather_and_stitch_depth_runs(local_runs: np.ndarray, region_start: int, dst: int = 0, group=None):
+    """Same for the depth runs (ContigDeviceResult.depth_runs): they are not additive, so they are gathered, not summed."""
+    parts = _gather_sorted(local_runs, RUN_DTYPE, region_start, dst, group)
+    return None if parts is None else stitch_depth_runs(parts)

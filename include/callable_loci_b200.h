@@ -194,6 +194,23 @@ int clb_set_depth_tiles(clb_ctx *ctx, uint32_t tile_len);
 int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64_t **callable, const uint64_t **raw_sum,
                     const uint64_t **qc_sum, uint32_t *n_tiles, uint32_t *tile_len);
 
+/* Depth runs (not in the reference; off by default; like bedtools genomecov -bga or mosdepth's per-base output): the raw
+ * depth of every position of [region_start, region_end) as runs of equal depth.  Raw depth is the depth of
+ * summed_coverage: admitted reads whose reference span covers the position, deletions and ref-skips included, no MAPQ or
+ * base-quality filter; REF_N positions and depth 0 are included.  Run i covers [start_i, start_{i+1}), the last one ends at
+ * region_end; starts ascend strictly from region_start and adjacent runs differ in depth.
+ * Region shards of one contig stitch by concatenation in genomic order, dropping a shard's first run when its depth equals
+ * the previous shard's last (runs are defined by depth alone: no soft flag is needed). */
+typedef struct clb_depth_run {
+    uint32_t start;
+    uint32_t depth;
+} clb_depth_run;
+/* on != 0: compute the runs from the next clb_begin_contig on; CLB_E_INVALID while a contig is open. */
+int clb_set_depth_runs(clb_ctx *ctx, int on);
+/* The runs of the last clb_finish_contig / clb_rerun_resident with a result, owned by the context like the intervals.
+ * When off: *runs = NULL, *n_runs = 0.  d2h_bytes counts their copy. */
+int clb_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_runs);
+
 /* Debug/parity: copy the per-base counters of [region_start, region_end) (computed by a separate
  * un-fused launch of the same pileup code).  Each pointer may be NULL. */
 int clb_debug_per_base(clb_ctx *ctx, uint32_t *raw, uint32_t *qc, uint32_t *low, uint8_t *state);
@@ -237,6 +254,14 @@ int  clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, uint32_t con
                                uint32_t *bins_inout, uint32_t n_bins, uint32_t stride, int *has_bins);
 const char *clb_bed_writer_buffer(clb_bed_writer *w, uint64_t *len);   /* in-memory mode */
 int  clb_bed_writer_close(clb_bed_writer *w);
+/* bedGraph writer for depth runs: lines "name\tstart\tend\tdepth\n", no header.  Runs must tile [0, contig_len) (stitched
+ * shards; none for an empty contig), else CLB_E_INVALID; a failed write gives CLB_E_IO.  A non-seekable path (a FIFO,
+ * /dev/stdout) is written in order. */
+typedef struct clb_bedgraph_writer clb_bedgraph_writer;
+clb_bedgraph_writer *clb_bedgraph_writer_open(const char *path /* NULL = in-memory */);
+int  clb_bedgraph_writer_add_contig(clb_bedgraph_writer *w, const char *name, uint32_t contig_len, const clb_depth_run *runs, uint64_t n);
+const char *clb_bedgraph_writer_buffer(clb_bedgraph_writer *w, uint64_t *len);   /* in-memory mode */
+int  clb_bedgraph_writer_close(clb_bedgraph_writer *w);
 /* Concatenate region shards of one contig in genomic order, merging soft starts.  Returns the number
  * of intervals written to out (capacity must be >= sum of inputs). */
 uint64_t clb_stitch_intervals(const clb_interval *const *shards, const uint64_t *n_per_shard, uint32_t n_shards,
