@@ -73,6 +73,12 @@ class ContigDeviceResult:
     tile_callable: Optional[np.ndarray] = None
     tile_raw_sum: Optional[np.ndarray] = None
     tile_qc_sum: Optional[np.ndarray] = None
+    # depth thresholds per tile (set_depth_thresholds, with the tiles): the thresholds, uint32[K], and per threshold j and
+    # tile t the tile's positions that are not REF_N with raw / QC depth >= tile_thresholds[j], uint64[K, n_tiles] each;
+    # None when off.
+    tile_thresholds: Optional[np.ndarray] = None
+    tile_raw_ge: Optional[np.ndarray] = None
+    tile_qc_ge: Optional[np.ndarray] = None
     # depth runs (set_depth_runs): RUN_DTYPE[n], None when off.  The raw depth of every position of the region as runs of
     # equal depth (depth_run_ends gives their ends); region shards join with stitch_depth_runs.
     depth_runs: Optional[np.ndarray] = None
@@ -166,6 +172,15 @@ class CallableLociContext:
         the default) from the next begin_contig on."""
         self._check(self._L.clb_set_depth_tiles(self._h, int(tile_len)))
 
+    def set_depth_thresholds(self, thresholds: Sequence[int]):
+        """Per depth tile, the positions with raw / QC depth >= each of 1..8 strictly ascending thresholds (1..2^32-1; an
+        empty sequence: off, the default) from the next begin_contig on.  Needs depth tiles on (set_depth_tiles)."""
+        vals = [int(t) for t in thresholds]
+        if any(t < 0 or t > 0xffffffff for t in vals):
+            raise ClbError(-1, f"depth thresholds {vals}: each 1..2^32-1")
+        arr = (C.c_uint32 * max(len(vals), 1))(*vals)
+        self._check(self._L.clb_set_depth_thresholds(self._h, arr, len(vals)))
+
     def set_depth_runs(self, on: bool):
         """Runs of equal raw depth over every position of the region (off by default) from the next begin_contig on."""
         self._check(self._L.clb_set_depth_runs(self._h, 1 if on else 0))
@@ -182,6 +197,13 @@ class CallableLociContext:
             r.tile_len = int(tl.value)
             r.tile_territory, r.tile_callable, r.tile_raw_sum, r.tile_qc_sum = (
                 np.ctypeslib.as_array(a, shape=(nt.value,)).copy() for a in arrs)
+        rg = C.POINTER(C.c_uint64)(); qg = C.POINTER(C.c_uint64)(); th = C.POINTER(C.c_uint32)(); k = C.c_uint32(0)
+        self._check(self._L.clb_depth_tile_thresholds(self._h, C.byref(rg), C.byref(qg), C.byref(th), C.byref(k), C.byref(nt)))
+        if k.value:
+            shape = (k.value, nt.value)
+            r.tile_thresholds = np.ctypeslib.as_array(th, shape=(k.value,)).copy()
+            r.tile_raw_ge = np.ctypeslib.as_array(rg, shape=shape).copy()
+            r.tile_qc_ge = np.ctypeslib.as_array(qg, shape=shape).copy()
         rp = C.c_void_p(0); nr = C.c_uint64(0)
         self._check(self._L.clb_depth_runs(self._h, C.byref(rp), C.byref(nr)))
         if rp.value:

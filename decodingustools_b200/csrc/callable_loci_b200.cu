@@ -57,6 +57,9 @@ struct clb_ctx {
     uint32_t tl_fetched = 0;            // tiles in the result of the last fetch (clb_depth_tiles)
     bool runs_next = false, runs = false;   // depth runs: set by clb_set_depth_runs, in force for the current contig
     bool runs_fetched = false;              // ... and in the result of the last fetch (clb_depth_runs)
+    uint32_t th_next[TH_MAX] = {}, th_k_next = 0;   // depth thresholds: set by clb_set_depth_thresholds,
+    uint32_t th[TH_MAX] = {}, th_k = 0;             // ... in force for the current contig (counted per depth tile)
+    uint32_t th_fetched = 0;                        // ... and in the result of the last fetch (clb_depth_tile_thresholds)
     bool long_mode = false, span_on_device = false;
     uint64_t n_reads = 0, n_cigar = 0, n_qual = 0;
     long long last_pos = -1;
@@ -131,9 +134,9 @@ int ensure(clb_ctx *ctx, DevBuf &b, size_t bytes, bool keep, cudaStream_t s) {
 void release(DevBuf &b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
 
 // u64 words of the counter buffer: [N_STATS stats][3 x n_bins bins][n raw][n qc][territory T][callable T][raw_sum T][qc_sum T]
-// (histograms and tiles only when on)
+// [raw_ge K x T][qc_ge K x T] (histograms, tiles and thresholds only when on)
 size_t tiles_offset(const clb_ctx *c) { return (size_t)N_STATS + 3 * (size_t)c->n_bins + 2 * (size_t)c->dh_n; }
-size_t n_counters(const clb_ctx *c) { return tiles_offset(c) + 4 * (size_t)c->n_tiles; }
+size_t n_counters(const clb_ctx *c) { return tiles_offset(c) + (4 + 2 * (size_t)c->th_k) * (size_t)c->n_tiles; }
 
 int get_events(clb_ctx *ctx, EvPair &ep) {
     if (!ctx->ev_pool.empty()) { ep = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); return CLB_OK; }
@@ -171,6 +174,8 @@ KParams make_params(clb_ctx *c) {
     P.timing = (long long *)c->timing.p;
     P.dhist = c->dh_n ? (unsigned long long *)c->dhist.p : nullptr; P.dh_n = c->dh_n;
     P.tiles = c->tl_len ? (unsigned long long *)c->counters.p + tiles_offset(c) : nullptr; P.tile_len = c->tl_len; P.n_tiles = c->n_tiles;
+    for (int j = 0; j < TH_MAX; j++) P.thr[j] = j < (int)c->th_k ? c->th[j] : 0xffffffffu;
+    P.n_thr = c->th_k;
     if (c->runs) {
         P.run_rec = (uint2 *)c->run_rec.p; P.run_cursor = (uint32_t *)c->misc.p + M_RUN_CURSOR; P.run_win_tab = (uint4 *)c->run_win_tab.p;
         P.run_cap = c->region_end - c->region_start;
@@ -184,8 +189,10 @@ KParams make_params(clb_ctx *c) {
 
 // The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
 // with the per-base dump (parity tests), FEAT the optional outputs that are on (FEAT_HIST: depth histograms, FEAT_TILES:
-// depth tiles, FEAT_RUNS: depth runs; only launched when on, so the others stay as they were).  f is called with two
-// std::integral_constant<bool, ...> and one std::integral_constant<unsigned, FEAT>.
+// depth tiles, FEAT_RUNS: depth runs, FEAT_THRESH: depth thresholds, only with FEAT_TILES; only launched when on, so the
+// others stay as they were).  f is called with two std::integral_constant<bool, ...> and one
+// std::integral_constant<unsigned, FEAT>; a feature set that has no instantiation (FEAT_THRESH without FEAT_TILES) calls
+// nothing.
 template <unsigned X> using FeatC = std::integral_constant<unsigned, X>;
 template <typename F>
 void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
@@ -199,13 +206,20 @@ void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
         case 4: f(b, d, FeatC<4u>{}); break;
         case 5: f(b, d, FeatC<5u>{}); break;
         case 6: f(b, d, FeatC<6u>{}); break;
-        default: f(b, d, FeatC<7u>{}); break;
+        case 7: f(b, d, FeatC<7u>{}); break;
+        case 10: f(b, d, FeatC<10u>{}); break;
+        case 11: f(b, d, FeatC<11u>{}); break;
+        case 14: f(b, d, FeatC<14u>{}); break;
+        case 15: f(b, d, FeatC<15u>{}); break;
+        default: break;
         }
     };
     if (bq_hi) { if (dbg) h(T{}, T{}); else h(T{}, N{}); }
     else { if (dbg) h(N{}, T{}); else h(N{}, N{}); }
 }
-unsigned features(const clb_ctx *c) { return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u) | (c->runs ? FEAT_RUNS : 0u); }
+unsigned features(const clb_ctx *c) {
+    return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u) | (c->runs ? FEAT_RUNS : 0u) | (c->th_k ? FEAT_THRESH : 0u);
+}
 
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
 // queue of windows the other two handed over) for windows [w0, w1) on the compute stream
@@ -317,7 +331,7 @@ int alloc_outputs(clb_ctx *ctx) {
 int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     const size_t n_cnt = n_counters(ctx);
     const size_t n_misc = ctx->runs ? M_WORDS_RUNS : M_WORDS;
-    ctx->dh_fetched = 0; ctx->tl_fetched = 0; ctx->runs_fetched = false;
+    ctx->dh_fetched = 0; ctx->tl_fetched = 0; ctx->runs_fetched = false; ctx->th_fetched = 0;
     ctx->h_counters.resize(n_cnt);
     CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, n_misc * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaMemcpyAsync(ctx->h_counters.data(), ctx->counters.p, n_cnt * 8, cudaMemcpyDeviceToHost, ctx->s_compute));
@@ -358,6 +372,7 @@ int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     for (size_t i = 0; i < ctx->h_bins.size(); i++) ctx->h_bins[i] = (uint32_t)ctx->h_counters[N_STATS + i];
     ctx->dh_fetched = ctx->dh_n;                                             // the histograms stay in h_counters, after the bins
     ctx->tl_fetched = ctx->n_tiles;                                          // ... and the tiles after them
+    ctx->th_fetched = ctx->th_k;                                             // ... and the threshold counts after the tiles
     ctx->runs_fetched = ctx->runs;
 
     float kms = 0, hms = 0, ums = 0;
@@ -451,7 +466,7 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-    for (int v = 0; v < 32; v++)                             // every instantiation of the pileup kernels
+    for (int v = 0; v < 64; v++)                             // every instantiation of the pileup kernels
         with_variant(v & 1, v & 2, (unsigned)v >> 2, [&](auto h, auto d, auto x) {
             constexpr bool H = decltype(h)::value, D = decltype(d)::value; constexpr unsigned X = decltype(x)::value;
             const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
@@ -514,6 +529,8 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
                      int ref_kind, uint32_t largest_contig_len, uint32_t region_start, uint32_t region_end, uint32_t max_ref_span) {
     if (!ctx) return CLB_E_INVALID;
     if (region_end > contig_len || region_start > region_end) return fail(ctx, CLB_E_INVALID, "bad region [%u,%u) for contig length %u", region_start, region_end, contig_len);
+    if (ctx->th_k_next && !ctx->tl_next)
+        return fail(ctx, CLB_E_INVALID, "depth thresholds (clb_set_depth_thresholds) are counted per depth tile: they need depth tiles on (clb_set_depth_tiles)");
     CU(cudaSetDevice(ctx->device));
     int rc;
     ctx->tid = tid; ctx->name = name ? name : ""; ctx->contig_len = contig_len; ctx->largest = largest_contig_len;
@@ -527,6 +544,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     ctx->dh_n = ctx->dh_next; ctx->dh_fetched = 0;
     ctx->tl_len = ctx->tl_next; ctx->tl_fetched = 0;
     ctx->runs = ctx->runs_next; ctx->runs_fetched = false; ctx->n_runs = 0;
+    std::copy(ctx->th_next, ctx->th_next + TH_MAX, ctx->th); ctx->th_k = ctx->th_k_next; ctx->th_fetched = 0;
     ctx->n_tiles = ctx->tl_len ? (uint32_t)(((uint64_t)contig_len + ctx->tl_len - 1) / ctx->tl_len) : 0u;
     clb_bin_geometry(ctx->name.c_str(), contig_len, largest_contig_len, &ctx->stride, &ctx->n_bins);
 
@@ -790,6 +808,34 @@ int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64
     if (qc_sum) *qc_sum = n ? t + 3 * (size_t)n : nullptr;
     if (n_tiles) *n_tiles = n;
     if (tile_len) *tile_len = n ? ctx->tl_len : 0u;
+    return CLB_OK;
+}
+
+int clb_set_depth_thresholds(clb_ctx *ctx, const uint32_t *thresholds, uint32_t k) {
+    if (!ctx) return CLB_E_INVALID;
+    if (ctx->in_contig && !ctx->finished) return fail(ctx, CLB_E_INVALID, "clb_set_depth_thresholds while a contig is open");
+    if (k > (uint32_t)TH_MAX) return fail(ctx, CLB_E_INVALID, "%u depth thresholds: at most %d", k, TH_MAX);
+    if (k && !thresholds) return fail(ctx, CLB_E_INVALID, "depth thresholds are NULL");
+    for (uint32_t j = 0; j < k; j++) {
+        if (thresholds[j] == 0) return fail(ctx, CLB_E_INVALID, "depth threshold 0: thresholds are 1..2^32-1");
+        if (j && thresholds[j] <= thresholds[j - 1]) return fail(ctx, CLB_E_INVALID, "depth thresholds must be strictly ascending");
+    }
+    std::fill(ctx->th_next, ctx->th_next + TH_MAX, 0u);
+    std::copy(thresholds, thresholds + k, ctx->th_next);
+    ctx->th_k_next = k;
+    return CLB_OK;
+}
+
+int clb_depth_tile_thresholds(const clb_ctx *ctx, const uint64_t **raw_ge, const uint64_t **qc_ge, const uint32_t **thresholds,
+                              uint32_t *k, uint32_t *n_tiles) {
+    if (!ctx) return CLB_E_INVALID;
+    const uint32_t kk = ctx->tl_fetched ? ctx->th_fetched : 0u, n = kk ? ctx->tl_fetched : 0u;
+    const uint64_t *g = kk ? (const uint64_t *)ctx->h_counters.data() + tiles_offset(ctx) + 4 * (size_t)n : nullptr;
+    if (raw_ge) *raw_ge = g;
+    if (qc_ge) *qc_ge = kk ? g + (size_t)kk * n : nullptr;
+    if (thresholds) *thresholds = kk ? ctx->th : nullptr;
+    if (k) *k = kk;
+    if (n_tiles) *n_tiles = n;
     return CLB_OK;
 }
 

@@ -52,9 +52,12 @@ constexpr int F_OFF_WSTATS = F_OFF_LAST + NT;
 constexpr int F_OFF_HIST = F_OFF_WSTATS + NWARPS * N_STATS * 8;    // depth table (HIST instantiations), 2 x DH_TAB u32
 constexpr int F_OFF_TILE = F_OFF_HIST + 2 * DH_TAB * 4;              // tile slots (TILES instantiations), TL_SLOT_BYTES
 constexpr int F_OFF_RUN = F_OFF_TILE + TL_SLOT_BYTES;                 // per warp its last raw depth (RUNS instantiations), u32
+constexpr int F_OFF_THSLOT = F_OFF_RUN + NWARPS * 4;                  // threshold slots (THRESH instantiations), TH_SLOT_BYTES
+constexpr int F_OFF_THTAB = F_OFF_THSLOT + TH_SLOT_BYTES;             // ... and their nibble table, TH_TAB u32
 static_assert(F_OFF_STAGE % 16 == 0 && F_WSTAGE % 16 == 0, "bulk copies need 16-byte aligned destinations");
 static_assert(F_OFF_WSTATS % 8 == 0 && F_OFF_BAR % 8 == 0 && F_OFF_X % 8 == 0 && F_OFF_MASK % 16 == 0 && F_OFF_FIRST % 16 == 0, "alignment");
-static_assert(F_OFF_RUN + NWARPS * 4 <= F_OFF_X, "phase C scratch fits the stages");
+static_assert(F_OFF_THSLOT % 16 == 0, "alignment");
+static_assert(F_OFF_THTAB + TH_TAB * 4 <= F_OFF_X, "phase C scratch fits the stages");
 static_assert(CLB_F_MINB * (F_SMEM + 1024) <= 228 * 1024, "shared memory per SM");
 enum { FC_BAIL = 0, FC_XCNT = 1 };
 
@@ -178,6 +181,8 @@ __device__ __forceinline__ void fmeta_load(const KParams &P, FMeta &M, uint32_t 
 template <bool BQ_HI, bool DBG, unsigned FEAT = 0u>
 __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P) {
     constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0, RUNS = (FEAT & FEAT_RUNS) != 0;
+    constexpr bool THRESH = (FEAT & FEAT_THRESH) != 0;
+    static_assert(!THRESH || TILES, "depth thresholds are counted per depth tile");
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint32_t w = P.win_first + blockIdx.x;
     // one table record per window, three independent 16-byte loads (no dependent round trip)
@@ -343,10 +348,12 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert(PPT == 8, "phase C of the fast kernel is written for 8 entries per thread");
     // The stages are dead since the barrier after the main loop (each warp's last sub-batch has streamed) and nothing has
-    // gone to global memory (a window that bailed returned above): zero the depth table here, the scan barrier below orders
-    // it before the first count.
+    // gone to global memory (a window that bailed returned above): zero the depth table and fill the threshold table here,
+    // the scan barrier below orders them before the first count.
     uint32_t *sHist = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_HIST);
     if constexpr (HIST) zero_depth_table(sHist);
+    uint32_t *sThTab = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_THTAB);
+    if constexpr (THRESH) fill_thresh_table(sThTab, P);
     uint32_t a[PPT], qcv[PPT];
     {
         const uint4 a0 = *reinterpret_cast<const uint4 *>(sA + ebase), a1 = *reinterpret_cast<const uint4 *>(sA + ebase + 4);
@@ -398,10 +405,13 @@ __global__ void __launch_bounds__(NT, CLB_F_MINB) k_pileup_fast(const KParams P)
     dbg_dump<DBG>(e, w * (uint32_t)WREAL, [&](int k) { return make_uint3(a[k] & 0xffffu, qcv[k], a[k] >> 16); }, P);
     unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(smem_raw + F_OFF_TILE);
     uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
-    if constexpr (TILES) count_tiles(e, wb0, nbits, [&](int k) { return make_uint2(a[k] & 0xffffu, qcv[k]); }, sTileSum, sTileFirst, P);
+    uint32_t *sThSlot = reinterpret_cast<uint32_t *>(smem_raw + F_OFF_THSLOT);
+    if constexpr (TILES)                                                  // qc <= raw <= 254: the threshold table holds every depth
+        count_tiles<THRESH, true>(e, wb0, nbits, [&](int k) { return make_uint2(a[k] & 0xffffu, qcv[k]); }, sTileSum, sTileFirst, P, sThTab,
+                                  sThSlot);
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
     if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
-    if constexpr (TILES) flush_tiles(sTileSum, sTileFirst, P);
+    if constexpr (TILES) flush_tiles<THRESH>(sTileSum, sTileFirst, P, sThSlot);
     // the window's first position always starts a record and a depth run (window soft: the gather drops them when the
     // previous window ended in the same state / at the same raw depth)
     const uint32_t rmask = RUNS ? run_starts(e, raw_of, 0u, sRunLast) : 0u;

@@ -59,6 +59,8 @@ constexpr uint32_t ERR_INPUT_REFUSED = ERR_UNSORTED | ERR_OFFSETS;
 // not be run; the host reports the error instead
 constexpr uint32_t ERR_RESULT_INVALID = ERR_INPUT_REFUSED | ERR_QUAL_SPAN;
 
+constexpr int TH_MAX = 8;             // depth thresholds per tile grid (KParams::thr)
+
 struct KParams {
     // packed read columns (device)
     const int32_t  *pos;
@@ -118,11 +120,16 @@ struct KParams {
     uint32_t *run_cursor;
     uint4 *run_win_tab;
     uint32_t run_cap;
+    // depth thresholds (THRESH instantiations, always with TILES): thr[0 .. n_thr) strictly ascending, thr[n_thr ..] unused;
+    // per tile the own positions that are not REF_N with raw / QC depth >= thr[j], at tiles + (4 + j) * n_tiles (raw) and
+    // tiles + (4 + n_thr + j) * n_tiles (QC)
+    uint32_t thr[TH_MAX];
+    uint32_t n_thr;
 };
 
 // The optional outputs of the pileup kernels (template argument FEAT); the instantiations with a feature are only launched
-// when it is on, so the ones without stay as they were.
-enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u, FEAT_RUNS = 4u };
+// when it is on, so the ones without stay as they were.  FEAT_THRESH is only instantiated together with FEAT_TILES.
+enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u, FEAT_RUNS = 4u, FEAT_THRESH = 8u };
 
 // Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
 // kernel with P and w in scope.  The stamps cost instruction-cache space, so production builds compile them out.
@@ -648,11 +655,38 @@ __device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
 // them with one global atomic per non-zero (tile, counter).  The slots sit beside the depth table (both may be on).
 constexpr int TL_MAX = 9;                                   // tiles one window can touch: 2047 positions, tiles of >= 256
 constexpr int TL_SLOT_BYTES = NWARPS * (8 * 8 + 4);         // per warp [2 tiles][4 counters] u64, then per warp its first tile (u32)
+// Depth thresholds (THRESH instantiations, always with TILES; DESIGN.md §4): per tile and threshold j, the tile's own
+// positions that are not REF_N with raw (QC) depth >= thr[j].  A depth maps to a word of unary nibbles, nibble j = (depth >=
+// thr[j]); a thread adds its entries' words per tile and kind (at most 8 per nibble: no carry) and the warp sums them as
+// 16-bit pairs of nibbles j and j + 4 (at most 256 per half), four REDUX per tile and kind.  Nibbles j >= n_thr are never
+// flushed.  The words of depths below TH_TAB come from a shared table filled once per window.
+constexpr int TH_TAB = 256;                                 // table entries: every depth the fast kernel can see (raw <= 254)
+constexpr int TH_SLOT_BYTES = NWARPS * 2 * 2 * 16;          // per warp [2 tiles][raw, qc] uint4 of 16-bit pairs
+static_assert(4 * TL_MAX + 2 * TH_MAX * TL_MAX <= NT, "one flush thread per tile counter and per tile threshold count");
+__device__ __forceinline__ uint32_t thresh_nibbles(uint32_t d, const KParams &P) {
+    uint32_t v = 0u;
+#pragma unroll
+    for (int j = 0; j < TH_MAX; j++) v += d >= P.thr[j] ? 1u << (4 * j) : 0u;
+    return v;
+}
+// Before the barrier that precedes count_tiles; the table must be dead (no other phase uses it any more).
+__device__ __forceinline__ void fill_thresh_table(uint32_t *tab, const KParams &P) {
+    for (int i = threadIdx.x; i < TH_TAB; i += NT) tab[i] = thresh_nibbles((uint32_t)i, P);
+}
+// The warp's sums of a nibble word as 16-bit pairs: .x = (nibble 0, nibble 4), .y = (1, 5), .z = (2, 6), .w = (3, 7)
+__device__ __forceinline__ uint4 warp_sum_nibbles(uint32_t v) {
+    const uint32_t m = 0x000f000fu;
+    return make_uint4(warp_sum(v & m), warp_sum((v >> 4) & m), warp_sum((v >> 8) & m), warp_sum((v >> 12) & m));
+}
+
 // After close_entries and the general kernel's halo correction: cnt_pack, sraw and sqc cover the own entries only (entries
-// past the region end carry no depth).  pos0: position of entry 0; depth(k) = (raw, qc) of entry k.
-template <typename Sum, typename Depth>
+// past the region end carry no depth).  pos0: position of entry 0; depth(k) = (raw, qc) of entry k.  THRESH: also the
+// threshold counts, from sThTab (filled by fill_thresh_table) for depths below TH_TAB (TAB_ONLY: the caller's depths always
+// are), into sThSlot (TH_SLOT_BYTES, 16-byte aligned).
+template <bool THRESH = false, bool TAB_ONLY = false, typename Sum, typename Depth>
 __device__ __forceinline__ void count_tiles(const Entries<Sum> &e, uint32_t pos0, uint32_t nbits, Depth depth, unsigned long long *sTileSum,
-                                            uint32_t *sTileFirst, const KParams &P) {
+                                            uint32_t *sTileFirst, const KParams &P, const uint32_t *sThTab = nullptr,
+                                            uint32_t *sThSlot = nullptr) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t L = P.tile_len;
     const uint32_t p = pos0 + e.ebase + e.k_first;                        // the thread's first own entry (never the halo)
@@ -672,8 +706,33 @@ __device__ __forceinline__ void count_tiles(const Entries<Sum> &e, uint32_t pos0
             else { ter1 += o; cal1 += c; raw1 += r; qc1 += q; }
         }
     }
+    uint32_t gr0 = 0u, gq0 = 0u, gr1 = 0u, gq1 = 0u;                      // THRESH: raw / QC nibble words of tiles t and t + 1
+    if constexpr (THRESH) {
+        const uint32_t in0 = own & ((1u << split) - 1u);                  // own entries in tile t
+        const auto add = [&](auto tab_tag) {
+#pragma unroll
+            for (int k = 0; k < PPT; k++) {
+                const uint2 d = depth(k);
+                const uint32_t r = decltype(tab_tag)::value ? sThTab[d.x] : thresh_nibbles(d.x, P);
+                const uint32_t q = decltype(tab_tag)::value ? sThTab[d.y] : thresh_nibbles(d.y, P);
+                if ((in0 >> k) & 1u) { gr0 += r; gq0 += q; }
+                else if ((own >> k) & 1u) { gr1 += r; gq1 += q; }
+            }
+        };
+        if constexpr (TAB_ONLY) {
+            add(std::true_type{});
+        } else {
+            uint32_t deepest = 0u;                                        // an upper bound of the thread's depths
+#pragma unroll
+            for (int k = 0; k < PPT; k++) { const uint2 d = depth(k); deepest |= d.x | d.y; }
+            if (deepest < (uint32_t)TH_TAB) add(std::true_type{}); else add(std::false_type{});
+        }
+    }
     const uint32_t T = __shfl_sync(FULL, t, 0);                           // the warp's first tile
-    if (t != T) { ter1 = ter0; cal1 = cal0; raw1 = raw0; qc1 = qc0; ter0 = cal0 = 0u; raw0 = qc0 = 0; }   // then nothing reached t + 1
+    if (t != T) {                                                         // then nothing reached t + 1
+        ter1 = ter0; cal1 = cal0; raw1 = raw0; qc1 = qc0; ter0 = cal0 = 0u; raw0 = qc0 = 0;
+        if constexpr (THRESH) { gr1 = gr0; gq1 = gq0; gr0 = gq0 = 0u; }
+    }
     const uint32_t s0 = warp_sum(ter0), s1 = warp_sum(cal0);
     const Sum s2 = warp_sum(raw0), s3 = warp_sum(qc0);
     uint32_t u0 = 0u, u1 = 0u; Sum u2 = 0, u3 = 0;
@@ -683,11 +742,41 @@ __device__ __forceinline__ void count_tiles(const Entries<Sum> &e, uint32_t pos0
         ws[0] = s0; ws[1] = s1; ws[2] = s2; ws[3] = s3; ws[4] = u0; ws[5] = u1; ws[6] = u2; ws[7] = u3;
         sTileFirst[warp] = T;
     }
+    if constexpr (THRESH) {
+        const uint4 r0 = warp_sum_nibbles(gr0), q0 = warp_sum_nibbles(gq0);
+        uint4 r1 = make_uint4(0u, 0u, 0u, 0u), q1 = r1;
+        if (__any_sync(FULL, ter1 != 0u)) { r1 = warp_sum_nibbles(gr1); q1 = warp_sum_nibbles(gq1); }   // warp-uniform
+        if (lane == 0) {
+            uint4 *ts = reinterpret_cast<uint4 *>(sThSlot) + warp * 4;
+            ts[0] = r0; ts[1] = q0; ts[2] = r1; ts[3] = q1;
+        }
+    }}
+// Thread 4 * TL_MAX + (kind * TH_MAX + j) * TL_MAX + i adds threshold j's raw (kind 0) or QC (kind 1) count of the window's
+// tile i; flush_tiles calls it.
+__device__ __forceinline__ void flush_thresholds(const uint32_t *sThSlot, const uint32_t *sTileFirst, const KParams &P) {
+    const uint32_t i = threadIdx.x - 4u * TL_MAX;
+    const uint32_t kind = i / (TH_MAX * TL_MAX), j = i / TL_MAX % TH_MAX, ti = i % TL_MAX, t0 = sTileFirst[0];
+    if (kind >= 2u || j >= P.n_thr) return;
+    const uint32_t word = kind * 4u + (j & 3u), shift = 16u * (j >> 2);   // [tile][kind][pair word]; nibble j in half j >> 2
+    uint32_t s = 0u;
+#pragma unroll
+    for (int w = 0; w < NWARPS; w++) {
+        const uint32_t d = sTileFirst[w] - t0;
+        if (d == ti) s += (sThSlot[w * 16 + word] >> shift) & 0xffffu;
+        if (d + 1u == ti) s += (sThSlot[w * 16 + 8 + word] >> shift) & 0xffffu;
+    }
+    if (s && t0 + ti < P.n_tiles) atomicAdd(P.tiles + (size_t)(4u + kind * P.n_thr + j) * P.n_tiles + t0 + ti, (unsigned long long)s);
 }
-// After a barrier that follows every count_tiles: thread c * TL_MAX + j adds counter c of the window's tile j.
-__device__ __forceinline__ void flush_tiles(const unsigned long long *sTileSum, const uint32_t *sTileFirst, const KParams &P) {
+// After a barrier that follows every count_tiles: thread c * TL_MAX + j adds counter c of the window's tile j; THRESH: the
+// next 2 * TH_MAX * TL_MAX threads add the threshold counts.
+template <bool THRESH = false>
+__device__ __forceinline__ void flush_tiles(const unsigned long long *sTileSum, const uint32_t *sTileFirst, const KParams &P,
+                                            const uint32_t *sThSlot = nullptr) {
     const uint32_t i = threadIdx.x;
-    if (i >= 4u * TL_MAX) return;
+    if (i >= 4u * TL_MAX) {
+        if constexpr (THRESH) flush_thresholds(sThSlot, sTileFirst, P);
+        return;
+    }
     const uint32_t c = i / TL_MAX, j = i % TL_MAX, t0 = sTileFirst[0];
     unsigned long long s = 0;
 #pragma unroll
@@ -867,6 +956,8 @@ __device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, u
 template <bool BQ_HI, bool WIDE, bool DBG, unsigned FEAT>
 __device__ __forceinline__ void pileup_classify_window(const KParams &P, const uint32_t w) {
     constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0, RUNS = (FEAT & FEAT_RUNS) != 0;
+    constexpr bool THRESH = (FEAT & FEAT_THRESH) != 0;
+    static_assert(!THRESH || TILES, "depth thresholds are counted per depth tile");
     extern __shared__ __align__(16) uint8_t smem_raw[];
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw);
     uint32_t *sB = sA + WN;
@@ -1080,11 +1171,17 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     // ------------------------------------------------------------------ phase C: scan, classify, segment
     static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4, "the depth table fits the segment pool");
     static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4, "the tile slots and run words fit the segment pool");
+    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4 + TH_SLOT_BYTES + TH_TAB * 4,
+                  "the threshold slots and table fit the segment pool");
+    static_assert((2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4) % 16 == 0, "threshold slots are 16-byte aligned");
     uint32_t *sHist = reinterpret_cast<uint32_t *>(sPool);
     unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(sHist + 2 * DH_TAB);
     uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
     uint32_t *sRunLast = sTileFirst + NWARPS;                              // per warp: its last raw depth (RUNS)
+    uint32_t *sThSlot = sRunLast + NWARPS;                                 // THRESH: per-warp slots, then the nibble table
+    uint32_t *sThTab = sThSlot + TH_SLOT_BYTES / 4;
     if constexpr (HIST) zero_depth_table(sHist);                           // the scan barrier below orders it before the counts
+    if constexpr (THRESH) fill_thresh_table(sThTab, P);                    // ... and the table before count_tiles
     const uint32_t ebase = tid * PPT;
     uint32_t a[PPT], b[PPT], lqv[PPT], lw[WIDE ? PPT : 1];
     {
@@ -1193,10 +1290,11 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
                   [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
     if constexpr (TILES)
-        count_tiles(e, (uint32_t)W.wb, nbits, [&](int k) { return make_uint2(WIDE ? a[k] : a[k] & 0xffffu, b[k]); }, sTileSum, sTileFirst, P);
+        count_tiles<THRESH>(e, (uint32_t)W.wb, nbits, [&](int k) { return make_uint2(WIDE ? a[k] : a[k] & 0xffffu, b[k]); }, sTileSum,
+                            sTileFirst, P, sThTab, sThSlot);
     reduce_stats(e, acc_sum, acc_mapq, sWStats, P);
     if constexpr (HIST) flush_depth_table(dh, sHist);                      // after reduce_stats' barrier
-    if constexpr (TILES) flush_tiles(sTileSum, sTileFirst, P);
+    if constexpr (TILES) flush_tiles<THRESH>(sTileSum, sTileFirst, P, sThSlot);
     CLB_STAMP(4);
     // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
     // previous shard's run; it always starts a depth run too (the halo is compared with for every other window)

@@ -308,6 +308,7 @@ struct Options {
     bool verbose = false, progress = false; std::string timing_json;
     std::string depth_hist; uint32_t depth_hist_max = 1000;      // --depth-histogram FILE: rows for depths 0 .. depth_hist_max (last: >=)
     std::string depth_tiles; uint32_t depth_tile_size = 1000;    // --depth-tiles FILE: one row per tile of depth_tile_size positions
+    std::vector<uint32_t> depth_thresholds;                      // --depth-thresholds T1,T2,...: per tile, bases at depth >= each
     std::string depth_bedgraph;                                  // --depth-bedgraph FILE: runs of equal raw depth of every position
 };
 
@@ -317,8 +318,24 @@ void usage() {
                     "       [--min-depth-for-low-mapq 10] [--max-low-mapq 1] [--max-low-mapq-fraction 0.1] [--threads N] [--device D]\n"
                     "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n"
                     "       [--depth-histogram FILE] [--depth-histogram-max 1000] [--depth-tiles FILE] [--depth-tile-size 1000]\n"
-                    "       [--depth-bedgraph FILE]\n");
+                    "       [--depth-thresholds T1,T2,... (with --depth-tiles; 1..8 ascending values >= 1)] [--depth-bedgraph FILE]\n");
     exit(2);
+}
+
+// --depth-thresholds: 1..8 comma-separated decimal values, strictly ascending, each 1..2^32-1; anything else is refused
+std::vector<uint32_t> parse_thresholds(const std::string &s) {
+    std::vector<uint32_t> v;
+    size_t i = 0;
+    while (true) {
+        const size_t j = s.find(',', i);
+        const std::string f = s.substr(i, j == std::string::npos ? std::string::npos : j - i);
+        if (f.empty() || f.size() > 10 || f.find_first_not_of("0123456789") != std::string::npos) usage();
+        const unsigned long long t = std::stoull(f);
+        if (t < 1 || t > 0xffffffffull || (!v.empty() && t <= v.back()) || v.size() == 8) usage();
+        v.push_back((uint32_t)t);
+        if (j == std::string::npos) return v;
+        i = j + 1;
+    }
 }
 
 Options parse_options(int argc, char **argv) {
@@ -357,10 +374,12 @@ Options parse_options(int argc, char **argv) {
             if (l < 256 || l > (1ull << 31)) usage();
             opt.depth_tile_size = (uint32_t)l;
         }
+        else if (a == "--depth-thresholds") opt.depth_thresholds = parse_thresholds(val());
         else if (!a.empty() && a[0] != '-' && opt.bam.empty()) opt.bam = a;
         else usage();
     }
     if (opt.bam.empty() || opt.reference.empty()) usage();
+    if (!opt.depth_thresholds.empty() && opt.depth_tiles.empty()) usage();     // the thresholds are columns of the tiles file
     return opt;
 }
 
@@ -391,17 +410,27 @@ struct DepthHistTsv {
 
 // --depth-tiles: "#contig\tstart\tend\tterritory\tcallable\tmean_raw\tmean_qc", then one row per tile, contigs in tid order.
 // start / end: the tile's 0-based half-open range; mean_raw / mean_qc: depth sums over territory (0.00 when it is 0).
+// With --depth-thresholds the header adds raw_ge_<T> for each threshold, then qc_ge_<T> for each, and the rows their counts.
 struct DepthTilesTsv {
-    std::string text = "#contig\tstart\tend\tterritory\tcallable\tmean_raw\tmean_qc\n";
+    std::string text;
+    explicit DepthTilesTsv(const std::vector<uint32_t> &thresholds) : text("#contig\tstart\tend\tterritory\tcallable\tmean_raw\tmean_qc") {
+        for (const char *kind : {"raw", "qc"})
+            for (uint32_t t : thresholds) text += std::string("\t") + kind + "_ge_" + std::to_string(t);
+        text += "\n";
+    }
+    // raw_ge / qc_ge: [k][n] threshold counts (k = 0: none)
     void add_contig(const std::string &name, uint32_t contig_len, uint32_t tile_len, const uint64_t *territory, const uint64_t *callable,
-                    const uint64_t *raw_sum, const uint64_t *qc_sum, uint32_t n) {
+                    const uint64_t *raw_sum, const uint64_t *qc_sum, uint32_t n, const uint64_t *raw_ge, const uint64_t *qc_ge, uint32_t k) {
         char buf[160];
         for (uint32_t t = 0; t < n; t++) {
             const uint64_t start = (uint64_t)t * tile_len, end = std::min<uint64_t>(start + tile_len, contig_len), ter = territory[t];
-            snprintf(buf, sizeof buf, "\t%llu\t%llu\t%llu\t%llu\t%.2f\t%.2f\n", (unsigned long long)start, (unsigned long long)end,
+            snprintf(buf, sizeof buf, "\t%llu\t%llu\t%llu\t%llu\t%.2f\t%.2f", (unsigned long long)start, (unsigned long long)end,
                      (unsigned long long)ter, (unsigned long long)callable[t], ter ? (double)raw_sum[t] / (double)ter : 0.0,
                      ter ? (double)qc_sum[t] / (double)ter : 0.0);
             text += name; text += buf;
+            for (const uint64_t *ge : {raw_ge, qc_ge})
+                for (uint32_t j = 0; j < k; j++) { text += '\t'; text += std::to_string(ge[(size_t)j * n + t]); }
+            text += '\n';
         }
     }
 };
@@ -488,7 +517,9 @@ Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, 
             if (tiles) {
                 const uint64_t *ter = nullptr, *cal = nullptr, *raw = nullptr, *qc = nullptr; uint32_t n = 0, len = 0;
                 check(clb_depth_tiles(ctx, &ter, &cal, &raw, &qc, &n, &len), "depth tiles");
-                tiles->add_contig(st.name, clen, len, ter, cal, raw, qc, n);
+                const uint64_t *raw_ge = nullptr, *qc_ge = nullptr; uint32_t k = 0;
+                check(clb_depth_tile_thresholds(ctx, &raw_ge, &qc_ge, nullptr, &k, nullptr), "depth thresholds");
+                tiles->add_contig(st.name, clen, len, ter, cal, raw, qc, n, raw_ge, qc_ge, k);
             }
             const auto tb = std::chrono::steady_clock::now();
             std::vector<uint32_t> bins(res.bins, res.bins + 3 * (size_t)res.n_bins);
@@ -634,6 +665,9 @@ int run(int argc, char **argv) {
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     if (!opt.depth_tiles.empty() && clb_set_depth_tiles(ctx.get(), opt.depth_tile_size) != 0)
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
+    if (!opt.depth_thresholds.empty() &&
+        clb_set_depth_thresholds(ctx.get(), opt.depth_thresholds.data(), (uint32_t)opt.depth_thresholds.size()) != 0)
+        die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     if (!opt.depth_bedgraph.empty() && clb_set_depth_runs(ctx.get(), 1) != 0)
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
@@ -660,7 +694,7 @@ int run(int argc, char **argv) {
     progress(opt, "Started");
     try {
         DepthHistTsv hist;
-        DepthTilesTsv tiles;
+        DepthTilesTsv tiles(opt.depth_thresholds);
         const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get(),
                                          opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles, bedgraph.get());
         report_timing(opt, t, stats.size(), bam.inflate_seconds());

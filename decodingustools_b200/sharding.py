@@ -73,32 +73,41 @@ TILE_FIELDS = ("tile_territory", "tile_callable", "tile_raw_sum", "tile_qc_sum")
 
 def pack_counters(res: ContigDeviceResult) -> np.ndarray:
     """The additive part of a shard result as one int64 vector: 6 state counts, 5 sums, 3 * n_bins bins, then the raw and
-    QC depth histograms when they are on, then the tiles' territory, callable, raw_sum and qc_sum when they are on (the
-    order of the device's counter buffer)."""
+    QC depth histograms when they are on, then the tiles' territory, callable, raw_sum and qc_sum when they are on, then
+    the tiles' raw_ge and qc_ge threshold counts (threshold-major) when they are on (the order of the device's counter
+    buffer)."""
     head = np.array(list(res.state_counts) + [getattr(res, k) for k in COUNTER_FIELDS], dtype=np.uint64)
     parts = [head, res.bins.astype(np.uint64).ravel()]
     if res.depth_hist_raw is not None:
         parts += [np.asarray(res.depth_hist_raw, np.uint64), np.asarray(res.depth_hist_qc, np.uint64)]
     if res.tile_territory is not None:
         parts += [np.asarray(getattr(res, k), np.uint64) for k in TILE_FIELDS]
+    if res.tile_thresholds is not None:
+        parts += [np.asarray(res.tile_raw_ge, np.uint64).ravel(), np.asarray(res.tile_qc_ge, np.uint64).ravel()]
     return np.concatenate(parts).view(np.int64)
 
 
 def unpack_counters(vec: np.ndarray, res: ContigDeviceResult) -> ContigDeviceResult:
-    """Inverse of pack_counters; whether `res` has depth histograms and tiles (and their lengths) says how the tail splits."""
+    """Inverse of pack_counters; whether `res` has depth histograms, tiles and tile thresholds (and their lengths, the
+    thresholds' from res.tile_thresholds) says how the tail splits."""
     v = np.asarray(vec).view(np.uint64)
     res.state_counts = v[:6].copy()
     for i, k in enumerate(COUNTER_FIELDS):
         setattr(res, k, int(v[6 + i]))
     n = 0 if res.depth_hist_raw is None else len(res.depth_hist_raw)
     nt = 0 if res.tile_territory is None else len(res.tile_territory)
-    end = v.shape[0] - 2 * n - 4 * nt
+    k = 0 if res.tile_thresholds is None else len(res.tile_thresholds)
+    end = v.shape[0] - 2 * n - (4 + 2 * k) * nt
     res.bins = v[11:end].reshape(3, -1).astype(np.uint32)
     if n:
         res.depth_hist_raw = v[end:end + n].copy()
         res.depth_hist_qc = v[end + n:end + 2 * n].copy()
-    for i, k in enumerate(TILE_FIELDS if nt else ()):
-        setattr(res, k, v[end + 2 * n + i * nt:end + 2 * n + (i + 1) * nt].copy())
+    for i, f in enumerate(TILE_FIELDS if nt else ()):
+        setattr(res, f, v[end + 2 * n + i * nt:end + 2 * n + (i + 1) * nt].copy())
+    if k:
+        g = end + 2 * n + 4 * nt
+        res.tile_raw_ge = v[g:g + k * nt].reshape(k, nt).copy()
+        res.tile_qc_ge = v[g + k * nt:g + 2 * k * nt].reshape(k, nt).copy()
     return res
 
 

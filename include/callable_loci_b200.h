@@ -194,6 +194,22 @@ int clb_set_depth_tiles(clb_ctx *ctx, uint32_t tile_len);
 int clb_depth_tiles(const clb_ctx *ctx, const uint64_t **territory, const uint64_t **callable, const uint64_t **raw_sum,
                     const uint64_t **qc_sum, uint32_t *n_tiles, uint32_t *tile_len);
 
+/* Depth thresholds per tile (not in the reference; off by default; like mosdepth's --thresholds with --by): k = 0 turns them
+ * off, else 1 <= k <= 8 strictly ascending values, each 1..2^32-1.  Counted on the depth-tile grid, so they need depth tiles
+ * on: clb_begin_contig returns CLB_E_INVALID for thresholds without tiles.  For tile t and threshold j: raw_ge[j][t], the
+ * region's positions in the tile that are not REF_N with raw depth >= thresholds[j], and qc_ge[j][t], the same for QC depth
+ * (depths as in the depth histograms).  So raw_ge[j] <= territory, qc_ge[j] <= raw_ge[j], and both are non-increasing in j.
+ * Takes effect at the next clb_begin_contig; CLB_E_INVALID while a contig is open, for k > 8, a 0 value or a list that is not
+ * strictly ascending.  When on, the two arrays follow the tiles in the counter buffer, threshold-major
+ * ([12 counters][3 x n_bins bins][hist raw][hist qc][territory][callable][raw_sum][qc_sum][raw_ge k x T][qc_ge k x T], all
+ * counted by clb_counters_device), so region shards of one contig sum into the same counts. */
+int clb_set_depth_thresholds(clb_ctx *ctx, const uint32_t *thresholds, uint32_t k);
+/* The threshold counts of the last clb_finish_contig / clb_rerun_resident / clb_refresh_counters, [k][n_tiles] each, and the
+ * thresholds they were counted at, owned by the context like the other results.  When off: *k = 0, *n_tiles = 0 and NULL
+ * pointers. */
+int clb_depth_tile_thresholds(const clb_ctx *ctx, const uint64_t **raw_ge, const uint64_t **qc_ge, const uint32_t **thresholds,
+                              uint32_t *k, uint32_t *n_tiles);
+
 /* Depth runs (not in the reference; off by default; like bedtools genomecov -bga or mosdepth's per-base output): the raw
  * depth of every position of [region_start, region_end) as runs of equal depth.  Raw depth is the depth of
  * summed_coverage: admitted reads whose reference span covers the position, deletions and ref-skips included, no MAPQ or
