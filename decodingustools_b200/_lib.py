@@ -57,6 +57,7 @@ SYMBOLS = [
     "clb_rerun_resident",
     "clb_counters_device", "clb_refresh_counters", "clb_set_nccl_allreduce", "clb_allreduce_nccl", "clb_debug_per_base",
     "clb_set_depth_histogram", "clb_depth_histogram", "clb_set_depth_tiles", "clb_depth_tiles", "clb_set_depth_runs", "clb_depth_runs",
+    "clb_set_qc_depth_runs", "clb_qc_depth_runs",
     "clb_set_depth_thresholds", "clb_depth_tile_thresholds",
     "clb_admit_reads", "clb_admit_reads_mt", "clb_admitter_new", "clb_admitter_push", "clb_admitter_free", "clb_compact_reads", "clb_bed_writer_open", "clb_bed_writer_add_contig", "clb_bed_writer_buffer",
     "clb_bed_writer_close", "clb_stitch_intervals", "clb_bin_geometry",
@@ -104,6 +105,8 @@ def lib() -> C.CDLL:
     L.clb_depth_tile_thresholds.argtypes = [vp, C.POINTER(C.POINTER(u64)), C.POINTER(C.POINTER(u64)), C.POINTER(C.POINTER(u32)),
                                             C.POINTER(u32), C.POINTER(u32)]
     L.clb_depth_runs.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
+    L.clb_set_qc_depth_runs.argtypes = [vp, C.c_int]
+    L.clb_qc_depth_runs.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
     L.clb_admit_reads.argtypes = [i32, u32, u64, vp, vp, vp, vp, vp]
     L.clb_host_alloc.restype = vp
     L.clb_host_alloc.argtypes = [C.c_size_t]

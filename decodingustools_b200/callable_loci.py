@@ -25,7 +25,8 @@ from .soa import ReadColumns
 
 INTERVAL_DTYPE = np.dtype([("start", "<u4"), ("end", "<u4"), ("state", "u1"), ("soft_start", "u1"), ("_pad", "<u2")])
 assert INTERVAL_DTYPE.itemsize == C.sizeof(_lib.Interval) == 12
-# clb_depth_run: a run of equal raw depth starts at `start` and ends where the next one starts (the last: at the region end)
+# clb_depth_run: a run of equal raw or QC depth starts at `start` and ends where the next one starts (the last: at the region
+# end)
 RUN_DTYPE = np.dtype([("start", "<u4"), ("depth", "<u4")])
 
 
@@ -82,6 +83,9 @@ class ContigDeviceResult:
     # depth runs (set_depth_runs): RUN_DTYPE[n], None when off.  The raw depth of every position of the region as runs of
     # equal depth (depth_run_ends gives their ends); region shards join with stitch_depth_runs.
     depth_runs: Optional[np.ndarray] = None
+    # QC depth runs (set_qc_depth_runs): the same for the QC depth, the depth the states are called on (the depth behind
+    # quality_bases); RUN_DTYPE[n], None when off.
+    qc_depth_runs: Optional[np.ndarray] = None
 
 
 def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDeviceResult:
@@ -100,14 +104,14 @@ def _result(res: _lib.ContigResult, copy_intervals: bool = True) -> ContigDevice
 
 
 def depth_run_ends(runs: np.ndarray, region_end: int) -> np.ndarray:
-    """End of each depth run: the next run's start, region_end for the last."""
+    """End of each depth run (raw or QC): the next run's start, region_end for the last."""
     starts = np.asarray(runs["start"], dtype=np.int64)
     return np.append(starts[1:], np.int64(region_end)) if starts.size else np.zeros(0, np.int64)
 
 
 def stitch_depth_runs(shards: Sequence[np.ndarray]) -> np.ndarray:
-    """Concatenate the depth runs of region shards of one contig in genomic order, dropping a shard's first run when its
-    depth equals the previous shard's last (runs are defined by depth alone)."""
+    """Concatenate the depth runs (raw or QC) of region shards of one contig in genomic order, dropping a shard's first run
+    when its depth equals the previous shard's last (runs are defined by depth alone)."""
     parts: List[np.ndarray] = []
     last = None
     for s in shards:
@@ -185,6 +189,11 @@ class CallableLociContext:
         """Runs of equal raw depth over every position of the region (off by default) from the next begin_contig on."""
         self._check(self._L.clb_set_depth_runs(self._h, 1 if on else 0))
 
+    def set_qc_depth_runs(self, on: bool):
+        """Runs of equal QC depth over every position of the region (off by default) from the next begin_contig on;
+        independent of set_depth_runs."""
+        self._check(self._L.clb_set_qc_depth_runs(self._h, 1 if on else 0))
+
     def _with_optional_counts(self, r: ContigDeviceResult) -> ContigDeviceResult:
         raw = C.POINTER(C.c_uint64)(); qc = C.POINTER(C.c_uint64)(); n = C.c_uint32(0)
         self._check(self._L.clb_depth_histogram(self._h, C.byref(raw), C.byref(qc), C.byref(n)))
@@ -204,12 +213,13 @@ class CallableLociContext:
             r.tile_thresholds = np.ctypeslib.as_array(th, shape=(k.value,)).copy()
             r.tile_raw_ge = np.ctypeslib.as_array(rg, shape=shape).copy()
             r.tile_qc_ge = np.ctypeslib.as_array(qg, shape=shape).copy()
-        rp = C.c_void_p(0); nr = C.c_uint64(0)
-        self._check(self._L.clb_depth_runs(self._h, C.byref(rp), C.byref(nr)))
-        if rp.value:
-            n = int(nr.value)
-            r.depth_runs = (np.ctypeslib.as_array(C.cast(rp, C.POINTER(C.c_uint8)), shape=(n * 8,)).view(RUN_DTYPE).copy()
-                            if n else np.zeros(0, RUN_DTYPE))
+        for fn, field in ((self._L.clb_depth_runs, "depth_runs"), (self._L.clb_qc_depth_runs, "qc_depth_runs")):
+            rp = C.c_void_p(0); nr = C.c_uint64(0)
+            self._check(fn(self._h, C.byref(rp), C.byref(nr)))
+            if rp.value:
+                n = int(nr.value)
+                setattr(r, field, np.ctypeslib.as_array(C.cast(rp, C.POINTER(C.c_uint8)), shape=(n * 8,)).view(RUN_DTYPE).copy()
+                        if n else np.zeros(0, RUN_DTYPE))
         return r
 
     def set_stream(self, cuda_stream: int):
@@ -378,7 +388,8 @@ class ContigProfiler:
 
 
 class BedGraphWriter:
-    """Depth runs as bedGraph text (clb_bedgraph_writer): "name\tstart\tend\tdepth" lines, contigs in the order added."""
+    """Depth runs (raw or QC) as bedGraph text (clb_bedgraph_writer): "name\tstart\tend\tdepth" lines, contigs in the order
+    added."""
 
     def __init__(self, path: Optional[str]):
         self._L = _lib.lib()

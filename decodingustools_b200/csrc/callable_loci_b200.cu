@@ -57,6 +57,8 @@ struct clb_ctx {
     uint32_t tl_fetched = 0;            // tiles in the result of the last fetch (clb_depth_tiles)
     bool runs_next = false, runs = false;   // depth runs: set by clb_set_depth_runs, in force for the current contig
     bool runs_fetched = false;              // ... and in the result of the last fetch (clb_depth_runs)
+    bool qruns_next = false, qruns = false; // QC depth runs: set by clb_set_qc_depth_runs, in force for the current contig
+    bool qruns_fetched = false;             // ... and in the result of the last fetch (clb_qc_depth_runs)
     uint32_t th_next[TH_MAX] = {}, th_k_next = 0;   // depth thresholds: set by clb_set_depth_thresholds,
     uint32_t th[TH_MAX] = {}, th_k = 0;             // ... in force for the current contig (counted per depth tile)
     uint32_t th_fetched = 0;                        // ... and in the result of the last fetch (clb_depth_tile_thresholds)
@@ -69,6 +71,7 @@ struct clb_ctx {
     DevBuf stats_padded, counters, rec, win_tab, win_rec, win_out, deep_list, intervals, misc;
     DevBuf gen_list, blk_tot, dhist;
     DevBuf run_rec, run_win_tab, runs_out;   // depth runs: records, window table, compacted runs (region length each)
+    DevBuf qrun_rec, qrun_win_tab, qruns_out;   // QC depth runs: the same
     DevBuf dbg_raw, dbg_qc, dbg_low, dbg_state, timing;
     uint32_t rec_cap = 0;
     bool dbg = false;
@@ -85,13 +88,16 @@ struct clb_ctx {
     clb_depth_run *h_runs = nullptr;       // pinned
     size_t h_runs_cap = 0;
     uint64_t n_runs = 0;
+    clb_depth_run *h_qruns = nullptr;      // pinned
+    size_t h_qruns_cap = 0;
+    uint64_t n_qruns = 0;
 };
 
 // misc layout (uint32): record cursor, error bits, n_total intervals, deep-window count, general-queue count / tickets taken
 // (these six are reset per run), then the maximum reference span; with depth runs on, the run cursor and run count follow
-// (reset per run too, and only copied then)
+// (reset per run too, and only copied then); with QC depth runs on, the QC run cursor and QC run count after those
 enum { M_CURSOR = 0, M_ERR = 1, M_NTOTAL = 2, M_DEEP = 3, M_GEN_COUNT = 4, M_GEN_TAKEN = 5, M_RESET_WORDS = 6, M_MAXSPAN = 7, M_MAXQLEN = 8, M_WORDS = 9,
-       M_RUN_CURSOR = 9, M_RUN_NTOTAL = 10, M_WORDS_RUNS = 11 };
+       M_RUN_CURSOR = 9, M_RUN_NTOTAL = 10, M_WORDS_RUNS = 11, M_QRUN_CURSOR = 11, M_QRUN_NTOTAL = 12, M_WORDS_QRUNS = 13 };
 
 namespace {
 
@@ -180,6 +186,10 @@ KParams make_params(clb_ctx *c) {
         P.run_rec = (uint2 *)c->run_rec.p; P.run_cursor = (uint32_t *)c->misc.p + M_RUN_CURSOR; P.run_win_tab = (uint4 *)c->run_win_tab.p;
         P.run_cap = c->region_end - c->region_start;
     }
+    if (c->qruns) {
+        P.qrun_rec = (uint2 *)c->qrun_rec.p; P.qrun_cursor = (uint32_t *)c->misc.p + M_QRUN_CURSOR; P.qrun_win_tab = (uint4 *)c->qrun_win_tab.p;
+        P.qrun_cap = c->region_end - c->region_start;
+    }
     if (c->dbg) {
         P.dbg_raw = (uint32_t *)c->dbg_raw.p; P.dbg_qc = (uint32_t *)c->dbg_qc.p;
         P.dbg_low = (uint32_t *)c->dbg_low.p; P.dbg_state = (uint8_t *)c->dbg_state.p;
@@ -189,8 +199,8 @@ KParams make_params(clb_ctx *c) {
 
 // The pileup kernels' template arguments: BQ_HI = (min_base_quality >= 128) picks the byte compare, DBG the instantiation
 // with the per-base dump (parity tests), FEAT the optional outputs that are on (FEAT_HIST: depth histograms, FEAT_TILES:
-// depth tiles, FEAT_RUNS: depth runs, FEAT_THRESH: depth thresholds, only with FEAT_TILES; only launched when on, so the
-// others stay as they were).  f is called with two std::integral_constant<bool, ...> and one
+// depth tiles, FEAT_RUNS: depth runs, FEAT_THRESH: depth thresholds, only with FEAT_TILES, FEAT_QRUNS: QC depth runs; only
+// launched when on, so the others stay as they were).  f is called with two std::integral_constant<bool, ...> and one
 // std::integral_constant<unsigned, FEAT>; a feature set that has no instantiation (FEAT_THRESH without FEAT_TILES) calls
 // nothing.
 template <unsigned X> using FeatC = std::integral_constant<unsigned, X>;
@@ -211,6 +221,18 @@ void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
         case 11: f(b, d, FeatC<11u>{}); break;
         case 14: f(b, d, FeatC<14u>{}); break;
         case 15: f(b, d, FeatC<15u>{}); break;
+        case 16: f(b, d, FeatC<16u>{}); break;
+        case 17: f(b, d, FeatC<17u>{}); break;
+        case 18: f(b, d, FeatC<18u>{}); break;
+        case 19: f(b, d, FeatC<19u>{}); break;
+        case 20: f(b, d, FeatC<20u>{}); break;
+        case 21: f(b, d, FeatC<21u>{}); break;
+        case 22: f(b, d, FeatC<22u>{}); break;
+        case 23: f(b, d, FeatC<23u>{}); break;
+        case 26: f(b, d, FeatC<26u>{}); break;
+        case 27: f(b, d, FeatC<27u>{}); break;
+        case 30: f(b, d, FeatC<30u>{}); break;
+        case 31: f(b, d, FeatC<31u>{}); break;
         default: break;
         }
     };
@@ -218,7 +240,8 @@ void with_variant(bool bq_hi, bool dbg, unsigned feat, F &&f) {
     else { if (dbg) h(N{}, T{}); else h(N{}, N{}); }
 }
 unsigned features(const clb_ctx *c) {
-    return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u) | (c->runs ? FEAT_RUNS : 0u) | (c->th_k ? FEAT_THRESH : 0u);
+    return (c->dh_n ? FEAT_HIST : 0u) | (c->tl_len ? FEAT_TILES : 0u) | (c->runs ? FEAT_RUNS : 0u) | (c->th_k ? FEAT_THRESH : 0u) |
+           (c->qruns ? FEAT_QRUNS : 0u);
 }
 
 // window ranges + classes, the fast kernel (one CTA per window) and the general kernel (persistent CTAs over the
@@ -260,6 +283,7 @@ int reset_accumulators(clb_ctx *ctx) {
     if (ctx->dh_n) CU(cudaMemsetAsync(ctx->dhist.p, 0, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, ctx->s_compute));
     CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_CURSOR, 0, M_RESET_WORDS * sizeof(uint32_t), ctx->s_compute));   // cursor, err, n_total, deep windows, general queue
     if (ctx->runs) CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_RUN_CURSOR, 0, 2 * sizeof(uint32_t), ctx->s_compute));   // run cursor, run count
+    if (ctx->qruns) CU(cudaMemsetAsync((uint32_t *)ctx->misc.p + M_QRUN_CURSOR, 0, 2 * sizeof(uint32_t), ctx->s_compute)); // QC run cursor, count
     return CLB_OK;
 }
 
@@ -302,6 +326,16 @@ int launch_compaction(clb_ctx *ctx) {
             (const uint32_t *)ctx->blk_tot.p, ctx->n_windows, (uint2 *)ctx->runs_out.p, (const uint32_t *)ctx->misc.p + M_ERR);
         ctx->launches += 3;
     }
+    if (ctx->qruns) {
+        // the QC depth runs the same way (win_out / blk_tot are free again after the previous gather)
+        k_scan_windows_local<uint4><<<n_blk, 1024, 0, ctx->s_compute>>>((const uint4 *)ctx->qrun_win_tab.p, ctx->n_windows, (uint32_t *)ctx->win_out.p,
+                                                                       (uint32_t *)ctx->blk_tot.p, (const uint32_t *)ctx->misc.p + M_ERR);
+        k_scan_blocks<<<1, 1024, 0, ctx->s_compute>>>((uint32_t *)ctx->blk_tot.p, n_blk, (uint32_t *)ctx->misc.p + M_QRUN_NTOTAL);
+        k_gather_intervals<uint4, uint2, uint2><<<(ctx->n_windows + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, ctx->s_compute>>>(
+            (const uint2 *)ctx->qrun_rec.p, (const uint4 *)ctx->qrun_win_tab.p, (const uint32_t *)ctx->win_out.p,
+            (const uint32_t *)ctx->blk_tot.p, ctx->n_windows, (uint2 *)ctx->qruns_out.p, (const uint32_t *)ctx->misc.p + M_ERR);
+        ctx->launches += 3;
+    }
     CU(cudaGetLastError());
     return CLB_OK;
 }
@@ -324,14 +358,21 @@ int alloc_outputs(clb_ctx *ctx) {
         if ((rc = ensure(ctx, ctx->run_rec, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
         if ((rc = ensure(ctx, ctx->runs_out, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
     }
+    if (ctx->qruns) {
+        // the same bound for the QC depth runs
+        const size_t rlen = ctx->region_end - ctx->region_start;
+        if ((rc = ensure(ctx, ctx->qrun_win_tab, nw * sizeof(uint4), false, ctx->s_compute))) return rc;
+        if ((rc = ensure(ctx, ctx->qrun_rec, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
+        if ((rc = ensure(ctx, ctx->qruns_out, rlen * sizeof(uint2), false, ctx->s_compute))) return rc;
+    }
     return CLB_OK;
 }
 
 // copy counters + interval count, validate device error bits, then copy the intervals
 int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
     const size_t n_cnt = n_counters(ctx);
-    const size_t n_misc = ctx->runs ? M_WORDS_RUNS : M_WORDS;
-    ctx->dh_fetched = 0; ctx->tl_fetched = 0; ctx->runs_fetched = false; ctx->th_fetched = 0;
+    const size_t n_misc = ctx->qruns ? M_WORDS_QRUNS : ctx->runs ? M_WORDS_RUNS : M_WORDS;
+    ctx->dh_fetched = 0; ctx->tl_fetched = 0; ctx->runs_fetched = false; ctx->th_fetched = 0; ctx->qruns_fetched = false;
     ctx->h_counters.resize(n_cnt);
     CU(cudaMemcpyAsync(ctx->h_misc, ctx->misc.p, n_misc * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(cudaMemcpyAsync(ctx->h_counters.data(), ctx->counters.p, n_cnt * 8, cudaMemcpyDeviceToHost, ctx->s_compute));
@@ -367,13 +408,28 @@ int fetch_result(clb_ctx *ctx, clb_contig_result *out) {
         }
     }
     ctx->n_runs = n_runs;
-    ctx->d2h_bytes = n_misc * 4 + n_cnt * 8 + n_iv * sizeof(clb_interval) + n_runs * sizeof(clb_depth_run);
+    const uint64_t n_qruns = ctx->qruns && ctx->n_windows ? ctx->h_misc[M_QRUN_NTOTAL] : 0;
+    if (ctx->qruns) {
+        if (n_qruns > ctx->h_qruns_cap || !ctx->h_qruns) {
+            if (ctx->h_qruns) cudaFreeHost(ctx->h_qruns);
+            ctx->h_qruns = nullptr;
+            ctx->h_qruns_cap = std::max<size_t>(n_qruns + n_qruns / 4, 1024);
+            CU(cudaHostAlloc((void **)&ctx->h_qruns, ctx->h_qruns_cap * sizeof(clb_depth_run), cudaHostAllocDefault));
+        }
+        if (n_qruns) {
+            CU(cudaMemcpyAsync(ctx->h_qruns, ctx->qruns_out.p, n_qruns * sizeof(clb_depth_run), cudaMemcpyDeviceToHost, ctx->s_compute));
+            CU(cudaStreamSynchronize(ctx->s_compute));
+        }
+    }
+    ctx->n_qruns = n_qruns;
+    ctx->d2h_bytes = n_misc * 4 + n_cnt * 8 + n_iv * sizeof(clb_interval) + (n_runs + n_qruns) * sizeof(clb_depth_run);
     ctx->h_bins.resize(3 * (size_t)ctx->n_bins);
     for (size_t i = 0; i < ctx->h_bins.size(); i++) ctx->h_bins[i] = (uint32_t)ctx->h_counters[N_STATS + i];
     ctx->dh_fetched = ctx->dh_n;                                             // the histograms stay in h_counters, after the bins
     ctx->tl_fetched = ctx->n_tiles;                                          // ... and the tiles after them
     ctx->th_fetched = ctx->th_k;                                             // ... and the threshold counts after the tiles
     ctx->runs_fetched = ctx->runs;
+    ctx->qruns_fetched = ctx->qruns;
 
     float kms = 0, hms = 0, ums = 0;
     for (auto &ep : ctx->ev_upload) { float t = 0; cudaEventElapsedTime(&t, ep.a, ep.b); ums += t; ctx->ev_pool.push_back(ep); }
@@ -466,7 +522,7 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
         const char *fg = getenv("CLB_FORCE_GENERAL");
         ctx->force_general = fg && fg[0] && fg[0] != '0';
     }
-    for (int v = 0; v < 64; v++)                             // every instantiation of the pileup kernels
+    for (int v = 0; v < 128; v++)                            // every instantiation of the pileup kernels
         with_variant(v & 1, v & 2, (unsigned)v >> 2, [&](auto h, auto d, auto x) {
             constexpr bool H = decltype(h)::value, D = decltype(d)::value; constexpr unsigned X = decltype(x)::value;
             const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
@@ -480,7 +536,7 @@ clb_ctx *clb_create(int device, const clb_options *opt, char *err, size_t err_le
     if ((e = cudaMalloc((void **)&ctx->d_first_tab, 65536 * 4 + WIN_TABLE_BYTES + 256)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaMalloc", e); }
     k_first_table<<<65536 / 256, 256, 0, ctx->s_compute>>>(ctx->d_first_tab, (uint8_t *)(ctx->d_first_tab + 65536) + WIN_TABLE_BYTES, opt->max_low_mapq_fraction);
     k_window_tables<<<1, 256, 0, ctx->s_compute>>>(ctx->d_first_tab + 65536, opt->max_low_mapq_fraction);
-    if ((e = cudaHostAlloc((void **)&ctx->h_misc, M_WORDS_RUNS * 4, cudaHostAllocDefault)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaHostAlloc", e); }
+    if ((e = cudaHostAlloc((void **)&ctx->h_misc, M_WORDS_QRUNS * 4, cudaHostAllocDefault)) != cudaSuccess) { clb_destroy(ctx); return bail("cudaHostAlloc", e); }
     if ((e = cudaStreamSynchronize(ctx->s_compute)) != cudaSuccess) { clb_destroy(ctx); return bail("first-table kernel", e); }
     return ctx;
 }
@@ -491,11 +547,13 @@ void clb_destroy(clb_ctx *ctx) {
     cudaDeviceSynchronize();
     for (DevBuf *b : {&ctx->pos, &ctx->flag, &ctx->mapq, &ctx->cigar_off, &ctx->cigar, &ctx->qual_off, &ctx->qual, &ctx->read_end, &ctx->cigar_ckpt,
                       &ctx->nmask, &ctx->ref_ascii, &ctx->stats_padded, &ctx->counters, &ctx->rec, &ctx->win_tab, &ctx->win_rec,
-                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dhist, &ctx->run_rec, &ctx->run_win_tab, &ctx->runs_out, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
+                      &ctx->win_out, &ctx->deep_list, &ctx->intervals, &ctx->misc, &ctx->gen_list, &ctx->blk_tot, &ctx->dhist, &ctx->run_rec, &ctx->run_win_tab, &ctx->runs_out,
+                      &ctx->qrun_rec, &ctx->qrun_win_tab, &ctx->qruns_out, &ctx->dbg_raw, &ctx->dbg_qc, &ctx->dbg_low, &ctx->dbg_state, &ctx->timing})
         release(*b);
     if (ctx->d_first_tab) cudaFree(ctx->d_first_tab);
     if (ctx->h_intervals) cudaFreeHost(ctx->h_intervals);
     if (ctx->h_runs) cudaFreeHost(ctx->h_runs);
+    if (ctx->h_qruns) cudaFreeHost(ctx->h_qruns);
     if (ctx->h_misc) cudaFreeHost(ctx->h_misc);
     for (auto &ep : ctx->ev_pool) { cudaEventDestroy(ep.a); cudaEventDestroy(ep.b); }
     for (auto &ep : ctx->ev_kernel) { cudaEventDestroy(ep.a); cudaEventDestroy(ep.b); }
@@ -544,6 +602,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     ctx->dh_n = ctx->dh_next; ctx->dh_fetched = 0;
     ctx->tl_len = ctx->tl_next; ctx->tl_fetched = 0;
     ctx->runs = ctx->runs_next; ctx->runs_fetched = false; ctx->n_runs = 0;
+    ctx->qruns = ctx->qruns_next; ctx->qruns_fetched = false; ctx->n_qruns = 0;
     std::copy(ctx->th_next, ctx->th_next + TH_MAX, ctx->th); ctx->th_k = ctx->th_k_next; ctx->th_fetched = 0;
     ctx->n_tiles = ctx->tl_len ? (uint32_t)(((uint64_t)contig_len + ctx->tl_len - 1) / ctx->tl_len) : 0u;
     clb_bin_geometry(ctx->name.c_str(), contig_len, largest_contig_len, &ctx->stride, &ctx->n_bins);
@@ -580,7 +639,7 @@ int clb_begin_contig(clb_ctx *ctx, int32_t tid, const char *name, uint32_t conti
     CU(cudaEventRecord(ep.b, ctx->s_compute));
     ctx->ev_h2d.push_back(ep);
 
-    if ((rc = ensure(ctx, ctx->misc, M_WORDS_RUNS * 4, false, ctx->s_compute))) return rc;
+    if ((rc = ensure(ctx, ctx->misc, M_WORDS_QRUNS * 4, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->stats_padded, (size_t)N_STATS * STAT_STRIDE * 8, false, ctx->s_compute))) return rc;
     if ((rc = ensure(ctx, ctx->counters, n_counters(ctx) * 8, false, ctx->s_compute))) return rc;
     if (ctx->dh_n && (rc = ensure(ctx, ctx->dhist, (size_t)DH_SLOTS * 2 * ctx->dh_n * 8, false, ctx->s_compute))) return rc;
@@ -850,6 +909,20 @@ int clb_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_r
     if (!ctx) return CLB_E_INVALID;
     if (runs) *runs = ctx->runs_fetched ? ctx->h_runs : nullptr;
     if (n_runs) *n_runs = ctx->runs_fetched ? ctx->n_runs : 0;
+    return CLB_OK;
+}
+
+int clb_set_qc_depth_runs(clb_ctx *ctx, int on) {
+    if (!ctx) return CLB_E_INVALID;
+    if (ctx->in_contig && !ctx->finished) return fail(ctx, CLB_E_INVALID, "clb_set_qc_depth_runs while a contig is open");
+    ctx->qruns_next = on != 0;
+    return CLB_OK;
+}
+
+int clb_qc_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_runs) {
+    if (!ctx) return CLB_E_INVALID;
+    if (runs) *runs = ctx->qruns_fetched ? ctx->h_qruns : nullptr;
+    if (n_runs) *n_runs = ctx->qruns_fetched ? ctx->n_qruns : 0;
     return CLB_OK;
 }
 

@@ -125,11 +125,18 @@ struct KParams {
     // tiles + (4 + n_thr + j) * n_tiles (QC)
     uint32_t thr[TH_MAX];
     uint32_t n_thr;
+    // QC depth runs (QRUNS instantiations): the depth runs keyed on the QC depth (the depth behind quality_bases) instead of
+    // the raw depth.  (position, QC depth) records reserved per window from qrun_cursor; qrun_win_tab in run_win_tab's
+    // format, with QC depths.  At most one record per position: qrun_cap = region length.
+    uint2 *qrun_rec;
+    uint32_t *qrun_cursor;
+    uint4 *qrun_win_tab;
+    uint32_t qrun_cap;
 };
 
 // The optional outputs of the pileup kernels (template argument FEAT); the instantiations with a feature are only launched
 // when it is on, so the ones without stay as they were.  FEAT_THRESH is only instantiated together with FEAT_TILES.
-enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u, FEAT_RUNS = 4u, FEAT_THRESH = 8u };
+enum : unsigned { FEAT_HIST = 1u, FEAT_TILES = 2u, FEAT_RUNS = 4u, FEAT_THRESH = 8u, FEAT_QRUNS = 16u };
 
 // Developer builds only (scripts/phase_timing.py): slot i of window w's 8 timing words, written by thread 0 of a pileup
 // kernel with P and w in scope.  The stamps cost instruction-cache space, so production builds compile them out.
@@ -503,8 +510,8 @@ __device__ __forceinline__ uint32_t win_drop_first(const uint2 *win_tab, uint32_
 __device__ __forceinline__ uint32_t win_count(uint2 t) { return win_count(t.y); }
 __device__ __forceinline__ IntervalOut gather_out(unsigned long long r) { return unpack_rec(r); }
 
-// The depth-run window table (KParams::run_win_tab) and records: the same compaction reads them.  A window-soft first run
-// (k_pileup_fast) is dropped when its raw depth equals the previous window's last.
+// The depth-run window tables (KParams::run_win_tab, qrun_win_tab) and records: the same compaction reads them.  A
+// window-soft first run (k_pileup_fast) is dropped when its depth (raw or QC, the table's kind) equals the previous window's last.
 __device__ __forceinline__ uint32_t win_count(uint4 t) { return t.y & 0xffffu; }
 __device__ __forceinline__ uint32_t win_drop_first(const uint4 *win_tab, uint32_t w) {
     const uint4 t = win_tab[w];
@@ -820,18 +827,21 @@ __device__ __forceinline__ void reduce_stats(const Entries<Sum> &e, uint32_t acc
 
 // Depth runs (RUNS instantiations; DESIGN.md §4).  Entry k starts a run iff its raw depth differs from entry k - 1's.  A
 // thread takes the previous thread's last raw depth by shuffle within the warp and, for lane 0, from the previous warp's
-// word in sRunLast.  raw(k): raw depth of entry k.
-static_assert(3 * NWARPS + 4 <= 4 * NWARPS && 3 * NWARPS + 4 <= 64, "sScan words 3 * NWARPS + 2 / + 3 (last raw depth, run base)");
-// Before reduce_stats' barrier: lane 31 parks the warp's last raw depth, the thread holding the window's last position that
-// position's raw depth.
+// word in sRunLast.  raw(k): raw depth of entry k.  QC depth runs (QRUNS) are the same calls with the QC depth, their own
+// per-warp words and their own sScan words.
+// sScan words: 3 * NWARPS + 2 / + 3 (window's last raw depth, run base), + 4 / + 5 (the same for QC runs), 5 * NWARPS + warp
+// (per-warp QC run counts when both kinds are on)
+static_assert(3 * NWARPS + 6 <= 4 * NWARPS && 6 * NWARPS <= 64, "sScan words of the depth runs");
+// Before reduce_stats' barrier: lane 31 parks the warp's last depth, the thread holding the window's last position that
+// position's depth in *sWinLast.
 template <typename Sum, typename Raw>
-__device__ __forceinline__ void publish_run_depth(const Entries<Sum> &e, uint32_t n_ent, Raw raw, uint32_t *sRunLast, uint32_t *sScan) {
+__device__ __forceinline__ void publish_run_depth(const Entries<Sum> &e, uint32_t n_ent, Raw raw, uint32_t *sRunLast, uint32_t *sWinLast) {
     if ((threadIdx.x & 31) == 31) sRunLast[threadIdx.x >> 5] = raw(PPT - 1);
     if (e.k_end > e.k_first && e.ebase + e.k_end == n_ent) {
         uint32_t last = 0;
 #pragma unroll
         for (int k = 0; k < PPT; k++) last = (uint32_t)k + 1u == e.k_end ? raw(k) : last;
-        sScan[3 * NWARPS + 2] = last;
+        *sWinLast = last;
     }
 }
 // After that barrier: the thread's own entries that start a run, plus those in force.  Thread 0's entry 0 always starts one
@@ -847,14 +857,37 @@ __device__ __forceinline__ uint32_t run_starts(const Entries<Sum> &e, Raw raw, u
     return (m | force) & e.vmask;
 }
 
+// One depth-run stream of write_records (thread 0): reserve the window's cnt records from cursor and describe them in
+// win_tab[w] = (first record, count | window soft << 16, depth of the first own entry, of the last); the first record's
+// index goes to *sBase.
+__device__ __forceinline__ void reserve_runs(uint32_t *cursor, uint4 *win_tab, uint32_t w, uint32_t cnt, uint32_t win_soft, uint32_t first,
+                                             uint32_t last, uint32_t *sBase) {
+    const uint32_t rbase = atomicAdd(cursor, cnt);
+    *sBase = rbase;
+    win_tab[w] = make_uint4(rbase, cnt | (win_soft << 16), first, last);
+}
+// ... and every thread: the starts in mask, (position, depth(k)) each, from record o on.  p0: position of entry 0.
+template <typename Depth>
+__device__ __forceinline__ void write_runs(uint32_t mask, Depth depth, uint32_t o, uint32_t p0, uint2 *rec, uint32_t cap) {
+#pragma unroll
+    for (int k = 0; k < PPT; k++) {                                       // unrolled: depth(k) stays in registers
+        if ((mask >> k) & 1u) {
+            if (o < cap) rec[o] = make_uint2(p0 + k, depth(k));
+            o++;
+        }
+    }
+}
+
 // Run boundaries -> records.  Entry k starts a run iff its state differs from entry k - 1's; thread 0's entry 0 always does.
 // The entries in force start a record regardless; those in soft (a subset of force) that merely continue a run are flagged
-// soft.  pos0: position of entry 0; win_soft: see pack_win_y.  RUNS: the depth-run starts in rmask go to the run records in
-// the same scan (state count | run count << 16: both <= 2047 per window); raw(k) is entry k's raw depth.
-template <bool RUNS, typename Sum, typename Raw>
+// soft.  pos0: position of entry 0; win_soft: see pack_win_y.  RUNS / QRUNS: the depth-run starts in rmask / qmask go to the
+// raw / QC run records in the same scan; raw(k) / qc(k) is entry k's raw / QC depth.  With one run kind on, its count rides
+// in the scan word (state count | run count << 16: both <= 2047 per window); with both, the QC count has a second word.
+template <bool RUNS, bool QRUNS, typename Sum, typename Raw, typename Qc>
 __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t pos0, uint32_t force, uint32_t soft, uint32_t win_soft,
                                               const uint8_t *sLast, uint32_t *sScan, uint32_t w, const KParams &P, uint32_t rmask,
-                                              Raw raw) {
+                                              Raw raw, uint32_t qmask, Qc qc) {
+    constexpr bool ANY = RUNS || QRUNS, BOTH = RUNS && QRUNS;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     uint32_t bmask, softmask;
     {
@@ -868,26 +901,33 @@ __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t po
         softmask = soft & ~bmask;
         bmask = (bmask | force) & e.vmask;
     }
-    const uint32_t nb = RUNS ? __popc(bmask) | (__popc(rmask) << 16) : __popc(bmask);
-    uint32_t inb = nb;
+    const uint32_t nb = ANY ? __popc(bmask) | (__popc(RUNS ? rmask : qmask) << 16) : __popc(bmask);
+    const uint32_t nq = BOTH ? __popc(qmask) : 0u;
+    uint32_t inb = nb, inq = nq;
 #pragma unroll
-    for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t t = __shfl_up_sync(FULL, inb, dd); if (lane >= dd) inb += t; }
-    if (lane == 31) sScan[2 * NWARPS + warp] = inb;
+    for (int dd = 1; dd < 32; dd <<= 1) {
+        const uint32_t t = __shfl_up_sync(FULL, inb, dd);
+        if (BOTH) { const uint32_t tq = __shfl_up_sync(FULL, inq, dd); if (lane >= dd) inq += tq; }
+        if (lane >= dd) inb += t;
+    }
+    if (lane == 31) { sScan[2 * NWARPS + warp] = inb; if (BOTH) sScan[5 * NWARPS + warp] = inq; }
     __syncthreads();
     const uint32_t wt = lane < NWARPS ? sScan[2 * NWARPS + lane] : 0u;             // lane j: boundaries in warp j
     uint32_t off = inb - nb + __reduce_add_sync(FULL, lane < warp ? wt : 0u), total = __reduce_add_sync(FULL, wt);
-    const uint32_t roff = off >> 16, rtotal = total >> 16;
-    if (RUNS) { off &= 0xffffu; total &= 0xffffu; }
+    const uint32_t roff = off >> 16, rtotal = total >> 16;                // the run kind in the high half
+    if (ANY) { off &= 0xffffu; total &= 0xffffu; }
+    uint32_t qoff = roff, qtotal = rtotal;                                 // QC runs: the high half, or the second word
+    if (BOTH) {
+        const uint32_t wq = lane < NWARPS ? sScan[5 * NWARPS + lane] : 0u;
+        qoff = inq - nq + __reduce_add_sync(FULL, lane < warp ? wq : 0u); qtotal = __reduce_add_sync(FULL, wq);
+    }
     if (tid == 0) {
         const uint32_t base = atomicAdd(P.rec_cursor, total);                 // total may be 0 (general kernel): base is not read then
         sScan[3 * NWARPS] = base;
         P.win_tab[w] = make_uint2(base, pack_win_y(total, e.state(0), win_soft, sScan[3 * NWARPS + 1]));
         if ((unsigned long long)base + total > P.rec_cap) atomicOr(P.err, ERR_REC_OVERFLOW);
-        if (RUNS) {
-            const uint32_t rbase = atomicAdd(P.run_cursor, rtotal);
-            sScan[3 * NWARPS + 3] = rbase;
-            P.run_win_tab[w] = make_uint4(rbase, rtotal | (win_soft << 16), raw(0), sScan[3 * NWARPS + 2]);
-        }
+        if (RUNS) reserve_runs(P.run_cursor, P.run_win_tab, w, rtotal, win_soft, raw(0), sScan[3 * NWARPS + 2], sScan + 3 * NWARPS + 3);
+        if (QRUNS) reserve_runs(P.qrun_cursor, P.qrun_win_tab, w, qtotal, win_soft, qc(0), sScan[3 * NWARPS + 4], sScan + 3 * NWARPS + 5);
     }
     __syncthreads();
     uint32_t o = sScan[3 * NWARPS] + off;
@@ -897,16 +937,8 @@ __device__ __forceinline__ void write_records(const Entries<Sum> &e, uint32_t po
         if (o < P.rec_cap) P.rec[o] = pack_rec(pos0 + e.ebase + k, e.state(k), (softmask >> k) & 1u);
         o++;
     }
-    if (RUNS) {
-        uint32_t ro = sScan[3 * NWARPS + 3] + roff;
-#pragma unroll
-        for (int k = 0; k < PPT; k++) {                                   // unrolled: raw(k) stays in registers
-            if ((rmask >> k) & 1u) {
-                if (ro < P.run_cap) P.run_rec[ro] = make_uint2(pos0 + e.ebase + k, raw(k));
-                ro++;
-            }
-        }
-    }
+    if (RUNS) write_runs(rmask, raw, sScan[3 * NWARPS + 3] + roff, pos0 + e.ebase, P.run_rec, P.run_cap);
+    if (QRUNS) write_runs(qmask, qc, sScan[3 * NWARPS + 5] + qoff, pos0 + e.ebase, P.qrun_rec, P.qrun_cap);
 }
 
 // Bins: positions of CALLABLE / POOR_MAPPING_QUALITY / REF_N per stride-sized bin.  pos0: position of entry 0; e_first: the
@@ -956,7 +988,7 @@ __device__ __forceinline__ void add_bins(const Entries<Sum> &e, uint32_t pos0, u
 template <bool BQ_HI, bool WIDE, bool DBG, unsigned FEAT>
 __device__ __forceinline__ void pileup_classify_window(const KParams &P, const uint32_t w) {
     constexpr bool HIST = (FEAT & FEAT_HIST) != 0, TILES = (FEAT & FEAT_TILES) != 0, RUNS = (FEAT & FEAT_RUNS) != 0;
-    constexpr bool THRESH = (FEAT & FEAT_THRESH) != 0;
+    constexpr bool THRESH = (FEAT & FEAT_THRESH) != 0, QRUNS = (FEAT & FEAT_QRUNS) != 0;
     static_assert(!THRESH || TILES, "depth thresholds are counted per depth tile");
     extern __shared__ __align__(16) uint8_t smem_raw[];
     uint32_t *sA = reinterpret_cast<uint32_t *>(smem_raw);
@@ -1174,12 +1206,15 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4 + TH_SLOT_BYTES + TH_TAB * 4,
                   "the threshold slots and table fit the segment pool");
     static_assert((2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4) % 16 == 0, "threshold slots are 16-byte aligned");
+    static_assert((size_t)DCAP * 8 >= 2 * DH_TAB * 4 + TL_SLOT_BYTES + NWARPS * 4 + TH_SLOT_BYTES + TH_TAB * 4 + NWARPS * 4,
+                  "the QC run words fit the segment pool");
     uint32_t *sHist = reinterpret_cast<uint32_t *>(sPool);
     unsigned long long *sTileSum = reinterpret_cast<unsigned long long *>(sHist + 2 * DH_TAB);
     uint32_t *sTileFirst = reinterpret_cast<uint32_t *>(sTileSum + NWARPS * 8);
     uint32_t *sRunLast = sTileFirst + NWARPS;                              // per warp: its last raw depth (RUNS)
     uint32_t *sThSlot = sRunLast + NWARPS;                                 // THRESH: per-warp slots, then the nibble table
     uint32_t *sThTab = sThSlot + TH_SLOT_BYTES / 4;
+    uint32_t *sQRunLast = sThTab + TH_TAB;                                 // per warp: its last QC depth (QRUNS)
     if constexpr (HIST) zero_depth_table(sHist);                           // the scan barrier below orders it before the counts
     if constexpr (THRESH) fill_thresh_table(sThTab, P);                    // ... and the table before count_tiles
     const uint32_t ebase = tid * PPT;
@@ -1286,7 +1321,9 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     }
     close_entries(e, n_ent, sLast, sScan);
     const auto raw_of = [&](int k) { return WIDE ? a[k] : a[k] & 0xffffu; };   // not the packed word: its high half is the low-MAPQ depth
-    if constexpr (RUNS) publish_run_depth(e, n_ent, raw_of, sRunLast, sScan);
+    const auto qc_of = [&](int k) { return b[k]; };                        // the QC depth since the classify loop, halo included
+    if constexpr (RUNS) publish_run_depth(e, n_ent, raw_of, sRunLast, sScan + 3 * NWARPS + 2);
+    if constexpr (QRUNS) publish_run_depth(e, n_ent, qc_of, sQRunLast, sScan + 3 * NWARPS + 4);
     dbg_dump<DBG>(e, (uint32_t)(W.wb - P.region_start),
                   [&](int k) { return make_uint3(WIDE ? a[k] : a[k] & 0xffffu, b[k], WIDE ? lw[WIDE ? k : 0] : a[k] >> 16); }, P);
     if constexpr (TILES)
@@ -1297,10 +1334,12 @@ __device__ __forceinline__ void pileup_classify_window(const KParams &P, const u
     if constexpr (TILES) flush_tiles<THRESH>(sTileSum, sTileFirst, P, sThSlot);
     CLB_STAMP(4);
     // entry 1 of window 0 is the region's first position: it always starts a record, soft when it merely continues the
-    // previous shard's run; it always starts a depth run too (the halo is compared with for every other window)
+    // previous shard's run; it always starts a raw and a QC depth run too (the halo is compared with for every other window)
     const uint32_t region_first = w == 0 && tid == 0 ? 2u : 0u;
     const uint32_t rmask = RUNS ? run_starts(e, raw_of, region_first, sRunLast) : 0u;
-    write_records<RUNS>(e, (uint32_t)W.wb, region_first, P.region_start != 0 ? region_first : 0u, 0u, sLast, sScan, w, P, rmask, raw_of);
+    const uint32_t qmask = QRUNS ? run_starts(e, qc_of, region_first, sQRunLast) : 0u;
+    write_records<RUNS, QRUNS>(e, (uint32_t)W.wb, region_first, P.region_start != 0 ? region_first : 0u, 0u, sLast, sScan, w, P, rmask,
+                               raw_of, qmask, qc_of);
     CLB_STAMP(5);
     add_bins(e, (uint32_t)W.wb, 1u, n_ent, sCtl[10], sCtl[11], P);        // first bin, next bin's entry: divided out once by thread 0
     CLB_STAMP(6);
@@ -1552,7 +1591,8 @@ __global__ void k_first_table(uint32_t *first_tab, uint8_t *first_tab8, double f
 // ---------------------------------------------------------------------------------------------
 // Interval compaction: per-window record chunks (arbitrary order) -> sorted clb_interval array
 // ---------------------------------------------------------------------------------------------
-// The same three steps compact the depth runs (Tab = uint4: KParams::run_win_tab, records uint2, copied as they are).
+// The same three steps compact the depth runs, raw and QC (Tab = uint4: KParams::run_win_tab / qrun_win_tab, records uint2,
+// copied as they are).
 // step 1: every block scans 1024 windows locally and publishes its total
 template <typename Tab>
 __global__ void __launch_bounds__(1024) k_scan_windows_local(const Tab *win_tab, uint32_t n_w, uint32_t *win_out, uint32_t *blk_tot,

@@ -310,6 +310,7 @@ struct Options {
     std::string depth_tiles; uint32_t depth_tile_size = 1000;    // --depth-tiles FILE: one row per tile of depth_tile_size positions
     std::vector<uint32_t> depth_thresholds;                      // --depth-thresholds T1,T2,...: per tile, bases at depth >= each
     std::string depth_bedgraph;                                  // --depth-bedgraph FILE: runs of equal raw depth of every position
+    std::string qc_depth_bedgraph;                               // --qc-depth-bedgraph FILE: the same for the QC depth
 };
 
 void usage() {
@@ -318,7 +319,8 @@ void usage() {
                     "       [--min-depth-for-low-mapq 10] [--max-low-mapq 1] [--max-low-mapq-fraction 0.1] [--threads N] [--device D]\n"
                     "       [--report-templates DIR] [--verbose] [--progress] [--timing-json FILE]\n"
                     "       [--depth-histogram FILE] [--depth-histogram-max 1000] [--depth-tiles FILE] [--depth-tile-size 1000]\n"
-                    "       [--depth-thresholds T1,T2,... (with --depth-tiles; 1..8 ascending values >= 1)] [--depth-bedgraph FILE]\n");
+                    "       [--depth-thresholds T1,T2,... (with --depth-tiles; 1..8 ascending values >= 1)] [--depth-bedgraph FILE]\n"
+                    "       [--qc-depth-bedgraph FILE]\n");
     exit(2);
 }
 
@@ -369,6 +371,7 @@ Options parse_options(int argc, char **argv) {
         }
         else if (a == "--depth-tiles") opt.depth_tiles = val();
         else if (a == "--depth-bedgraph") opt.depth_bedgraph = val();
+        else if (a == "--qc-depth-bedgraph") opt.qc_depth_bedgraph = val();
         else if (a == "--depth-tile-size") {
             const unsigned long long l = std::stoull(val());
             if (l < 256 || l > (1ull << 31)) usage();
@@ -455,7 +458,7 @@ struct Timing {
 //                 decoding of the next batch) / clb_finish_contig, BED text, plots
 Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, const std::map<std::string, FaiEntry> &fai,
                        std::map<int32_t, ContigStats> &stats, uint32_t largest, clb_ctx *ctx, clb_bed_writer *bed, DepthHistTsv *hist,
-                       DepthTilesTsv *tiles, clb_bedgraph_writer *bedgraph) {
+                       DepthTilesTsv *tiles, clb_bedgraph_writer *bedgraph, clb_bedgraph_writer *qc_bedgraph) {
     auto check = [&](int rc, const char *what) { if (rc != 0) die(std::string("Error processing contig: ") + what + ": " + clb_last_error(ctx)); };
     // coverage plots land next to the BED file (callable_profiler.rs:24-27,80-83)
     const size_t slash = opt.out_bed.find_last_of('/');
@@ -527,12 +530,21 @@ Timing process_contigs(const Options &opt, BamReader &bam, const BaiIndex *bai, 
             const int rc = clb_bed_writer_add_contig(bed, st.name.c_str(), clen, res.intervals, res.n_intervals, bins.data(), res.n_bins, res.stride, &has_bins);
             if (rc == CLB_E_IO) die("Error processing contig: cannot write " + opt.out_bed);
             if (rc != 0) die("Error processing contig: interval list does not tile the contig");
+            // raw and QC depth runs, each to its own bedGraph
+            auto write_runs = [&](clb_bedgraph_writer *w, const clb_depth_run *runs, uint64_t n, const std::string &path) {
+                const int rg = clb_bedgraph_writer_add_contig(w, st.name.c_str(), clen, runs, n);
+                if (rg == CLB_E_IO) die("cannot write " + path);
+                if (rg != 0) die("Error processing contig: depth runs do not tile the contig");
+            };
             if (bedgraph) {
                 const clb_depth_run *runs = nullptr; uint64_t n = 0;
                 check(clb_depth_runs(ctx, &runs, &n), "depth runs");
-                const int rg = clb_bedgraph_writer_add_contig(bedgraph, st.name.c_str(), clen, runs, n);
-                if (rg == CLB_E_IO) die("cannot write " + opt.depth_bedgraph);
-                if (rg != 0) die("Error processing contig: depth runs do not tile the contig");
+                write_runs(bedgraph, runs, n, opt.depth_bedgraph);
+            }
+            if (qc_bedgraph) {
+                const clb_depth_run *runs = nullptr; uint64_t n = 0;
+                check(clb_qc_depth_runs(ctx, &runs, &n), "QC depth runs");
+                write_runs(qc_bedgraph, runs, n, opt.qc_depth_bedgraph);
             }
             if (has_bins && res.stride) {                                        // finish_contig, callable_profiler.rs:64-86
                 const std::string path = out_dir + st.name + "_coverage.svg";
@@ -670,6 +682,8 @@ int run(int argc, char **argv) {
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     if (!opt.depth_bedgraph.empty() && clb_set_depth_runs(ctx.get(), 1) != 0)
         die(std::string("GPU context: ") + clb_last_error(ctx.get()));
+    if (!opt.qc_depth_bedgraph.empty() && clb_set_qc_depth_runs(ctx.get(), 1) != 0)
+        die(std::string("GPU context: ") + clb_last_error(ctx.get()));
     std::unique_ptr<clb_bed_writer, decltype(&clb_bed_writer_close)> bed(clb_bed_writer_open(opt.out_bed.c_str(), largest), clb_bed_writer_close);
     if (!bed) die("Failed to create CallableProfiler: cannot create " + opt.out_bed);
     // opened before the first contig (a FIFO blocks here until its reader is there), written per contig after its BED lines
@@ -677,6 +691,11 @@ int run(int argc, char **argv) {
     if (!opt.depth_bedgraph.empty()) {
         bedgraph.reset(clb_bedgraph_writer_open(opt.depth_bedgraph.c_str()));
         if (!bedgraph) die("cannot write " + opt.depth_bedgraph);
+    }
+    std::unique_ptr<clb_bedgraph_writer, decltype(&clb_bedgraph_writer_close)> qc_bedgraph(nullptr, clb_bedgraph_writer_close);
+    if (!opt.qc_depth_bedgraph.empty()) {
+        qc_bedgraph.reset(clb_bedgraph_writer_open(opt.qc_depth_bedgraph.c_str()));
+        if (!qc_bedgraph) die("cannot write " + opt.qc_depth_bedgraph);
     }
 
     // BamStats: its own pass over the first 10 000 records of the file, primary alignments only (bam_stats.rs:44-76)
@@ -696,10 +715,12 @@ int run(int argc, char **argv) {
         DepthHistTsv hist;
         DepthTilesTsv tiles(opt.depth_thresholds);
         const Timing t = process_contigs(opt, bam, indexed ? &bai : nullptr, fai, stats, largest, ctx.get(), bed.get(),
-                                         opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles, bedgraph.get());
+                                         opt.depth_hist.empty() ? nullptr : &hist, opt.depth_tiles.empty() ? nullptr : &tiles, bedgraph.get(),
+                                         qc_bedgraph.get());
         report_timing(opt, t, stats.size(), bam.inflate_seconds());
         if (clb_bed_writer_close(bed.release()) != 0) die("failed to write " + opt.out_bed);
         if (bedgraph && clb_bedgraph_writer_close(bedgraph.release()) != 0) die("cannot write " + opt.depth_bedgraph);
+        if (qc_bedgraph && clb_bedgraph_writer_close(qc_bedgraph.release()) != 0) die("cannot write " + opt.qc_depth_bedgraph);
         if (!opt.depth_hist.empty() && !write_file(opt.depth_hist, hist.finish())) die("cannot write " + opt.depth_hist);
         if (!opt.depth_tiles.empty() && !write_file(opt.depth_tiles, tiles.text)) die("cannot write " + opt.depth_tiles);
         ctx.reset();

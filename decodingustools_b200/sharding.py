@@ -140,6 +140,7 @@ def gather_and_stitch(local_intervals: np.ndarray, region_start: int, dst: int =
 
 
 def gather_and_stitch_depth_runs(local_runs: np.ndarray, region_start: int, dst: int = 0, group=None):
-    """Same for the depth runs (ContigDeviceResult.depth_runs): they are not additive, so they are gathered, not summed."""
+    """Same for the depth runs (ContigDeviceResult.depth_runs or qc_depth_runs): they are not additive, so they are
+    gathered, not summed."""
     parts = _gather_sorted(local_runs, RUN_DTYPE, region_start, dst, group)
     return None if parts is None else stitch_depth_runs(parts)

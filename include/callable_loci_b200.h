@@ -211,10 +211,13 @@ int clb_depth_tile_thresholds(const clb_ctx *ctx, const uint64_t **raw_ge, const
                               uint32_t *k, uint32_t *n_tiles);
 
 /* Depth runs (not in the reference; off by default; like bedtools genomecov -bga or mosdepth's per-base output): the raw
- * depth of every position of [region_start, region_end) as runs of equal depth.  Raw depth is the depth of
+ * or QC depth of every position of [region_start, region_end) as runs of equal depth.  Raw depth is the depth of
  * summed_coverage: admitted reads whose reference span covers the position, deletions and ref-skips included, no MAPQ or
- * base-quality filter; REF_N positions and depth 0 are included.  Run i covers [start_i, start_{i+1}), the last one ends at
- * region_end; starts ascend strictly from region_start and adjacent runs differ in depth.
+ * base-quality filter.  QC depth is the depth of quality_bases, the depth the states are called on: reads with MAPQ >=
+ * min_mapping_quality whose base at the position has quality >= min_base_quality, deletions excluded.  REF_N positions and
+ * depth 0 are included.  Run i covers [start_i, start_{i+1}), the last one ends at region_end; starts ascend strictly from
+ * region_start and adjacent runs differ in depth.  depth is the raw or the QC depth, depending on the call that returned
+ * the run (clb_depth_runs / clb_qc_depth_runs).
  * Region shards of one contig stitch by concatenation in genomic order, dropping a shard's first run when its depth equals
  * the previous shard's last (runs are defined by depth alone: no soft flag is needed). */
 typedef struct clb_depth_run {
@@ -226,6 +229,9 @@ int clb_set_depth_runs(clb_ctx *ctx, int on);
 /* The runs of the last clb_finish_contig / clb_rerun_resident with a result, owned by the context like the intervals.
  * When off: *runs = NULL, *n_runs = 0.  d2h_bytes counts their copy. */
 int clb_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_runs);
+/* The same for runs of equal QC depth, independent of the raw runs: either, both or neither may be on. */
+int clb_set_qc_depth_runs(clb_ctx *ctx, int on);
+int clb_qc_depth_runs(const clb_ctx *ctx, const clb_depth_run **runs, uint64_t *n_runs);
 
 /* Debug/parity: copy the per-base counters of [region_start, region_end) (computed by a separate
  * un-fused launch of the same pileup code).  Each pointer may be NULL. */
@@ -270,7 +276,7 @@ int  clb_bed_writer_add_contig(clb_bed_writer *w, const char *name, uint32_t con
                                uint32_t *bins_inout, uint32_t n_bins, uint32_t stride, int *has_bins);
 const char *clb_bed_writer_buffer(clb_bed_writer *w, uint64_t *len);   /* in-memory mode */
 int  clb_bed_writer_close(clb_bed_writer *w);
-/* bedGraph writer for depth runs: lines "name\tstart\tend\tdepth\n", no header.  Runs must tile [0, contig_len) (stitched
+/* bedGraph writer for depth runs (raw or QC): lines "name\tstart\tend\tdepth\n", no header.  Runs must tile [0, contig_len) (stitched
  * shards; none for an empty contig), else CLB_E_INVALID; a failed write gives CLB_E_IO.  A non-seekable path (a FIFO,
  * /dev/stdout) is written in order. */
 typedef struct clb_bedgraph_writer clb_bedgraph_writer;
